@@ -24,6 +24,10 @@ reported under `per_config`.
   cpu_baseline : the C++ oracle ("port" — the Rust reference cannot be built here) on all host cores, bounded sample
   --impl reference : the same CPU port as the reference arm (rank 0 only); every step is a bounded sample of the workload
              and the line reports the times it measured.
+  --dump-outputs DIR : after the timed steps, rank 0 writes what the last timed step of the headline workload returned —
+             the resolved image and the fp32 sample sums — as DIR/image.npy and DIR/sum.npy (float32; of an image above
+             DUMP_PIXELS pixels, a fixed seeded sample of pixels, listed in DIR/pixel_index.npy).  Inputs are fixed
+             (committed scene, seed 1), so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import gzip
@@ -55,6 +59,7 @@ B_NODE, B_SPHERE, B_RECT, B_TRI, B_CONIC, B_XROT, B_XTRANS, B_RAY = 32, 16, 32, 
 HBM_BYTES_PER_RAY = 176  # wavefront streams per extend + shade round (queues carry the records, all coalesced):
                          # extend: ray 32 r + hit record 48 w;  shade: hit record 48 r + next ray 32 w + attenuation 16 w
 FP32_NOMINAL_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12   # 148 SMs x 128 lanes x 2 flop x 1.965 GHz = 74.4
+DUMP_PIXELS = 1 << 20            # --dump-outputs keeps at most this many pixels: 2 x 12 MiB of float32 + 8 MiB of indices
 
 
 def read_scene_text(cfg):
@@ -173,6 +178,21 @@ def run_cpu(cfg, doc, assets, width, height, spp, target_seconds, seed):
     return st["samples"] / st["seconds"] / 1e6, st["rays"] / st["seconds"] / 1e6, st, port.describe(n), work
 
 
+def dump_outputs(out_dir, rgb, sums):
+    """Writes a render's u8 image and fp32 sums (both (H, W, 3)) as out_dir/image.npy and out_dir/sum.npy in float32.  An
+    image of more than DUMP_PIXELS pixels is reduced to the same fixed, seeded sample of pixels in both files, (n, 3) each,
+    whose flat pixel indices (y * W + x) go to out_dir/pixel_index.npy (float64, exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    rgb, sums = rgb.astype(np.float32), sums.astype(np.float32)
+    npix = rgb.shape[0] * rgb.shape[1]
+    if npix > DUMP_PIXELS:
+        idx = np.sort(np.random.default_rng(0).choice(npix, DUMP_PIXELS, replace=False))
+        rgb, sums = rgb.reshape(-1, 3)[idx], sums.reshape(-1, 3)[idx]
+        np.save(os.path.join(out_dir, "pixel_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "image.npy"), rgb)
+    np.save(os.path.join(out_dir, "sum.npy"), sums)
+
+
 def committed_profile(name, width, height, cfg):
     """ncu-derived facts of the extend kernels for this workload, from the committed capture (None if absent or if the
     run is not at the captured size): DRAM bytes per launch, busy lanes per instruction, IPC."""
@@ -199,7 +219,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-per-config", action="store_true", help="skip the table of the other BASELINE.json configs")
     ap.add_argument("--per-config-steps", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the image and fp32 sums of the last timed step to DIR/*.npy (see the docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -275,7 +299,7 @@ def main():
     except Exception:
         hbm_peak = 6650.0
 
-    def measure(c, w, h, spp, steps, warm, text_c, doc_c, assets_c, e2e_steps, cpu_seconds, sample_clocks):
+    def measure(c, w, h, spp, steps, warm, text_c, doc_c, assets_c, e2e_steps, cpu_seconds, sample_clocks, dump_dir=None):
         """Device-resident throughput, a separately profiled step, e2e through the host-buffer API, CPU port beside it."""
         ns = NativeScene(text_c, device=local_rank, assets=assets_c)
         renderer = c.renderer(width=w, height=h, samples=spp, seed=1)
@@ -284,12 +308,12 @@ def main():
         tot = {"rays": 0, "launches": 0}
 
         def step(timed_reduce=None):
-            img, _ = shard.render(spp, rank, world, reduce_events=timed_reduce)
+            img, total = shard.render(spp, rank, world, reduce_events=timed_reduce)
             st = shard.last_stats
             if st:
                 tot["rays"] += st["rays"]; tot["launches"] += st["launches"]
             tot["launches"] += 1 if rank == 0 else 0   # resolve
-            return img
+            return img, total
 
         sampler = ClockSampler(local_rank) if (rank == 0 and sample_clocks) else None
         for _ in range(warm):
@@ -300,10 +324,13 @@ def main():
         red = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)] if world > 1 else None
         t_wall0 = time.time()
         for i, (e0, e1) in enumerate(evs):
+            # the previous step's buffers go back to the allocator first, so that every step reuses the same sum buffer:
+            # with two buffers in turn, part2_all steps measured 0.4 % slower (B200, 1000 W power limit)
+            outs = None
             flush_buf.fill_(1)          # evict L2 between timed steps (not timed)
             barrier()
             e0.record(shard.stream)     # every kernel of the step is launched on shard.stream
-            step(red[i] if red else None)
+            outs = step(red[i] if red else None)
             e1.record(shard.stream)
         barrier()
         t_wall1 = time.time()
@@ -318,6 +345,9 @@ def main():
                "rays_per_sample": rays_all / samples_all, "gpu_launches": int(launches_all), "steps": steps, "clocks": clocks}
         if world > 1:
             out["reduce"] = {"ms_per_step": ms_reduce / steps, "bytes": npix * 12, "what": "ncclReduce(SUM, fp32) of the sum buffers to rank 0 (torch.distributed), CUDA events around it, max over ranks"}
+        if dump_dir and rank == 0:
+            dump_outputs(dump_dir, outs[0], outs[1].cpu().numpy().reshape(h, w, 3))
+        outs = None
 
         # ---- one extra step with per-launch events around the extend kernels (never inside the timed region) -----
         ns.set_profiling(True)
@@ -409,7 +439,8 @@ def main():
                                        "kind": "port", "sample": sample}
         return out
 
-    main_res = measure(cfg, width, height, spp_total, args.steps, warmup, text, doc, assets, args.steps, args.cpu_seconds, True)
+    main_res = measure(cfg, width, height, spp_total, args.steps, warmup, text, doc, assets, args.steps, args.cpu_seconds, True,
+                       args.dump_outputs)
 
     per_config = {}
     if not args.no_per_config:
