@@ -29,6 +29,14 @@ class FwStats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class FwAdaptive(C.Structure):
+    _fields_ = [("min_samples", C.c_uint32), ("threshold", C.c_float), ("floor", C.c_float)]
+
+
+class FwAdaptiveResult(C.Structure):
+    _fields_ = [("rounds", C.c_uint32), ("samples", C.c_uint64), ("active", C.c_uint32 * 32)]
+
+
 class FireworkError(RuntimeError):
     def __init__(self, code, msg):
         super().__init__(f"firework_b200 error {code}: {msg}")
@@ -44,7 +52,7 @@ EXPORTS = [
     "fw_env_sample", "fw_texture_sample", "fw_material_texture", "fw_camera", "fw_last_error", "fw_version",
     "fw_device_count", "fw_measure_peaks", "fw_selftest_shared_division", "fw_obj_load", "fw_obj_num_models",
     "fw_obj_model_name", "fw_obj_model_sizes", "fw_obj_model_copy", "fw_obj_destroy", "fw_hdr_load", "fw_hdr_free", "fw_image_load", "fw_image_free", "fw_png_write", "fw_set_profiling", "fw_set_batch_paths", "fw_release_cached_memory", "fw_texture_store_stats",
-    "fw_resolve_host", "fw_render_multi", "fw_scene_walk_info", "fw_first_hit_wavefront",
+    "fw_resolve_host", "fw_render_multi", "fw_scene_walk_info", "fw_first_hit_wavefront", "fw_render_adaptive",
 ]
 
 _lib = None
@@ -127,6 +135,9 @@ def lib():
         L.fw_resolve_host.argtypes = [C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_float, C.c_void_p]
         L.fw_render_multi.argtypes = [C.c_void_p, C.POINTER(FwParams), C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                       C.POINTER(FwStats), C.POINTER(C.c_double)]
+        if hasattr(L, "fw_render_adaptive"):        # absent only in older builds used for A/B timing
+            L.fw_render_adaptive.argtypes = [C.c_void_p, C.POINTER(FwParams), C.POINTER(FwAdaptive)] + [C.c_void_p] * 4 + \
+                                            [C.POINTER(FwStats), C.POINTER(FwAdaptiveResult)]
         _lib = L
     return _lib
 

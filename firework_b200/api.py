@@ -587,7 +587,8 @@ class CameraSettings:
 class Renderer:
     """render.rs:57-107; defaults per render.rs:198-218 (1920x1080, 128 spp, use_bvh=false, gamma 2.2).
 
-    Extra (not in the reference): `seed` keys the counter-based RNG, `device` picks the GPU.
+    Extra (not in the reference): `seed` keys the counter-based RNG, `device` picks the GPU, `gpus` spreads the samples over
+    several GPUs, `adaptive` renders each pixel until its noise estimate meets a target.
     """
 
     def __init__(self):
@@ -596,6 +597,7 @@ class Renderer:
         self._camera = CameraSettings()
         self._seed = 0
         self._gpus, self._reduce = 1, "nccl"
+        self._adaptive = None
         self.last_stats = None
 
     @staticmethod
@@ -607,6 +609,23 @@ class Renderer:
         into one slice per GPU, the fp32 sums are combined by one NCCL reduce ("nccl") or by the fused peer-memory
         reduce + resolve kernel ("peer")."""
         self._gpus, self._reduce = int(n), reduce
+        return self
+
+    def adaptive(self, threshold, min_samples=16, floor=None):
+        """Extra (not in the reference): adaptive sampling (fw_render_adaptive).  `samples` becomes the cap per pixel; every
+        pixel renders `min_samples` samples, then rounds of doubling sample counts go on for the pixels whose relative standard
+        error of the mean luminance is still above `threshold` (e.g. 0.05 = 5 %).  A pixel that ends with k samples has
+        exactly the value a uniform render at k samples gives it.  `floor` (default 0.01, linear luminance) bounds the
+        error's denominator from below: under it the target becomes the absolute error threshold * floor, which for
+        threshold 0.05 is under one u8 level after gamma 2.2, so near-black pixels stop early instead of chasing a relative
+        error their displayed value can not show.  `threshold=None` switches adaptive sampling off.  Single GPU only:
+        together with gpus(n > 1) `render` raises ValueError.  last_stats then carries `counts` (per-pixel samples), `error`
+        (per-pixel final relative error), `rounds` and `active` (pixels rendered in each round)."""
+        if threshold is None:
+            self._adaptive = None
+        else:
+            from .engine import ADAPTIVE_FLOOR
+            self._adaptive = (float(threshold), int(min_samples), ADAPTIVE_FLOOR if floor is None else float(floor))
         return self
 
     def width(self, w):
@@ -659,6 +678,18 @@ class Renderer:
     def render(self, scene: Scene) -> np.ndarray:
         """GPU drop-in for `Renderer::render` — returns (height, width, 3) u8, row 0 = top."""
         from .engine import NativeScene, render_scene
+        if self._adaptive is not None:
+            if self._gpus > 1:
+                raise ValueError("adaptive sampling renders on one GPU: gpus(n > 1) and adaptive() can not be combined")
+            threshold, min_samples, floor = self._adaptive
+            ns = NativeScene.from_scene(scene, 0)
+            try:
+                rgb, _sum, counts, err, stats = ns.render_adaptive(self.params(), threshold, min_samples, floor, want_sum=False)
+            finally:
+                ns.close()
+            stats["counts"], stats["error"] = counts, err
+            self.last_stats = stats
+            return rgb
         if self._gpus > 1:
             ns = NativeScene.from_scene(scene, 0)
             try:

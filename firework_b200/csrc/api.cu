@@ -273,6 +273,8 @@ static void destroy_ctx(RenderCtx* c) {
     if (c->arena) cudaFree(c->arena);
     for (void* p : c->arena_retired) cudaFree(p);
     fr(c->d_sum); fr(c->d_rgb);
+    fr(c->adapt.m1); fr(c->adapt.m2); fr(c->adapt.count); fr(c->adapt.err); fr(c->adapt.list[0]); fr(c->adapt.list[1]);
+    fr(c->adapt.keep); fr(c->adapt.block_base);
     if (c->h_rays) cudaFreeHost(c->h_rays);
     if (c->h_stage) cudaFreeHost(c->h_stage);
     if (c->d_rays) cudaFree(c->d_rays);
@@ -1008,9 +1010,10 @@ static int debug_extend(fw_scene* sc, const Batch& b, uint2 seed, uint32_t bounc
     return FW_OK;
 }
 
-// One batch: raygen, up to FW_MAX_DEPTH+1 extend/shade rounds, accumulate into d_sum.
+// One batch: raygen, up to FW_MAX_DEPTH+1 extend/shade rounds, accumulate into d_sum (and, for a round of an adaptive render,
+// into the moments and counts of `adapt`).
 static int run_batch(fw_scene* sc, const CameraRec& cam, const Batch& b, uint2 seed, bool use_bvh, float* d_sum,
-                     cudaStream_t st, RunTotals& tot, size_t& ev_next) {
+                     const AdaptiveState* adapt, cudaStream_t st, RunTotals& tot, size_t& ev_next) {
     PathState& ps = sc->ctx->ps;
     const DeviceScene& S = sc->dscene;
     uint32_t N = b.npix * b.ns;
@@ -1086,7 +1089,8 @@ static int run_batch(fw_scene* sc, const CameraRec& cam, const Batch& b, uint2 s
                 }
         }
     }
-    launch_accumulate(d_sum, ps, b, grid_for(b.npix, 256, sm * 8), st);
+    if (adapt) launch_accumulate_adaptive(d_sum, *adapt, ps, b, grid_for(b.npix, 256, sm * 8), st);
+    else launch_accumulate(d_sum, ps, b, grid_for(b.npix, 256, sm * 8), st);
     tot.launches++;
     launch_tally(ps, sc->ctx->d_rays, st);
     tot.launches++;
@@ -1096,17 +1100,9 @@ static int run_batch(fw_scene* sc, const CameraRec& cam, const Batch& b, uint2 s
     return FW_OK;
 }
 
-int fw::render_into(fw_scene* sc, const fw_params* p, float* d_sum, cudaStream_t st, fw_stats* stats) {
-    if (!sc->committed) return set_error(FW_ERR_STATE, "fw_scene_commit must be called before rendering");
-    if (!p || p->width == 0 || p->height == 0 || p->samples == 0)
-        return set_error(FW_ERR_ARG, "width, height and samples must be non-zero");
-    if ((uint64_t)p->width * p->height > 0x7fffffffull) return set_error(FW_ERR_ARG, "image too large");
-    FW_CUDA(cudaSetDevice(sc->device));
-    RenderParamsHost hp;
-    memcpy(&hp, p, sizeof(hp));
-    CameraRec cam = make_camera(hp);
-    uint2 seed = make_uint2((uint32_t)p->seed, (uint32_t)(p->seed >> 32));
-    size_t npix = (size_t)p->width * p->height;
+// Paths in flight per batch for a render of `paths` paths in all, and path state for batches of that size (FW_BATCH_PATHS /
+// fw_set_batch_paths, shrunk to what the device can give).  Results do not depend on the batch split, only the speed does.
+static int prepare_batches(fw_scene* sc, size_t paths, size_t* cap_out) {
     // Paths in flight per batch.  Larger batches keep the deep, thinly populated bounces big enough to fill the
     // GPU and amortise the ~8 launches per bounce (measured: +6 % cornell, +18 % random_spheres, +34 % teapot
     // from 4 Mi to 32 Mi paths; part2_all at 4K another +6 % / +9 % at 64 Mi / 128 Mi); up to ~500 B of state per path
@@ -1114,12 +1110,12 @@ int fw::render_into(fw_scene* sc, const fw_params* p, float* d_sum, cudaStream_t
     size_t cap = sc->batch_paths ? sc->batch_paths : ((size_t)FW_DEFAULT_BATCH_PATHS);
     if (const char* e = getenv("FW_BATCH_PATHS")) cap = std::max<size_t>(1024, strtoull(e, nullptr, 10));
     if (const char* e = getenv("FW_TWO_PASS")) sc->plan.two_pass = atoi(e) != 0;
-    cap = std::min<size_t>(cap, npix * std::max<uint32_t>(p->sample_count, 1));
+    cap = std::min<size_t>(cap, paths);
     cap = std::max<size_t>(cap, 32);
     int rc;
     if (cap > sc->ctx->ps_cap) {
         // The context has to grow: keep the batch inside what the device can give (other scenes of this process hold
-        // contexts of their own).  Results do not depend on the batch split, only the speed does.
+        // contexts of their own).
         size_t queues = 1;   // + mesh queue
         for (int k = 0; k < MAT_NUM_QUEUES; ++k) queues += (k != MAT_MISS && sc->mat_present[k]) ? 1 : 0;
         const size_t per_path = 64 + 16 * FW_MAX_DEPTH + 16 + 16 + 48 * queues + (sc->plan.walk ? 8 + 16 * (size_t)sc->flat.n_top_meshes : 0);
@@ -1157,33 +1153,44 @@ int fw::render_into(fw_scene* sc, const fw_params* p, float* d_sum, cudaStream_t
         cap >>= 1;
     }
     if (rc != FW_OK) return rc;
-    cap = std::min<size_t>(cap, sc->ctx->ps_cap);
-    RunTotals tot;
-    size_t ev_next = 0;
-    FW_CUDA(cudaMemsetAsync(sc->ctx->d_rays, 0, sizeof(unsigned long long), st));
-    FW_CUDA(cudaEventRecord(sc->ctx->ev_begin, st));
-    // pixel tiles outer, sample chunks inner: every pixel's samples are accumulated in sample order
+    *cap_out = std::min<size_t>(cap, sc->ctx->ps_cap);
+    return FW_OK;
+}
+
+// Samples [s_begin, s_begin + s_count) of `npix` pixels — the image's pixels 0 .. npix-1, or the first npix entries of a pixel
+// list — in batches of at most `cap` paths: pixel tiles outer, sample chunks inner, so every pixel's samples are accumulated
+// in sample order.
+static int run_tiles(fw_scene* sc, const fw_params* p, const CameraRec& cam, uint2 seed, size_t cap, size_t npix, const uint32_t* pixels,
+                     uint32_t s_begin, uint32_t s_count, float* d_sum, const AdaptiveState* adapt, cudaStream_t st, RunTotals& tot,
+                     size_t& ev_next) {
+    int rc;
     size_t tile = std::min(npix, cap);
     for (size_t pix0 = 0; pix0 < npix; pix0 += tile) {
         size_t np = std::min(tile, npix - pix0);
         uint32_t chunk = (uint32_t)std::max<size_t>(1, cap / np);
-        for (uint32_t s = 0; s < p->sample_count; s += chunk) {
+        for (uint32_t s = 0; s < s_count; s += chunk) {
             Batch b;
             b.pix0 = (uint32_t)pix0; b.npix = (uint32_t)np;
-            b.s0 = p->sample_begin + s; b.ns = std::min(chunk, p->sample_count - s);
+            b.s0 = s_begin + s; b.ns = std::min(chunk, s_count - s);
             b.width = p->width; b.height = p->height;
             b.npix_magic = np <= 1 ? 0xffffffffu : (uint32_t)((((uint64_t)1 << 32) + np - 1) / np);
             b.width_magic = p->width <= 1 ? 0xffffffffu : (uint32_t)((((uint64_t)1 << 32) + p->width - 1) / p->width);
-            if ((rc = run_batch(sc, cam, b, seed, p->use_bvh != 0, d_sum, st, tot, ev_next)) != FW_OK) return rc;
+            b.pixels = pixels;
+            if ((rc = run_batch(sc, cam, b, seed, p->use_bvh != 0, d_sum, adapt, st, tot, ev_next)) != FW_OK) return rc;
         }
     }
+    return FW_OK;
+}
+
+// Closes the device work of one call (ev_begin was recorded at its start): ray tally, event times -> stats.  Synchronises `st`.
+static int finish_call(fw_scene* sc, cudaStream_t st, RunTotals& tot, uint64_t samples, fw_stats* stats) {
     FW_CUDA(cudaEventRecord(sc->ctx->ev_end, st));
     FW_CUDA(cudaMemcpyAsync(sc->ctx->h_rays, sc->ctx->d_rays, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     FW_CUDA(cudaStreamSynchronize(st));
     tot.rays = *sc->ctx->h_rays;
     if (stats) {
         memset(stats, 0, sizeof(*stats));
-        stats->samples = (uint64_t)npix * p->sample_count;
+        stats->samples = samples;
         stats->rays = tot.rays;
         stats->launches = tot.launches;
         stats->extend_launches = tot.extend_launches;
@@ -1201,6 +1208,29 @@ int fw::render_into(fw_scene* sc, const fw_params* p, float* d_sum, cudaStream_t
     return FW_OK;
 }
 
+int fw::render_into(fw_scene* sc, const fw_params* p, float* d_sum, cudaStream_t st, fw_stats* stats) {
+    if (!sc->committed) return set_error(FW_ERR_STATE, "fw_scene_commit must be called before rendering");
+    if (!p || p->width == 0 || p->height == 0 || p->samples == 0)
+        return set_error(FW_ERR_ARG, "width, height and samples must be non-zero");
+    if ((uint64_t)p->width * p->height > 0x7fffffffull) return set_error(FW_ERR_ARG, "image too large");
+    FW_CUDA(cudaSetDevice(sc->device));
+    RenderParamsHost hp;
+    memcpy(&hp, p, sizeof(hp));
+    CameraRec cam = make_camera(hp);
+    uint2 seed = make_uint2((uint32_t)p->seed, (uint32_t)(p->seed >> 32));
+    size_t npix = (size_t)p->width * p->height;
+    size_t cap = 0;
+    int rc = prepare_batches(sc, npix * std::max<uint32_t>(p->sample_count, 1), &cap);
+    if (rc != FW_OK) return rc;
+    RunTotals tot;
+    size_t ev_next = 0;
+    FW_CUDA(cudaMemsetAsync(sc->ctx->d_rays, 0, sizeof(unsigned long long), st));
+    FW_CUDA(cudaEventRecord(sc->ctx->ev_begin, st));
+    if ((rc = run_tiles(sc, p, cam, seed, cap, npix, nullptr, p->sample_begin, p->sample_count, d_sum, nullptr, st, tot, ev_next)) != FW_OK)
+        return rc;
+    return finish_call(sc, st, tot, (uint64_t)npix * p->sample_count, stats);
+}
+
 int fw::ensure_sum_buffers(fw_scene* sc, size_t npix) {
     if (sc->ctx->d_sum_pix >= npix) return FW_OK;
     if (sc->ctx->d_sum) cudaFree(sc->ctx->d_sum);
@@ -1209,6 +1239,24 @@ int fw::ensure_sum_buffers(fw_scene* sc, size_t npix) {
     FW_CUDA(cudaMalloc(&sc->ctx->d_sum, npix * 3 * sizeof(float)));
     FW_CUDA(cudaMalloc(&sc->ctx->d_rgb, npix * 3));
     sc->ctx->d_sum_pix = npix;
+    return FW_OK;
+}
+int fw::ensure_adaptive_buffers(fw_scene* sc, size_t npix) {
+    RenderCtx* c = sc->ctx;
+    if (c->adapt_pix >= npix) return FW_OK;
+    AdaptiveState& a = c->adapt;
+    auto fr = [](auto*& p) { if (p) { cudaFree(p); p = nullptr; } };
+    fr(a.m1); fr(a.m2); fr(a.count); fr(a.err); fr(a.list[0]); fr(a.list[1]); fr(a.keep); fr(a.block_base);
+    c->adapt_pix = 0;
+    FW_CUDA(cudaMalloc(&a.m1, npix * sizeof(double)));
+    FW_CUDA(cudaMalloc(&a.m2, npix * sizeof(double)));
+    FW_CUDA(cudaMalloc(&a.count, npix * sizeof(uint32_t)));
+    FW_CUDA(cudaMalloc(&a.err, npix * sizeof(float)));
+    FW_CUDA(cudaMalloc(&a.list[0], npix * sizeof(uint32_t)));
+    FW_CUDA(cudaMalloc(&a.list[1], npix * sizeof(uint32_t)));
+    FW_CUDA(cudaMalloc(&a.keep, npix));
+    FW_CUDA(cudaMalloc(&a.block_base, ((size_t)adaptive_blocks((uint32_t)npix) + 1) * sizeof(uint32_t)));
+    c->adapt_pix = npix;
     return FW_OK;
 }
 int fw::commit_scene(fw_scene* sc, int device) { return fw_scene_commit(sc, device); }
@@ -1270,6 +1318,80 @@ int fw_render(fw_scene* sc, const fw_params* p, uint8_t* rgb_out, float* sum_out
         }
         if (sum_out) FW_CUDA(cudaMemcpyAsync(sum_out, sc->ctx->d_sum, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, sc->ctx->stream));
         FW_CUDA(cudaStreamSynchronize(sc->ctx->stream));
+        return FW_OK;
+});
+}
+
+// Adaptive sampling (DESIGN.md §11).  Round 0 renders samples [0, n0) of every pixel; after round r the pixels whose relative
+// error is not yet <= threshold render [n_r, min(2 n_r, cap)) in round r + 1.  Each round is the ordinary batch loop over the
+// active pixel list, so a pixel with k samples holds the sums of fw_render at samples = k.
+int fw_render_adaptive(fw_scene* sc, const fw_params* p, const fw_adaptive* ad, uint8_t* rgb_out, float* sum_out, uint32_t* count_out,
+                       float* error_out, fw_stats* stats, fw_adaptive_result* result) {
+    return guarded([&]() -> int {
+        // every argument check comes before the first CUDA call
+        if (!sc || !p || !ad) return set_error(FW_ERR_ARG, "null argument");
+        if (p->width == 0 || p->height == 0 || p->samples == 0) return set_error(FW_ERR_ARG, "width, height and samples must be non-zero");
+        if ((uint64_t)p->width * p->height > 0x7fffffffull) return set_error(FW_ERR_ARG, "image too large");
+        if (p->sample_begin != 0 || p->sample_count != p->samples)
+            return set_error(FW_ERR_ARG, "an adaptive render owns the sample range: sample_begin must be 0 and sample_count == samples (the cap)");
+        if (ad->min_samples == 0) return set_error(FW_ERR_ARG, "min_samples must be >= 1");
+        if (!(ad->threshold >= 0.0f) || !std::isfinite(ad->threshold)) return set_error(FW_ERR_ARG, "threshold must be finite and >= 0");
+        if (!(ad->floor > 0.0f) || !std::isfinite(ad->floor)) return set_error(FW_ERR_ARG, "floor must be finite and > 0");
+        if (!sc->committed || !sc->ctx) return set_error(FW_ERR_STATE, "fw_scene_commit must be called before rendering");
+        FW_CUDA(cudaSetDevice(sc->device));
+        const size_t npix = (size_t)p->width * p->height;
+        int rc;
+        if ((rc = ensure_sum_buffers(sc, npix)) != FW_OK || (rc = ensure_adaptive_buffers(sc, npix)) != FW_OK) return rc;
+        RenderParamsHost hp;
+        memcpy(&hp, p, sizeof(hp));
+        const CameraRec cam = make_camera(hp);
+        const uint2 seed = make_uint2((uint32_t)p->seed, (uint32_t)(p->seed >> 32));
+        size_t cap = 0;
+        if ((rc = prepare_batches(sc, npix * p->samples, &cap)) != FW_OK) return rc;
+        RenderCtx* c = sc->ctx;
+        const AdaptiveState& A = c->adapt;
+        cudaStream_t st = c->stream;
+        const unsigned grid = grid_for(npix, 256, sc->sm_count * 8);
+        const double threshold = ad->threshold, floor = ad->floor;
+        FW_CUDA(cudaMemsetAsync(c->d_sum, 0, npix * 3 * sizeof(float), st));
+        FW_CUDA(cudaMemsetAsync(A.m1, 0, npix * sizeof(double), st));
+        FW_CUDA(cudaMemsetAsync(A.m2, 0, npix * sizeof(double), st));
+        FW_CUDA(cudaMemsetAsync(A.count, 0, npix * sizeof(uint32_t), st));
+        RunTotals tot;
+        size_t ev_next = 0;
+        FW_CUDA(cudaMemsetAsync(c->d_rays, 0, sizeof(unsigned long long), st));
+        FW_CUDA(cudaEventRecord(c->ev_begin, st));
+        launch_adaptive_init(A.list[0], (uint32_t)npix, grid, st);
+        tot.launches++;
+        fw_adaptive_result res;
+        memset(&res, 0, sizeof(res));
+        uint32_t active = (uint32_t)npix, n_prev = 0, n = std::min(ad->min_samples, p->samples);
+        int cur = 0;
+        for (;;) {
+            if ((rc = run_tiles(sc, p, cam, seed, cap, active, A.list[cur], n_prev, n - n_prev, c->d_sum, &A, st, tot, ev_next)) != FW_OK) return rc;
+            if (res.rounds < 32) res.active[res.rounds] = active;
+            res.rounds++;
+            res.samples += (uint64_t)active * (n - n_prev);
+            if (n == p->samples) break;   // the cap: nothing left to decide
+            tot.launches += launch_converge_compact(A, A.list[cur], active, threshold, floor, A.list[cur ^ 1], st);
+            FW_CUDA(cudaGetLastError());
+            FW_CUDA(cudaMemcpyAsync(&active, A.block_base + adaptive_blocks(active), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+            FW_CUDA(cudaStreamSynchronize(st));
+            cur ^= 1;
+            if (active == 0) break;
+            n_prev = n;
+            n = n > p->samples / 2 ? p->samples : 2 * n;
+        }
+        launch_resolve_adaptive(c->d_sum, A, (uint32_t)npix, p->gamma, floor, c->d_rgb, grid, st);
+        FW_CUDA(cudaGetLastError());
+        tot.launches++;
+        if ((rc = finish_call(sc, st, tot, res.samples, stats)) != FW_OK) return rc;
+        if (rgb_out) FW_CUDA(cudaMemcpyAsync(rgb_out, c->d_rgb, npix * 3, cudaMemcpyDeviceToHost, st));
+        if (sum_out) FW_CUDA(cudaMemcpyAsync(sum_out, c->d_sum, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
+        if (count_out) FW_CUDA(cudaMemcpyAsync(count_out, A.count, npix * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        if (error_out) FW_CUDA(cudaMemcpyAsync(error_out, A.err, npix * sizeof(float), cudaMemcpyDeviceToHost, st));
+        FW_CUDA(cudaStreamSynchronize(st));
+        if (result) *result = res;
         return FW_OK;
 });
 }
@@ -1348,7 +1470,7 @@ int fw_first_hit_wavefront(fw_scene* sc, int use_bvh, uint64_t seed, uint32_t n,
     FW_CUDA(cudaMemsetAsync(ps.counters, 0, sizeof(uint32_t) * (FW_MAX_DEPTH + 2) * FW_NUM_QUEUES * (size_t)ps.nseg, st));
     FW_CUDA(cudaMemsetAsync(ps.poison, 0, sizeof(uint32_t), st));
     Batch b;   // ray i = path i = "pixel" i of a one-sample batch: RNG key (pixel i, sample, bounce)
-    b.pix0 = 0; b.npix = n; b.s0 = sample; b.ns = 1; b.width = n; b.height = 1;
+    b.pix0 = 0; b.npix = n; b.s0 = sample; b.ns = 1; b.width = n; b.height = 1; b.pixels = nullptr;
     b.npix_magic = n <= 1 ? 0xffffffffu : (uint32_t)((((uint64_t)1 << 32) + n - 1) / n);
     b.width_magic = b.npix_magic;   // width == n
     const uint2 sd = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));

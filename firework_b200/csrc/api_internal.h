@@ -45,6 +45,8 @@ struct RenderCtx {
     float* d_sum = nullptr;
     unsigned char* d_rgb = nullptr;
     size_t d_sum_pix = 0;
+    AdaptiveState adapt{};       // fw_render_adaptive: moments, counts, active lists (~33 B per pixel), sized on first use
+    size_t adapt_pix = 0;
     unsigned long long* d_rays = nullptr;   // device-side ray tally of the current render call
     unsigned long long* h_rays = nullptr;   // pinned
     std::vector<cudaEvent_t> ev_pool;
@@ -114,6 +116,7 @@ namespace fw {
 // One sample range of `p` added into d_sum (device, width*height*3 fp32) on stream `st`; synchronises `st`.
 int render_into(fw_scene* sc, const fw_params* p, float* d_sum, cudaStream_t st, fw_stats* stats);
 int ensure_sum_buffers(fw_scene* sc, size_t npix);   // ctx->d_sum / d_rgb sized for npix pixels
+int ensure_adaptive_buffers(fw_scene* sc, size_t npix);   // ctx->adapt sized for npix pixels
 int commit_scene(fw_scene* sc, int device);          // fw_scene_commit
 void destroy_scene(fw_scene* sc);                    // fw_scene_destroy
 unsigned grid_for(size_t n, unsigned threads, unsigned max_blocks);

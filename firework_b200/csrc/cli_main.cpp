@@ -7,13 +7,16 @@
 // Extras (not in the reference): --width / --height / --seed, --gpus N (fw_render_multi: sample range split over N GPUs of
 // the box), a .gz scene file is inflated on the fly, and --checkpoint FILE [--chunk N]: the samples are rendered N at a time,
 // the fp32 sums and the number of samples done are saved after every chunk, and a later run with the same arguments continues
-// where the file stops (SURVEY.md §8f row 2; the reference's 3.36 h render had no way to resume).  The file format is shared
+// where the file stops (SURVEY.md §8f row 2; the reference's 3.36 h render had no way to resume).  --target-error E
+// [--min-samples N]: adaptive sampling (fw_render_adaptive), each pixel renders until its relative standard error is <= E,
+// with -s as the cap per pixel; it owns its sample schedule, so it is refused together with --checkpoint, --chunk or --gpus > 1.  The file format is shared
 // with `python -m firework_b200 --checkpoint x.fwck` (firework_b200/progressive.py), so either driver finishes what the other began.
 // Links libfirework_b200.a: nothing here goes through Python.
 #include <zlib.h>
 
 #include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -31,7 +34,9 @@ void usage(FILE* f) {
             "    -n, --name <name>\n    -o, --output <output>\n    -s, --samples <samples>\n        --scene-file <scene-file>\n"
             "        --width <px>       (default 960)\n        --height <px>      (default 540)\n        --seed <u64>       (default 0)\n"
             "        --gpus <n>         render on n GPUs of this box (default 1)\n"
-            "        --checkpoint <f>   resume from / save to this file after every chunk\n        --chunk <n>        samples per chunk (default: all)\n    -h, --help\n");
+            "        --checkpoint <f>   resume from / save to this file after every chunk\n        --chunk <n>        samples per chunk (default: all)\n"
+            "        --target-error <e> adaptive sampling: render each pixel until its relative standard error <= e (-s is the cap)\n"
+            "        --min-samples <n>  adaptive sampling: samples of the first round (default 16)\n    -h, --help\n");
 }
 [[noreturn]] void die(const std::string& msg) {
     fprintf(stderr, "error: %s\n", msg.c_str());
@@ -130,7 +135,9 @@ void save_checkpoint(const std::string& path, const fw_params& p, uint64_t fp, c
 
 int main(int argc, char** argv) {
     std::string scene_file, name, output, checkpoint;
-    long samples = -1, width = 960, height = 540, gpus = 1, chunk = 0;
+    long samples = -1, width = 960, height = 540, gpus = 1, chunk = 0, min_samples = 16;
+    double target_error = -1.0;   // < 0: uniform render
+    bool adaptive = false;
     unsigned long long seed = 0;
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
@@ -154,6 +161,8 @@ int main(int argc, char** argv) {
         else if (is("--seed", nullptr)) seed = strtoull(value("--seed").c_str(), nullptr, 10);
         else if (is("--checkpoint", nullptr)) checkpoint = value("--checkpoint");
         else if (is("--chunk", nullptr)) chunk = atol(value("--chunk").c_str());
+        else if (is("--target-error", nullptr)) { target_error = atof(value("--target-error <e>").c_str()); adaptive = true; }
+        else if (is("--min-samples", nullptr)) min_samples = atol(value("--min-samples <n>").c_str());
         else { usage(stderr); die("Found argument '" + a + "' which wasn't expected"); }
     }
     if (scene_file.empty() || samples < 0) {
@@ -162,6 +171,11 @@ int main(int argc, char** argv) {
             (samples < 0 ? "--samples <samples>" : ""));
     }
     if (width <= 0 || height <= 0 || width > 65535 || height > 65535 || gpus < 1) die("bad --width / --height / --gpus");
+    if (adaptive) {   // an adaptive render owns its sample schedule: no chunks, no checkpoint, one GPU
+        if (!checkpoint.empty() || chunk > 0) die("--target-error can not be combined with --checkpoint or --chunk");
+        if (gpus > 1) die("--target-error renders on one GPU: it can not be combined with --gpus > 1");
+        if (!(target_error >= 0.0) || !std::isfinite(target_error) || min_samples < 1) die("--target-error must be finite and >= 0, --min-samples >= 1");
+    }
 
     // main.rs:25-26
     const std::string text = read_text(scene_file);
@@ -206,7 +220,13 @@ int main(int argc, char** argv) {
         if (gpus > 1) check(fw_render_multi(scene, &q, (int)gpus, nullptr, FW_REDUCE_NCCL, rgb_out, sum_out, &st, nullptr), "render");
         else check(fw_render(scene, &q, rgb_out, sum_out, &st), "render");
     };
-    if (checkpoint.empty() && chunk <= 0) {
+    fw_adaptive_result ares;
+    memset(&ares, 0, sizeof ares);
+    if (adaptive) {
+        fw_adaptive ad;
+        ad.min_samples = (uint32_t)min_samples; ad.threshold = (float)target_error; ad.floor = 0.01f;   // engine.ADAPTIVE_FLOOR
+        check(fw_render_adaptive(scene, &p, &ad, rgb.data(), nullptr, nullptr, nullptr, &st, &ares), "render");
+    } else if (checkpoint.empty() && chunk <= 0) {
         render_range(p, rgb.data(), nullptr);
     } else {
         // sample-range chunks: RNG streams are keyed by the global sample index, so [0, k) now and [k, n) later are the
@@ -230,6 +250,9 @@ int main(int argc, char** argv) {
     }
     const auto end = std::chrono::steady_clock::now();
     printf("Finished Rendering in %lld s\n", (long long)std::chrono::duration_cast<std::chrono::seconds>(end - start).count());
+    if (adaptive)
+        printf("Adaptive: %llu samples in %u rounds, %.2f spp mean (cap %ld)\n", (unsigned long long)ares.samples, ares.rounds,
+               (double)ares.samples / ((double)width * height), samples);
     fw_scene_destroy(scene);
 
     if (name.empty()) name = "Firework Render";

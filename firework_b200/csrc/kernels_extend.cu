@@ -5,12 +5,13 @@
 namespace fw {
 
 // Debug twin of the BVH extend: also records the number of box tests each path needed (FW_DEBUG_STEPS=1).
+template <bool LIST>
 __global__ void __launch_bounds__(FW_BLOCK) extend_bvh_debug_kernel(DeviceScene S, PathState ps, Batch b, uint2 seed, uint32_t bounce,
                                                                     uint32_t* steps) {
     FW_EXTEND_PROLOGUE(MAT_NUM_QUEUES)
         if (valid) {
             RngKey key{seed, 0u, 0u, bounce};
-            batch_path(b, path, key.pixel, key.sample);
+            batch_path<LIST>(b, path, key.pixel, key.sample);
             Counters cnt{0, 0};
             trace_unified<true, true>(S, o, d, key, w, &cnt);
             steps[path] = (uint32_t)cnt.node_tests;
@@ -25,7 +26,7 @@ __global__ void __launch_bounds__(FW_BLOCK) extend_bvh_debug_kernel(DeviceScene 
 // ENTRIES: the mesh walk (kernels_walk.cu) finishes the bounce instead of pass 2: every ray that must enter a mesh also
 // gets its pass-1 winner written as a 64-bit key (walk.cuh pack_key) and one (mesh-queue slot, mesh rank) entry per mesh
 // root box it hit.
-template <bool NESTED, bool ENTRIES>
+template <bool NESTED, bool ENTRIES, bool LIST>
 __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_pass1_kernel(DeviceScene S, PathState ps, Batch b, uint2 seed,
                                                                                 uint32_t bounce, WalkAux aux) {
     __shared__ uint32_t s_fill[FW_NUM_QUEUES];
@@ -46,7 +47,7 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_pass1_k
             float4 ro = ld_stream(&ps.xo[bounce & 1][slot_in]), rd = ld_stream(&ps.xd[bounce & 1][slot_in]);
             o = f3(ro); d = f3(rd); path = __float_as_uint(ro.w);
             RngKey key{seed, 0u, 0u, bounce};
-            batch_path(b, path, key.pixel, key.sample);
+            batch_path<LIST>(b, path, key.pixel, key.sample);
             UnifiedWalker<false, NESTED, true, 1> wk;
             int stack_code[FW_STACK];
             float stack_te[FW_STACK];
@@ -79,7 +80,7 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_pass1_k
 // slab arithmetic is monotonic in the box planes), so the leaves are scanned in DFS order — every lane of the warp at the
 // same leaf — and hits are merged by the (t, rank) rule of bvh.rs:120-146, which in rank order is "later wins unless
 // strictly farther".  No stack, no traversal divergence; always with ENTRIES (it only serves the mesh walk).
-template <bool NESTED>
+template <bool NESTED, bool LIST>
 __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_pass1_small_kernel(DeviceScene S, PathState ps, Batch b, uint2 seed,
                                                                                       uint32_t bounce, WalkAux aux) {
     __shared__ uint32_t s_fill[FW_NUM_QUEUES];
@@ -107,7 +108,7 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_pass1_s
                 nan_direction_winner(S.nan_bvh_obj, S.nan_bvh_prim, w);
             } else {
                 RngKey key{seed, 0u, 0u, bounce};
-                if (S.has_medium) batch_path(b, path, key.pixel, key.sample);
+                if (S.has_medium) batch_path<LIST>(b, path, key.pixel, key.sample);
                 const float3 inv = f3(1.0f / d.x, 1.0f / d.y, 1.0f / d.z);
                 float bnd = FW_FLT_MAX;
                 for (int l = 0; l < S.n_top_leaves; ++l) {
@@ -152,7 +153,7 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_pass1_s
     seg_close<FW_NUM_QUEUES>(s_fill, ps, counter_row(ps, bounce, 0), seg);
 }
 
-template <bool NESTED>
+template <bool NESTED, bool LIST>
 __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_pass2_kernel(DeviceScene S, PathState ps, Batch b, uint2 seed,
                                                                                 uint32_t bounce) {
     __shared__ uint32_t s_fill[FW_NUM_QUEUES];
@@ -169,7 +170,7 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_pass2_k
         if (valid) {
             h = get_hit<FW_Q_MESH>(ps, blockIdx.x * ps.seg_cap + e0 + threadIdx.x);
             RngKey key{seed, 0u, 0u, bounce};
-            batch_path(b, h.path, key.pixel, key.sample);
+            batch_path<LIST>(b, h.path, key.pixel, key.sample);
             UnifiedWalker<false, NESTED, true, 2> wk;
             wk.w = h.w;   // the pass-1 winner (a non-mesh object) and its rank
             wk.w.h.b0 = wk.w.h.b1 = wk.w.h.b2 = 0.0f;
@@ -187,7 +188,7 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_pass2_k
     seg_close<MAT_NUM_QUEUES>(s_fill, ps, counter_row(ps, bounce, 0), blockIdx.x);
 }
 
-template <bool NESTED, bool MESHES>
+template <bool NESTED, bool MESHES, bool LIST>
 __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_bvh_simple_kernel(DeviceScene S, PathState ps, Batch b, uint2 seed,
                                                                                      uint32_t bounce) {
 #if FW_SMEM_TOP_NODES > 0
@@ -201,7 +202,7 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_bvh_sim
     FW_EXTEND_PROLOGUE(MAT_NUM_QUEUES)
         if (valid) {
             RngKey key{seed, 0u, 0u, bounce};
-            batch_path(b, path, key.pixel, key.sample);
+            batch_path<LIST>(b, path, key.pixel, key.sample);
             trace_unified<false, NESTED, MESHES>(S, o, d, key, w, nullptr, top);
         }
     FW_EXTEND_EPILOGUE(MAT_NUM_QUEUES)
@@ -211,12 +212,12 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_bvh_sim
 // order, so there is no traversal-length divergence to balance.
 // NESTED: the scene contains a TriangleMesh (its own BVH is walked inside the object test).
 // This object-loop form serves scenes whose LinProgram does not fit kernel-parameter space.
-template <bool NESTED>
+template <bool NESTED, bool LIST>
 __global__ void __launch_bounds__(FW_BLOCK) extend_linear_kernel(DeviceScene S, PathState ps, Batch b, uint2 seed, uint32_t bounce) {
     FW_EXTEND_PROLOGUE(MAT_NUM_QUEUES)
         if (valid) {
             RngKey key{seed, 0u, 0u, bounce};
-            batch_path(b, path, key.pixel, key.sample);
+            batch_path<LIST>(b, path, key.pixel, key.sample);
             trace_linear_scan<false, NESTED>(S, o, d, key, w, nullptr);
         }
     FW_EXTEND_EPILOGUE(MAT_NUM_QUEUES)
@@ -225,73 +226,93 @@ __global__ void __launch_bounds__(FW_BLOCK) extend_linear_kernel(DeviceScene S, 
 // The same query driven by the scene's LinProgram in kernel-parameter space (intersect.cuh trace_linear_prog):
 // no per-lane loads of scene records, uniform item dispatch.  Every lane of a warp runs the program (lanes past
 // the end of the segment trace a dummy ray and drop the result) so that the PRETEST vote sees the whole warp.
-template <bool GENERIC, bool NESTED, bool PRETEST, bool SHDIV>
+template <bool GENERIC, bool NESTED, bool PRETEST, bool SHDIV, bool LIST>
 __global__ void __launch_bounds__(FW_BLOCK) extend_linear_prog_kernel(const __grid_constant__ LinProgram P, DeviceScene S, PathState ps,
                                                                       Batch b, uint2 seed, uint32_t bounce) {
     FW_EXTEND_PROLOGUE(MAT_NUM_QUEUES)
         RngKey key{seed, 0u, 0u, bounce};
-        if (GENERIC) batch_path(b, path, key.pixel, key.sample);
+        if (GENERIC) batch_path<LIST>(b, path, key.pixel, key.sample);
         trace_linear_prog<false, GENERIC, NESTED, PRETEST, SHDIV>(P, S, o, d, key, w, nullptr);
     FW_EXTEND_EPILOGUE(MAT_NUM_QUEUES)
 }
 
 // ---- launchers -------------------------------------------------------------------------------------------
-int launch_extend(const ExtendPlan& plan, bool use_bvh, const LinProgram& P, const DeviceScene& S, const PathState& ps,
-                  const Batch& b, uint2 seed, uint32_t bounce, cudaStream_t st) {
+template <bool LIST>
+static int launch_extend_t(const ExtendPlan& plan, bool use_bvh, const LinProgram& P, const DeviceScene& S, const PathState& ps,
+                           const Batch& b, uint2 seed, uint32_t bounce, cudaStream_t st) {
     const unsigned G = ps.nseg;   // one block per segment
     if (use_bvh && plan.has_top_mesh && plan.two_pass) {
         WalkAux none{};
         if (plan.has_medium_mesh) {
-            extend_pass1_kernel<true, false><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, none);
-            extend_pass2_kernel<true><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
+            extend_pass1_kernel<true, false, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, none);
+            extend_pass2_kernel<true, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
         } else {
-            extend_pass1_kernel<false, false><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, none);
-            extend_pass2_kernel<false><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
+            extend_pass1_kernel<false, false, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, none);
+            extend_pass2_kernel<false, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
         }
         return 2;
     }
     if (use_bvh) {
         if (plan.has_medium_mesh)
-            extend_bvh_simple_kernel<true, true><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
+            extend_bvh_simple_kernel<true, true, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
         else if (plan.has_mesh)
-            extend_bvh_simple_kernel<false, true><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
+            extend_bvh_simple_kernel<false, true, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
         else
-            extend_bvh_simple_kernel<false, false><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
+            extend_bvh_simple_kernel<false, false, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
     } else if (plan.lin_prog_ok) {
         if (plan.lin_generic) {
             if (plan.has_mesh)
-                extend_linear_prog_kernel<true, true, false, false><<<G, FW_BLOCK, 0, st>>>(P, S, ps, b, seed, bounce);
+                extend_linear_prog_kernel<true, true, false, false, LIST><<<G, FW_BLOCK, 0, st>>>(P, S, ps, b, seed, bounce);
             else
-                extend_linear_prog_kernel<true, false, false, false><<<G, FW_BLOCK, 0, st>>>(P, S, ps, b, seed, bounce);
+                extend_linear_prog_kernel<true, false, false, false, LIST><<<G, FW_BLOCK, 0, st>>>(P, S, ps, b, seed, bounce);
         } else if (plan.lin_rect_tests >= 8) {   // rectangle-heavy: shared-reciprocal division (SHDIV)
             // coherent primary rays: whole warps skip Rect3d boxes they do not enter (PRETEST)
-            if (bounce == 0) extend_linear_prog_kernel<false, false, true, true><<<G, FW_BLOCK, 0, st>>>(P, S, ps, b, seed, bounce);
-            else extend_linear_prog_kernel<false, false, false, true><<<G, FW_BLOCK, 0, st>>>(P, S, ps, b, seed, bounce);
+            if (bounce == 0) extend_linear_prog_kernel<false, false, true, true, LIST><<<G, FW_BLOCK, 0, st>>>(P, S, ps, b, seed, bounce);
+            else extend_linear_prog_kernel<false, false, false, true, LIST><<<G, FW_BLOCK, 0, st>>>(P, S, ps, b, seed, bounce);
         } else {
-            extend_linear_prog_kernel<false, false, false, false><<<G, FW_BLOCK, 0, st>>>(P, S, ps, b, seed, bounce);
+            extend_linear_prog_kernel<false, false, false, false, LIST><<<G, FW_BLOCK, 0, st>>>(P, S, ps, b, seed, bounce);
         }
     } else if (plan.has_mesh) {
-        extend_linear_kernel<true><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
+        extend_linear_kernel<true, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
     } else {
-        extend_linear_kernel<false><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
+        extend_linear_kernel<false, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
     }
     return 1;
 }
-void launch_extend_pass1_entries(bool small_top, bool nested, const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed, uint32_t bounce,
-                                 const WalkAuxHost& ax, cudaStream_t st) {
+template <bool LIST>
+static void launch_extend_pass1_entries_t(bool small_top, bool nested, const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed,
+                                          uint32_t bounce, const WalkAuxHost& ax, cudaStream_t st) {
     WalkAux aux;
     aux.tkey = ax.tkey; aux.entries = reinterpret_cast<uint4*>(ax.entries); aux.ent_cap = ax.ent_cap; aux.prim_bits = ax.prim_bits;
     if (small_top) {
-        if (nested) extend_pass1_small_kernel<true><<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, aux);
-        else extend_pass1_small_kernel<false><<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, aux);
+        if (nested) extend_pass1_small_kernel<true, LIST><<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, aux);
+        else extend_pass1_small_kernel<false, LIST><<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, aux);
         return;
     }
-    if (nested) extend_pass1_kernel<true, true><<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, aux);
-    else extend_pass1_kernel<false, true><<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, aux);
+    if (nested) extend_pass1_kernel<true, true, LIST><<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, aux);
+    else extend_pass1_kernel<false, true, LIST><<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, aux);
+}
+template <bool LIST>
+static void launch_extend_debug_t(const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed, uint32_t bounce, uint32_t* steps,
+                                  cudaStream_t st) {
+    extend_bvh_debug_kernel<LIST><<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, steps);
+}
+
+// Batches over a pixel list (b.pixels set: adaptive rounds) run the LIST instantiations.
+int launch_extend(const ExtendPlan& plan, bool use_bvh, const LinProgram& P, const DeviceScene& S, const PathState& ps,
+                  const Batch& b, uint2 seed, uint32_t bounce, cudaStream_t st) {
+    return b.pixels ? launch_extend_t<true>(plan, use_bvh, P, S, ps, b, seed, bounce, st)
+                    : launch_extend_t<false>(plan, use_bvh, P, S, ps, b, seed, bounce, st);
+}
+void launch_extend_pass1_entries(bool small_top, bool nested, const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed, uint32_t bounce,
+                                 const WalkAuxHost& ax, cudaStream_t st) {
+    if (b.pixels) launch_extend_pass1_entries_t<true>(small_top, nested, S, ps, b, seed, bounce, ax, st);
+    else launch_extend_pass1_entries_t<false>(small_top, nested, S, ps, b, seed, bounce, ax, st);
 }
 void launch_extend_debug(const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed, uint32_t bounce, uint32_t* steps,
                          cudaStream_t st) {
-    extend_bvh_debug_kernel<<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, steps);
+    if (b.pixels) launch_extend_debug_t<true>(S, ps, b, seed, bounce, steps, st);
+    else launch_extend_debug_t<false>(S, ps, b, seed, bounce, steps, st);
 }
 
 }  // namespace fw

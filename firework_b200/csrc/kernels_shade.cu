@@ -7,6 +7,7 @@ namespace fw {
 // One block per segment.  Tile t (FW_TILE consecutive paths) belongs to segment t % nseg, so every segment gets an
 // even mix of the image; entry e of segment `seg` is path ((e / TILE) * nseg + seg) * TILE + e % TILE.  The rays
 // go straight into the segment's bounce-0 extend queue.
+template <bool LIST>
 __global__ void __launch_bounds__(FW_BLOCK) raygen_kernel(CameraRec cam, Batch b, uint2 seed, PathState ps) {
     const uint32_t total = b.npix * b.ns;
     const uint32_t seg = blockIdx.x;
@@ -16,7 +17,7 @@ __global__ void __launch_bounds__(FW_BLOCK) raygen_kernel(CameraRec cam, Batch b
         uint32_t p = ((e / FW_TILE) * ps.nseg + seg) * FW_TILE + (e % FW_TILE);
         if (p >= total) break;   // p grows with e: the valid entries are a prefix
         uint32_t pixel, sample;
-        batch_path(b, p, pixel, sample);
+        batch_path<LIST>(b, p, pixel, sample);
         float3 o, d;
         uint32_t row, px;
         div_magic(pixel, b.width, b.width_magic, row, px);
@@ -96,7 +97,7 @@ __global__ void __launch_bounds__(FW_BLOCK) shade_emissive_kernel(DeviceScene S,
 // Not launched for bounce == FW_MAX_DEPTH (render.rs:21: no scatter at depth 10; emit is zero).
 // The material kernels of one bounce run back to back and append to the same regions of the next extend queue.
 // The entries of material MAT's queue of one segment; s_fill[0] is the segment's open fill count of the next extend queue.
-template <int MAT>
+template <int MAT, bool LIST>
 FW_DEV void scatter_segment(const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed, uint32_t bounce, uint32_t seg, uint32_t total,
                             uint32_t* s_fill) {
     const uint32_t base = seg * ps.seg_cap;
@@ -122,7 +123,7 @@ FW_DEV void scatter_segment(const DeviceScene& S, const PathState& ps, const Bat
             finalize_hit(S, h.w, h.o, h.d, rec, __float_as_int(m0.w) != 0);
             float3 point = rec.point, normal = rec.normal;
             uint32_t pixel, sample;
-            batch_path(b, path, pixel, sample);
+            batch_path<LIST>(b, path, pixel, sample);
             RngKey key{seed, pixel, sample, bounce};
             PhiloxStream rng(key, STREAM_SCATTER);
             if (MAT == MAT_LAMBERTIAN) {
@@ -150,7 +151,7 @@ FW_DEV void scatter_segment(const DeviceScene& S, const PathState& ps, const Bat
         }
     }
 }
-template <int MAT>
+template <int MAT, bool LIST>
 __global__ void __launch_bounds__(FW_BLOCK, FW_SHADE_MIN_BLOCKS) shade_scatter_kernel(DeviceScene S, PathState ps, Batch b, uint2 seed, uint32_t bounce) {
     __shared__ uint32_t s_fill[1];
     const uint32_t seg = blockIdx.x;
@@ -158,7 +159,7 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_SHADE_MIN_BLOCKS) shade_scatter_k
     if (total == 0) return;  // block-uniform
     uint32_t* row_out = counter_row(ps, bounce + 1, FW_Q_EXTEND);
     seg_open<1>(s_fill, ps, row_out, seg);
-    scatter_segment<MAT>(S, ps, b, seed, bounce, seg, total, s_fill);
+    scatter_segment<MAT, LIST>(S, ps, b, seed, bounce, seg, total, s_fill);
     seg_close<1>(s_fill, ps, row_out, seg);
 }
 
@@ -193,15 +194,7 @@ __global__ void __launch_bounds__(256) accumulate_kernel(float* __restrict__ sum
     }
 }
 
-// render.rs:184-189 + util.rs:14-23: mean, powf(1/gamma), clamp, *255.99 -> saturating u8 (NaN -> 0)
-FW_DEV unsigned char quantise(float mean, float inv_gamma) {
-    float x = powf(mean, inv_gamma);
-    if (x < 0.0f) x = 0.0f;
-    if (x > 1.0f) x = 1.0f;
-    float y = x * 255.99f;
-    if (!(y == y)) return 0;
-    return (unsigned char)fminf(fmaxf(truncf(y), 0.0f), 255.0f);
-}
+// quantise (wavefront.cuh): render.rs:184-189 + util.rs:14-23
 __global__ void __launch_bounds__(256) resolve_kernel(const float* __restrict__ sum, uint32_t npix, float samples,
                                                       float gamma, unsigned char* __restrict__ rgb) {
     float inv_gamma = 1.0f / gamma;
@@ -214,7 +207,8 @@ __global__ void __launch_bounds__(256) resolve_kernel(const float* __restrict__ 
 
 // ---- launchers -------------------------------------------------------------------------------------------
 void launch_raygen(const CameraRec& cam, const Batch& b, uint2 seed, const PathState& ps, cudaStream_t st) {
-    raygen_kernel<<<ps.nseg, FW_BLOCK, 0, st>>>(cam, b, seed, ps);
+    if (b.pixels) raygen_kernel<true><<<ps.nseg, FW_BLOCK, 0, st>>>(cam, b, seed, ps);   // a pixel list (adaptive rounds)
+    else raygen_kernel<false><<<ps.nseg, FW_BLOCK, 0, st>>>(cam, b, seed, ps);
 }
 void launch_miss(const DeviceScene& S, const PathState& ps, uint32_t bounce, bool black_env, cudaStream_t st) {
     if (black_env) miss_kernel<true><<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, bounce);
@@ -223,16 +217,22 @@ void launch_miss(const DeviceScene& S, const PathState& ps, uint32_t bounce, boo
 void launch_shade_emissive(const DeviceScene& S, const PathState& ps, uint32_t bounce, cudaStream_t st) {
     shade_emissive_kernel<<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, bounce);
 }
-void launch_shade_scatter(int mat, const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed, uint32_t bounce,
-                          cudaStream_t st) {
+template <bool LIST>
+static void launch_shade_scatter_t(int mat, const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed, uint32_t bounce,
+                                   cudaStream_t st) {
     const unsigned G = ps.nseg;
     switch (mat) {
-        case MAT_LAMBERTIAN: shade_scatter_kernel<MAT_LAMBERTIAN><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce); break;
-        case MAT_METAL: shade_scatter_kernel<MAT_METAL><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce); break;
-        case MAT_DIELECTRIC: shade_scatter_kernel<MAT_DIELECTRIC><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce); break;
-        case MAT_ISOTROPIC: shade_scatter_kernel<MAT_ISOTROPIC><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce); break;
+        case MAT_LAMBERTIAN: shade_scatter_kernel<MAT_LAMBERTIAN, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce); break;
+        case MAT_METAL: shade_scatter_kernel<MAT_METAL, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce); break;
+        case MAT_DIELECTRIC: shade_scatter_kernel<MAT_DIELECTRIC, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce); break;
+        case MAT_ISOTROPIC: shade_scatter_kernel<MAT_ISOTROPIC, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce); break;
         default: break;
     }
+}
+void launch_shade_scatter(int mat, const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed, uint32_t bounce,
+                          cudaStream_t st) {
+    if (b.pixels) launch_shade_scatter_t<true>(mat, S, ps, b, seed, bounce, st);
+    else launch_shade_scatter_t<false>(mat, S, ps, b, seed, bounce, st);
 }
 void launch_accumulate(float* d_sum, const PathState& ps, const Batch& b, unsigned blocks, cudaStream_t st) {
     accumulate_kernel<<<blocks, 256, 0, st>>>(d_sum, ps, b);

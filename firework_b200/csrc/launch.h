@@ -54,6 +54,26 @@ void launch_tally(const PathState& ps, unsigned long long* d_rays, cudaStream_t 
 void launch_resolve(const float* d_sum, uint32_t npix, float samples, float gamma, unsigned char* d_rgb, unsigned blocks,
                     cudaStream_t st);
 
+// Per-pixel state of an adaptive render (kernels_adaptive.cu), in the render context next to d_sum.
+struct AdaptiveState {
+    double* m1 = nullptr;           // [npix] sum of the samples' luminance
+    double* m2 = nullptr;           // [npix] sum of its squares
+    uint32_t* count = nullptr;      // [npix] samples rendered
+    float* err = nullptr;           // [npix] final relative error (written by the resolve)
+    uint32_t* list[2] = {nullptr, nullptr};   // active pixel lists, ascending (ping-pong between rounds)
+    uint8_t* keep = nullptr;        // [npix] by list position: the pixel goes on to the next round
+    uint32_t* block_base = nullptr; // [adaptive_blocks(npix) + 1] compaction block counts -> bases; [nb] = survivors
+};
+uint32_t adaptive_blocks(uint32_t n);   // compaction blocks of a list of n entries
+void launch_accumulate_adaptive(float* d_sum, const AdaptiveState& a, const PathState& ps, const Batch& b, unsigned blocks, cudaStream_t st);
+void launch_adaptive_init(uint32_t* list, uint32_t n, unsigned blocks, cudaStream_t st);   // list = 0, 1, ..., n - 1
+// Stop rule over list_in[0, n), survivors to list_out in the same order, their number to a.block_base[adaptive_blocks(n)].
+// Returns the number of kernels launched.
+int launch_converge_compact(const AdaptiveState& a, const uint32_t* list_in, uint32_t n, double threshold, double floor, uint32_t* list_out,
+                            cudaStream_t st);
+void launch_resolve_adaptive(const float* d_sum, const AdaptiveState& a, uint32_t npix, float gamma, double floor, unsigned char* d_rgb,
+                             unsigned blocks, cudaStream_t st);
+
 // probes (tests/ parity gates)
 void launch_primary_rays_probe(const CameraRec& cam, uint32_t width, uint32_t height, uint32_t sample, uint2 seed,
                                uint32_t pix_begin, uint32_t n, float* origins, float* dirs, unsigned blocks, cudaStream_t st);

@@ -42,13 +42,26 @@ FW_DEV uint32_t* counter_row(const PathState& ps, uint32_t row, int queue) {
 }
 // pixel = pix0 + p % npix, sample = s0 + p / npix.  q = umulhi(p, ceil(2^32 / npix)) is floor(p / npix) or one more
 // (one less for npix == 1); one correction step makes it exact for every 32-bit p.
+// LIST (adaptive rounds): pix0 / npix index the pixel list b.pixels instead of the image.  A template parameter rather than
+// a run-time branch on b.pixels: the branch costs the shade and two-pass extend kernels 4-12 bytes of extra spills.
+template <bool LIST>
 FW_DEV void batch_path(const Batch& b, uint32_t p, uint32_t& pixel, uint32_t& sample) {
     uint32_t q = __umulhi(p, b.npix_magic);
     int r = (int)(p - q * b.npix);
     if (r < 0) { q -= 1u; r += (int)b.npix; }
     else if (r >= (int)b.npix) { q += 1u; r -= (int)b.npix; }
     pixel = b.pix0 + (uint32_t)r;
+    if (LIST) pixel = __ldg(&b.pixels[pixel]);
     sample = b.s0 + q;
+}
+// render.rs:184-189 + util.rs:14-23: mean, powf(1/gamma), clamp, *255.99 -> saturating u8 (NaN -> 0)
+FW_DEV unsigned char quantise(float mean, float inv_gamma) {
+    float x = powf(mean, inv_gamma);
+    if (x < 0.0f) x = 0.0f;
+    if (x > 1.0f) x = 1.0f;
+    float y = x * 255.99f;
+    if (!(y == y)) return 0;
+    return (unsigned char)fminf(fmaxf(truncf(y), 0.0f), 255.0f);
 }
 
 // render.rs:173-180 + camera.rs:109-116 + util.rs:31-33

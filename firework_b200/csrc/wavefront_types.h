@@ -42,6 +42,7 @@ struct Batch {
     uint32_t width, height;
     uint32_t npix_magic;   // ceil(2^32 / npix) (0xffffffff for npix == 1): p / npix without the emulated 32-bit division
     uint32_t width_magic;  // the same for `width` (pixel -> column / row in raygen)
+    const uint32_t* pixels;   // null: pixel = pix0 + p % npix.  Else a pixel list (adaptive rounds): pixel = pixels[pix0 + p % npix]
 };
 
 struct FirstHitOut {

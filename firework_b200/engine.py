@@ -13,6 +13,12 @@ import numpy as np
 from . import _native as N
 from .assets import load_asset
 
+# Default luminance floor of the adaptive stop rule's denominator, max(|mean|, floor).  Below it the rule asks for an absolute
+# standard error of threshold * floor instead of a relative one: at 0.01 (linear; u8 31 after gamma 2.2) and threshold 0.05
+# that is 5e-4, under one u8 level after the gamma curve, so black and near-black pixels (shadows, an unlit background)
+# stop instead of chasing a relative error their displayed value can not show.
+ADAPTIVE_FLOOR = 0.01
+
 
 class NativeScene:
     """A committed fw_scene on one GPU."""
@@ -131,6 +137,27 @@ class NativeScene:
         N.check(N.lib().fw_render(self._h, C.byref(params), N.ptr(rgb) if want_rgb else None,
                                   N.ptr(s) if want_sum else None, C.byref(st)))
         return rgb, s, st.as_dict()
+
+    def render_adaptive(self, params: N.FwParams, threshold: float, min_samples: int = 16, floor: float = ADAPTIVE_FLOOR,
+                        want_rgb=True, want_sum=True):
+        """fw_render_adaptive: every pixel renders until its relative standard error is <= `threshold`, with
+        `params.samples` as the cap (params must cover the whole range: sample_begin 0, sample_count == samples).
+        Returns (rgb (H,W,3) u8 | None, sum (H,W,3) f32 | None, counts (H,W) u32, err (H,W) f32, stats dict); stats adds
+        `rounds` and `active` (pixels rendered in each round) to the fw_stats fields, and stats["samples"] is the sum of
+        the counts."""
+        h, w = params.height, params.width
+        rgb = np.empty((h, w, 3), np.uint8) if want_rgb else None
+        s = np.empty((h, w, 3), np.float32) if want_sum else None
+        counts = np.empty((h, w), np.uint32)
+        err = np.empty((h, w), np.float32)
+        ad = N.FwAdaptive(int(min_samples), float(threshold), float(floor))
+        st, res = N.FwStats(), N.FwAdaptiveResult()
+        N.check(N.lib().fw_render_adaptive(self._h, C.byref(params), C.byref(ad), N.ptr(rgb) if want_rgb else None,
+                                           N.ptr(s) if want_sum else None, N.ptr(counts), N.ptr(err), C.byref(st), C.byref(res)))
+        d = st.as_dict()
+        d["rounds"] = int(res.rounds)
+        d["active"] = [int(res.active[r]) for r in range(min(res.rounds, 32))]
+        return rgb, s, counts, err, d
 
     def render_multi(self, params: N.FwParams, n_gpus: int, devices=None, reduce="nccl", want_rgb=True, want_sum=True):
         """fw_render_multi: the call's sample range split over `n_gpus` devices of this box (single process), sums

@@ -484,6 +484,12 @@ public:
     Renderer seed(uint64_t s) const { Renderer c = *this; c.seed_ = s; return c; }
     Renderer gpus(int n) const { Renderer c = *this; c.gpus_ = n; return c; }
     Renderer asset_dir(std::string d) const { Renderer c = *this; c.asset_dir_ = std::move(d); return c; }
+    // adaptive sampling (fw_render_adaptive): samples_ becomes the cap per pixel, each pixel renders until its relative standard
+    // error is <= threshold; floor 0.01 as the Python mirror's Renderer.adaptive (engine.ADAPTIVE_FLOOR).  threshold < 0: off.
+    // Single GPU: together with gpus(n > 1) render() throws.
+    Renderer adaptive(float threshold, uint32_t min_samples = 16, float floor = 0.01f) const {
+        Renderer c = *this; c.threshold_ = threshold; c.min_samples_ = min_samples; c.floor_ = floor; return c;
+    }
 
     fw_params params() const {
         fw_params p;
@@ -525,8 +531,16 @@ public:
         detail::check(fw_scene_commit(h, 0), "commit");
         const fw_params p = params();
         std::vector<uint8_t> rgb(width_ * height_ * 3);
-        if (gpus_ > 1) detail::check(fw_render_multi(h, &p, gpus_, nullptr, FW_REDUCE_NCCL, rgb.data(), nullptr, nullptr, nullptr), "render");
-        else detail::check(fw_render(h, &p, rgb.data(), nullptr, nullptr), "render");
+        if (threshold_ >= 0.0f) {
+            if (gpus_ > 1) throw Error("adaptive sampling renders on one GPU: gpus(n > 1) and adaptive() can not be combined");
+            fw_adaptive ad;
+            ad.min_samples = min_samples_; ad.threshold = threshold_; ad.floor = floor_;
+            detail::check(fw_render_adaptive(h, &p, &ad, rgb.data(), nullptr, nullptr, nullptr, nullptr, nullptr), "render");
+        } else if (gpus_ > 1) {
+            detail::check(fw_render_multi(h, &p, gpus_, nullptr, FW_REDUCE_NCCL, rgb.data(), nullptr, nullptr, nullptr), "render");
+        } else {
+            detail::check(fw_render(h, &p, rgb.data(), nullptr, nullptr), "render");
+        }
         std::vector<Color> out(width_ * height_);
         for (size_t i = 0; i < out.size(); ++i) out[i] = Color{rgb[3 * i], rgb[3 * i + 1], rgb[3 * i + 2]};
         return out;
@@ -545,6 +559,8 @@ private:
     CameraSettings camera_;
     uint64_t seed_ = 0;
     int gpus_ = 1;
+    float threshold_ = -1.0f, floor_ = 0.01f;
+    uint32_t min_samples_ = 16;
     std::string asset_dir_ = ".";
 };
 

@@ -109,6 +109,35 @@ int fw_scene_walk_info(const fw_scene* scene, int out[6]);
  * Host buffers; the call is synchronous.                                                                */
 int fw_render(fw_scene* scene, const fw_params* params, uint8_t* rgb_out, float* sum_out, fw_stats* stats);
 
+/* ---- adaptive sampling (no reference counterpart) -------------------------------------------------------
+ * Renders each pixel until its noise estimate meets a target, with params->samples as the cap per pixel.  The call owns
+ * the sample range: sample_begin must be 0 and sample_count == samples (else FW_ERR_ARG).  Single GPU.
+ * Schedule: round 0 renders samples [0, n0), n0 = min(min_samples, samples), of every pixel; a pixel that does not stop
+ *   after round r renders [n_r, n_{r+1}), n_{r+1} = min(2 n_r, samples), in round r + 1.  The render ends when no pixel is
+ *   active or n_r == samples.
+ * Stop rule (fp64, in this order): per sample Y = (0.2126 r + 0.7152 g) + 0.0722 b of the fp32 radiance; per pixel in
+ *   sample order A = sum Y, B = sum Y^2; after n samples mean = A / n, var = max(0, (B - A mean) / (n - 1)),
+ *   err = sqrt(var / n) / max(|mean|, floor), both maxima propagating NaN.  A pixel stops when n >= 2 and err <= threshold;
+ *   a NaN error (NaN radiance; n = 1) never stops a pixel.
+ * Exactness: a pixel that received k samples has the fp32 sum, bit for bit, and the u8 value of fw_render at samples = k.
+ * Outputs (each nullable, width*height entries, row 0 = top): rgb_out u8 x3 = quantise(sum / (float)count); sum_out fp32 x3
+ *   un-normalised sums; count_out samples per pixel; error_out the final err of each pixel.  stats->samples = sum of the
+ *   counts; rays / launches / ms_device cover the whole call.  result->active[r] = pixels rendered in round r (r < 32).
+ * Argument errors (null scene / params / adaptive, min_samples == 0, threshold negative or not finite, floor not > 0 or not
+ * finite, the sample range) are reported before any CUDA call; an uncommitted scene gives FW_ERR_STATE. */
+typedef struct fw_adaptive {
+    uint32_t min_samples;   /* samples every pixel gets in round 0 (>= 1)                                 */
+    float threshold;        /* stop a pixel when its relative standard error <= threshold (>= 0, finite) */
+    float floor;            /* luminance floor of the relative error's denominator (> 0, finite)         */
+} fw_adaptive;
+typedef struct fw_adaptive_result {
+    uint32_t rounds;
+    uint64_t samples;       /* sum of the per-pixel counts */
+    uint32_t active[32];    /* pixels rendered in round r  */
+} fw_adaptive_result;
+int fw_render_adaptive(fw_scene* scene, const fw_params* params, const fw_adaptive* adaptive, uint8_t* rgb_out, float* sum_out,
+                       uint32_t* count_out, float* error_out, fw_stats* stats, fw_adaptive_result* result);
+
 /* Device-resident variant for multi-GPU sharding: ADDS the sample range into d_sum (device pointer,
  * width*height*3 fp32, on the scene's device) on `cuda_stream` (a cudaStream_t, or NULL for the scene's own
  * stream) and returns once the work is enqueued and statistics are read back. */
