@@ -709,7 +709,6 @@ static int commit_uploads(fw_scene* sc) {
         }
         for (const MatRec& m : F.mats)
             if (m.kind == MAT_METAL && !(small(m.albedo[0]) && small(m.albedo[1]) && small(m.albedo[2]))) ok = false;
-        if (const char* e = getenv("FW_SKIP_ZERO_MISS")) ok = ok && atoi(e) != 0;
         sc->miss_is_zero = ok;
         sc->env_black = sc->desc.env_kind == ENV_COLOR && sc->desc.env_a[0] == 0.0f && sc->desc.env_a[1] == 0.0f && sc->desc.env_a[2] == 0.0f;
         if (const char* e = getenv("FW_BLACK_ENV_SKIP")) sc->env_black = sc->env_black && atoi(e) != 0;
@@ -721,9 +720,7 @@ static int commit_uploads(fw_scene* sc) {
     sc->plan.has_mesh = F.has_mesh; sc->plan.has_top_mesh = F.has_top_mesh; sc->plan.has_medium_mesh = F.has_medium_mesh;
     sc->plan.lin_prog_ok = sc->lin_prog_ok; sc->plan.lin_generic = F.lin_generic; sc->plan.lin_rect_tests = F.lin_rect_tests;
     sc->plan.small_top = F.top_leaves.size() / 2 <= 16;   // few top-level leaves: scanned straight through (pass 1 of the mesh walk)
-    if (const char* e = getenv("FW_SMALL_TOP")) sc->plan.small_top = sc->plan.small_top && atoi(e) != 0;
     sc->plan.walk = F.walk_ok && F.has_top_mesh;   // mesh walk kernels (sphere-only trees stay on the lock-step kernel)
-    if (const char* e = getenv("FW_WALK")) sc->plan.walk = sc->plan.walk && atoi(e) != 0;
     // uploads ran on the context's stream; renders may be issued on another one (fw_render_accumulate_device)
     FW_CUDA(cudaStreamSynchronize(sc->ctx->stream));
     sc->committed = true;
@@ -852,11 +849,10 @@ int fw_set_batch_paths(fw_scene* sc, uint64_t paths) {
 #ifndef FW_DEFAULT_BATCH_PATHS
 #define FW_DEFAULT_BATCH_PATHS (1ull << 27)
 #endif
-static constexpr uint32_t FW_SEG_PER_SM_MAX = 64;
+static constexpr uint32_t FW_SEG_PER_SM_MAX = 32;   // measured: sm x 32 (segment-count sweep, profiles/r01_extend_variants.md)
 static void segment_geometry(const fw_scene* sc, size_t n, uint32_t* nseg, uint32_t* seg_cap) {
     size_t tiles = (n + FW_TILE - 1) / FW_TILE;
-    size_t want = std::max<size_t>((size_t)sc->sm_count, std::min<size_t>((size_t)sc->sm_count * 32, tiles / 8));  // measured: sm x 32 (FW_SEGMENTS sweep, profiles/r01e)
-    if (const char* e = getenv("FW_SEGMENTS")) want = std::max<size_t>(1, std::min<size_t>((size_t)sc->sm_count * FW_SEG_PER_SM_MAX, strtoull(e, nullptr, 10)));
+    size_t want = std::max<size_t>((size_t)sc->sm_count, std::min<size_t>((size_t)sc->sm_count * FW_SEG_PER_SM_MAX, tiles / 8));
     *nseg = (uint32_t)want;
     *seg_cap = (uint32_t)(((tiles + want - 1) / want) * FW_TILE);
 }
@@ -943,70 +939,35 @@ unsigned fw::grid_for(size_t n, unsigned threads, unsigned max_blocks) {
     return (unsigned)std::max<size_t>(1, std::min<size_t>(g, max_blocks));
 }
 
-// FW_DEBUG_STEPS=1: per-path box-test counts of one bounce, worst path printed to stderr (FW_DEBUG_DUMP: per-bounce dump).
-static int debug_extend(fw_scene* sc, const Batch& b, uint2 seed, uint32_t bounce, cudaStream_t st) {
-    PathState& ps = sc->ctx->ps;
-    const DeviceScene& S = sc->dscene;
-    const uint32_t N = b.npix * b.ns;
-    // debug: per-path box-test counts, worst path of every bounce printed to stderr
-    static uint32_t* d_steps = nullptr;
-    static size_t d_steps_cap = 0;
-    if (d_steps_cap < ps.cap) {
-        if (d_steps) cudaFree(d_steps);
-        FW_CUDA(cudaMalloc(&d_steps, (size_t)ps.cap * 4));
-        d_steps_cap = ps.cap;
+// FW_DEBUG_SYNC=1: synchronise after every kernel stage and name the one that faulted (debugging aid; slow).
+static int sync_stage(cudaStream_t st, const char* what, uint32_t bounce) {
+    static const bool debug_sync = getenv("FW_DEBUG_SYNC") != nullptr;
+    if (!debug_sync) return FW_OK;
+    cudaError_t e = cudaStreamSynchronize(st);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e != cudaSuccess)
+        return set_error(FW_ERR_CUDA, std::string(what) + " (bounce " + std::to_string(bounce) + "): " + cudaGetErrorString(e));
+    return FW_OK;
+}
+#define FW_STAGE(what, bounce) do { int rc__ = sync_stage(st, what, bounce); if (rc__ != FW_OK) return rc__; } while (0)
+
+// The extend of one bounce, chosen from the scene alone: the collect / test mesh walk where the plan allows it, else the
+// lock-step or linear-scan kernels of launch_extend.  Renders and fw_first_hit_wavefront both come here, so the probe runs
+// exactly the kernels a render runs.  Adds the number of kernels launched to `launches`.
+static int extend_bounce(fw_scene* sc, bool use_bvh, const Batch& b, uint2 seed, uint32_t bounce, cudaStream_t st, uint64_t& launches) {
+    const PathState& ps = sc->ctx->ps;
+    if (!(use_bvh && sc->plan.walk)) {
+        launches += launch_extend(sc->plan, use_bvh, sc->lin_prog, sc->dscene, ps, b, seed, bounce, st);
+        return FW_OK;
     }
-    FW_CUDA(cudaMemsetAsync(d_steps, 0xff, (size_t)ps.cap * 4, st));   // 0xffffffff = path not traced this bounce
-    launch_extend_debug(S, ps, b, seed, bounce, d_steps, st);
-    FW_CUDA(cudaStreamSynchronize(st));
-    std::vector<uint32_t> hs(N);
-    FW_CUDA(cudaMemcpy(hs.data(), d_steps, (size_t)N * 4, cudaMemcpyDeviceToHost));
-    size_t worst = 0;
-    unsigned long long sum = 0;
-    bool any = false;
-    for (size_t i = 0; i < N; ++i) {
-        if (hs[i] == 0xffffffffu) continue;
-        sum += hs[i];
-        if (!any || hs[i] > hs[worst]) { worst = i; any = true; }
+    WalkAuxHost ax = sc->ctx->walk;
+    ax.ent_cap = ps.seg_cap * (uint32_t)std::max(1, sc->flat.n_top_meshes);
+    static const char* const part_name[3] = {"extend pass 1 (entries)", "mesh walk", "mesh classify"};
+    for (int part = 0; part < 3; ++part) {
+        launch_extend_walk_part(part, sc->plan, sc->dscene, ps, b, seed, bounce, ax, st);
+        launches++;
+        FW_STAGE(part_name[part], bounce);
     }
-    // the segments' extend-queue records of this bounce: (o, path), (d, -)
-    std::vector<float4> qo, qd;
-    {
-        std::vector<uint32_t> cnts(ps.nseg);
-        FW_CUDA(cudaMemcpy(cnts.data(), ps.counters + ((size_t)bounce * FW_NUM_QUEUES + FW_Q_EXTEND) * ps.nseg,
-                           (size_t)ps.nseg * 4, cudaMemcpyDeviceToHost));
-        for (uint32_t seg = 0; seg < ps.nseg; ++seg) {
-            if (!cnts[seg]) continue;
-            size_t at = qo.size();
-            qo.resize(at + cnts[seg]); qd.resize(at + cnts[seg]);
-            FW_CUDA(cudaMemcpy(qo.data() + at, ps.xo[bounce & 1] + (size_t)seg * ps.seg_cap, (size_t)cnts[seg] * 16, cudaMemcpyDeviceToHost));
-            FW_CUDA(cudaMemcpy(qd.data() + at, ps.xd[bounce & 1] + (size_t)seg * ps.seg_cap, (size_t)cnts[seg] * 16, cudaMemcpyDeviceToHost));
-        }
-    }
-    float4 ro = make_float4(0, 0, 0, 0), rd = ro;
-    for (size_t i = 0; i < qo.size(); ++i) {
-        uint32_t pth;
-        memcpy(&pth, &qo[i].w, 4);
-        if (pth == worst) { ro = qo[i]; rd = qd[i]; }
-    }
-    if (const char* dump = getenv("FW_DEBUG_DUMP")) {
-        // per-bounce dump for offline coherence analysis: queue order, per-path box tests, rays
-        uint32_t cnt = (uint32_t)qo.size();
-        std::string fn = std::string(dump) + "_b" + std::to_string(bounce) + ".bin";
-        FILE* f = fopen(fn.c_str(), "wb");
-        if (f) {
-            fwrite(&cnt, 4, 1, f);
-            for (uint32_t i = 0; i < cnt; ++i) {
-                uint32_t pth;
-                memcpy(&pth, &qo[i].w, 4);
-                float rec[8] = {qo[i].x, qo[i].y, qo[i].z, qd[i].x, qd[i].y, qd[i].z, (float)hs[pth], (float)pth};
-                fwrite(rec, 4, 8, f);
-            }
-            fclose(f);
-        }
-    }
-    fprintf(stderr, "[fw debug] bounce %u: box tests total %llu, worst path %zu (pixel %zu sample %zu): %u tests, o=(%.9g %.9g %.9g) d=(%.9g %.9g %.9g)\n",
-            bounce, sum, worst, (size_t)b.pix0 + worst % b.npix, (size_t)b.s0 + worst / b.npix, any ? hs[worst] : 0u, ro.x, ro.y, ro.z, rd.x, rd.y, rd.z);
     return FW_OK;
 }
 
@@ -1022,17 +983,6 @@ static int run_batch(fw_scene* sc, const CameraRec& cam, const Batch& b, uint2 s
     FW_CUDA(cudaMemsetAsync(ps.counters, 0, counter_bytes, st));
     FW_CUDA(cudaMemsetAsync(ps.poison, 0, sizeof(uint32_t), st));
     unsigned sm = (unsigned)sc->sm_count;
-    // FW_DEBUG_SYNC=1: synchronise after every stage and name the one that faulted (debugging aid; slow)
-    static const bool debug_sync = getenv("FW_DEBUG_SYNC") != nullptr;
-    auto stage = [&](const char* what, uint32_t bounce) -> int {
-        if (!debug_sync) return FW_OK;
-        cudaError_t e = cudaStreamSynchronize(st);
-        if (e == cudaSuccess) e = cudaGetLastError();
-        if (e != cudaSuccess)
-            return set_error(FW_ERR_CUDA, std::string(what) + " (bounce " + std::to_string(bounce) + "): " + cudaGetErrorString(e));
-        return FW_OK;
-    };
-#define FW_STAGE(what, bounce) do { int rc__ = stage(what, bounce); if (rc__ != FW_OK) return rc__; } while (0)
     launch_raygen(cam, b, seed, ps, st);
     tot.launches++;
     FW_STAGE("raygen", 0);
@@ -1043,27 +993,8 @@ static int run_batch(fw_scene* sc, const CameraRec& cam, const Batch& b, uint2 s
             if ((rc = get_event(sc, ev_next, &e0)) != FW_OK || (rc = get_event(sc, ev_next, &e1)) != FW_OK) return rc;
             FW_CUDA(cudaEventRecord(e0, st));
         }
-        if (use_bvh && getenv("FW_DEBUG_STEPS")) {
-            int rc = debug_extend(sc, b, seed, bounce, st);
-            if (rc != FW_OK) return rc;
-            tot.launches++;
-        } else {
-            if (use_bvh && sc->plan.walk && sc->plan.two_pass) {
-                WalkAuxHost ax = sc->ctx->walk;
-                ax.ent_cap = ps.seg_cap * (uint32_t)std::max(1, sc->flat.n_top_meshes);
-                if (debug_sync) {
-                    for (int part = 0; part < 3; ++part) {
-                        launch_extend_walk_part(part, sc->plan, S, ps, b, seed, bounce, ax, st);
-                        FW_STAGE(part == 0 ? "extend pass 1 (entries)" : part == 1 ? "mesh walk" : "mesh classify", bounce);
-                    }
-                    tot.launches += 3;
-                } else {
-                    tot.launches += launch_extend_walk(sc->plan, S, ps, b, seed, bounce, ax, st);
-                }
-            } else {
-                tot.launches += launch_extend(sc->plan, use_bvh, sc->lin_prog, S, ps, b, seed, bounce, st);
-            }
-        }
+        const int rc = extend_bounce(sc, use_bvh, b, seed, bounce, st, tot.launches);
+        if (rc != FW_OK) return rc;
         if (sc->profiling) {
             FW_CUDA(cudaEventRecord(e1, st));
             tot.extend_events.emplace_back(e0, e1);
@@ -1109,7 +1040,6 @@ static int prepare_batches(fw_scene* sc, size_t paths, size_t* cap_out) {
     // (five material queues) -> 66 GB at 128 Mi paths, laid out for the 180 GB of HBM3e of a B200.
     size_t cap = sc->batch_paths ? sc->batch_paths : ((size_t)FW_DEFAULT_BATCH_PATHS);
     if (const char* e = getenv("FW_BATCH_PATHS")) cap = std::max<size_t>(1024, strtoull(e, nullptr, 10));
-    if (const char* e = getenv("FW_TWO_PASS")) sc->plan.two_pass = atoi(e) != 0;
     cap = std::min<size_t>(cap, paths);
     cap = std::max<size_t>(cap, 32);
     int rc;
@@ -1157,6 +1087,19 @@ static int prepare_batches(fw_scene* sc, size_t paths, size_t* cap_out) {
     return FW_OK;
 }
 
+// ceil(2^32 / n), 0xffffffff for n <= 1: the magic number of div_magic / batch_path.
+static uint32_t div_magic_number(uint32_t n) { return n <= 1 ? 0xffffffffu : (uint32_t)((((uint64_t)1 << 32) + n - 1) / n); }
+// Samples [s0, s0 + ns) of pixels pix0 .. pix0 + npix - 1 of a width x height image, or of those entries of the pixel list `pixels`.
+static Batch make_batch(uint32_t pix0, uint32_t npix, uint32_t s0, uint32_t ns, uint32_t width, uint32_t height, const uint32_t* pixels) {
+    Batch b;
+    b.pix0 = pix0; b.npix = npix; b.s0 = s0; b.ns = ns;
+    b.width = width; b.height = height;
+    b.npix_magic = div_magic_number(npix);
+    b.width_magic = div_magic_number(width);
+    b.pixels = pixels;
+    return b;
+}
+
 // Samples [s_begin, s_begin + s_count) of `npix` pixels — the image's pixels 0 .. npix-1, or the first npix entries of a pixel
 // list — in batches of at most `cap` paths: pixel tiles outer, sample chunks inner, so every pixel's samples are accumulated
 // in sample order.
@@ -1169,13 +1112,7 @@ static int run_tiles(fw_scene* sc, const fw_params* p, const CameraRec& cam, uin
         size_t np = std::min(tile, npix - pix0);
         uint32_t chunk = (uint32_t)std::max<size_t>(1, cap / np);
         for (uint32_t s = 0; s < s_count; s += chunk) {
-            Batch b;
-            b.pix0 = (uint32_t)pix0; b.npix = (uint32_t)np;
-            b.s0 = s_begin + s; b.ns = std::min(chunk, s_count - s);
-            b.width = p->width; b.height = p->height;
-            b.npix_magic = np <= 1 ? 0xffffffffu : (uint32_t)((((uint64_t)1 << 32) + np - 1) / np);
-            b.width_magic = p->width <= 1 ? 0xffffffffu : (uint32_t)((((uint64_t)1 << 32) + p->width - 1) / p->width);
-            b.pixels = pixels;
+            const Batch b = make_batch((uint32_t)pix0, (uint32_t)np, s_begin + s, std::min(chunk, s_count - s), p->width, p->height, pixels);
             if ((rc = run_batch(sc, cam, b, seed, p->use_bvh != 0, d_sum, adapt, st, tot, ev_next)) != FW_OK) return rc;
         }
     }
@@ -1469,19 +1406,11 @@ int fw_first_hit_wavefront(fw_scene* sc, int use_bvh, uint64_t seed, uint32_t n,
     segment_geometry(sc, n, &ps.nseg, &ps.seg_cap);
     FW_CUDA(cudaMemsetAsync(ps.counters, 0, sizeof(uint32_t) * (FW_MAX_DEPTH + 2) * FW_NUM_QUEUES * (size_t)ps.nseg, st));
     FW_CUDA(cudaMemsetAsync(ps.poison, 0, sizeof(uint32_t), st));
-    Batch b;   // ray i = path i = "pixel" i of a one-sample batch: RNG key (pixel i, sample, bounce)
-    b.pix0 = 0; b.npix = n; b.s0 = sample; b.ns = 1; b.width = n; b.height = 1; b.pixels = nullptr;
-    b.npix_magic = n <= 1 ? 0xffffffffu : (uint32_t)((((uint64_t)1 << 32) + n - 1) / n);
-    b.width_magic = b.npix_magic;   // width == n
+    const Batch b = make_batch(0, n, sample, 1, n, 1, nullptr);   // ray i = path i = "pixel" i of a one-sample batch: RNG key (pixel i, sample, bounce)
     const uint2 sd = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
     launch_probe_fill(ps, n, dO.as<float>(), dD.as<float>(), bounce, st);
-    if (use_bvh && sc->plan.walk && sc->plan.two_pass) {
-        WalkAuxHost ax = sc->ctx->walk;
-        ax.ent_cap = ps.seg_cap * (uint32_t)std::max(1, sc->flat.n_top_meshes);
-        launch_extend_walk(sc->plan, sc->dscene, ps, b, sd, bounce, ax, st);
-    } else {
-        launch_extend(sc->plan, use_bvh != 0, sc->lin_prog, sc->dscene, ps, b, sd, bounce, st);
-    }
+    uint64_t launches = 0;
+    TRY(extend_bounce(sc, use_bvh != 0, b, sd, bounce, st, launches));
     launch_probe_collect(sc->dscene, ps, bounce, out, st);
     FW_CUDA(cudaGetLastError());
     FW_CUDA(cudaStreamSynchronize(st));

@@ -4,19 +4,20 @@
 
 namespace fw {
 
-// Debug twin of the BVH extend: also records the number of box tests each path needed (FW_DEBUG_STEPS=1).
-template <bool LIST>
-__global__ void __launch_bounds__(FW_BLOCK) extend_bvh_debug_kernel(DeviceScene S, PathState ps, Batch b, uint2 seed, uint32_t bounce,
-                                                                    uint32_t* steps) {
-    FW_EXTEND_PROLOGUE(MAT_NUM_QUEUES)
-        if (valid) {
-            RngKey key{seed, 0u, 0u, bounce};
-            batch_path<LIST>(b, path, key.pixel, key.sample);
-            Counters cnt{0, 0};
-            trace_unified<true, true>(S, o, d, key, w, &cnt);
-            steps[path] = (uint32_t)cnt.node_tests;
-        }
-    FW_EXTEND_EPILOGUE(MAT_NUM_QUEUES)
+// What the mesh walk needs of a ray that pass 1 put into mesh-queue slot `slot` of segment `seg` because it must enter a
+// mesh (`pending` != 0): its pass-1 winner as a 64-bit key (walk.cuh pack_key), and one (slot in the segment, mesh rank,
+// mesh root node, first triangle slot) entry per mesh root box it hit.
+FW_DEV void put_mesh_entries(const DeviceScene& S, const WalkAux& aux, uint32_t* s_fill, uint32_t seg, uint32_t seg_base, uint32_t slot,
+                             uint32_t pending, const Winner& w) {
+    aux.tkey[slot] = w.found ? pack_key(w.t, w.rank, w.h.prim, aux.prim_bits) : FW_KEY_NONE;
+    uint32_t m = pending;
+    while (m) {
+        const int ord = __ffs(m) - 1;
+        m &= m - 1u;
+        const uint32_t e = atomicAdd(&s_fill[FW_Q_ENTRY], 1u);
+        FW_WALK_CHECK(e < aux.ent_cap && ord < FW_MAX_WALK_MESHES, "entry overflow e=%u cap=%u ord=%d\n", e, aux.ent_cap, ord);
+        aux.entries[(size_t)seg * aux.ent_cap + e] = make_uint4(slot - seg_base, (uint32_t)S.mesh_rank[ord], (uint32_t)S.mesh_root[ord], (uint32_t)S.mesh_tri0[ord]);
+    }
 }
 
 // Two-pass extend for BVH scenes with TriangleMesh objects (see UnifiedWalker PHASE).  Pass 1 settles every ray
@@ -24,8 +25,7 @@ __global__ void __launch_bounds__(FW_BLOCK) extend_bvh_debug_kernel(DeviceScene 
 // queue (with the pass-1 winner and its rank) and finished by pass 2, where every lane of a warp is doing real
 // mesh traversal.
 // ENTRIES: the mesh walk (kernels_walk.cu) finishes the bounce instead of pass 2: every ray that must enter a mesh also
-// gets its pass-1 winner written as a 64-bit key (walk.cuh pack_key) and one (mesh-queue slot, mesh rank) entry per mesh
-// root box it hit.
+// gets its key and entries (put_mesh_entries).
 template <bool NESTED, bool ENTRIES, bool LIST>
 __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_pass1_kernel(DeviceScene S, PathState ps, Batch b, uint2 seed,
                                                                                 uint32_t bounce, WalkAux aux) {
@@ -61,17 +61,7 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_pass1_k
             else mine = classify_winner(S, w, material);
         }
         const uint32_t slot = enqueue_hit<FW_Q_MESH + 1>(ps, s_fill, seg_base, mine, o, d, path, w, material);
-        if (ENTRIES && pending) {
-            aux.tkey[slot] = w.found ? pack_key(w.t, w.rank, w.h.prim, aux.prim_bits) : FW_KEY_NONE;
-            uint32_t m = pending;
-            while (m) {
-                const int ord = __ffs(m) - 1;
-                m &= m - 1u;
-                const uint32_t e = atomicAdd(&s_fill[FW_Q_ENTRY], 1u);
-                FW_WALK_CHECK(e < aux.ent_cap && ord < FW_MAX_WALK_MESHES, "entry overflow e=%u cap=%u ord=%d\n", e, aux.ent_cap, ord);
-                aux.entries[(size_t)seg * aux.ent_cap + e] = make_uint4(slot - seg_base, (uint32_t)S.mesh_rank[ord], (uint32_t)S.mesh_root[ord], (uint32_t)S.mesh_tri0[ord]);
-            }
-        }
+        if (ENTRIES && pending) put_mesh_entries(S, aux, s_fill, seg, seg_base, slot, pending, w);
     }
     seg_close<FW_NUM_QUEUES>(s_fill, ps, counter_row(ps, bounce, 0), seg);
 }
@@ -101,7 +91,7 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_pass1_s
             const size_t slot_in = (size_t)seg_base + e0 + threadIdx.x;
             float4 ro = ld_stream(&ps.xo[bounce & 1][slot_in]), rd = ld_stream(&ps.xd[bounce & 1][slot_in]);
             o = f3(ro); d = f3(rd); path = __float_as_uint(ro.w);
-            if (FW_EXTEND_PREFETCH && e0 + FW_BLOCK + threadIdx.x < in_count) {
+            if (e0 + FW_BLOCK + threadIdx.x < in_count) {
                 prefetch_l2(&ps.xo[bounce & 1][slot_in + FW_BLOCK]); prefetch_l2(&ps.xd[bounce & 1][slot_in + FW_BLOCK]);
             }
             if (nan_direction(d)) {
@@ -138,17 +128,7 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_pass1_s
             else mine = classify_winner(S, w, material);
         }
         const uint32_t slot = enqueue_hit<FW_Q_MESH + 1>(ps, s_fill, seg_base, mine, o, d, path, w, material);
-        if (pending) {
-            aux.tkey[slot] = w.found ? pack_key(w.t, w.rank, w.h.prim, aux.prim_bits) : FW_KEY_NONE;
-            uint32_t m = pending;
-            while (m) {
-                const int ord = __ffs(m) - 1;
-                m &= m - 1u;
-                const uint32_t e = atomicAdd(&s_fill[FW_Q_ENTRY], 1u);
-                FW_WALK_CHECK(e < aux.ent_cap && ord < FW_MAX_WALK_MESHES, "entry overflow e=%u cap=%u ord=%d\n", e, aux.ent_cap, ord);
-                aux.entries[(size_t)seg * aux.ent_cap + e] = make_uint4(slot - seg_base, (uint32_t)S.mesh_rank[ord], (uint32_t)S.mesh_root[ord], (uint32_t)S.mesh_tri0[ord]);
-            }
-        }
+        if (pending) put_mesh_entries(S, aux, s_fill, seg, seg_base, slot, pending, w);
     }
     seg_close<FW_NUM_QUEUES>(s_fill, ps, counter_row(ps, bounce, 0), seg);
 }
@@ -191,19 +171,11 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_pass2_k
 template <bool NESTED, bool MESHES, bool LIST>
 __global__ void __launch_bounds__(FW_BLOCK, FW_EXTEND_MIN_BLOCKS) extend_bvh_simple_kernel(DeviceScene S, PathState ps, Batch b, uint2 seed,
                                                                                      uint32_t bounce) {
-#if FW_SMEM_TOP_NODES > 0
-    __shared__ __align__(128) float4 s_top[FW_SMEM_TOP_NODES * 8];
-    for (int i = threadIdx.x; i < FW_SMEM_TOP_NODES * 8; i += FW_BLOCK) s_top[i] = i < S.n_nodes * 8 ? __ldg(&S.nodes[i]) : make_float4(0, 0, 0, 0);
-    __syncthreads();
-    const float4* top = s_top;
-#else
-    const float4* top = nullptr;
-#endif
     FW_EXTEND_PROLOGUE(MAT_NUM_QUEUES)
         if (valid) {
             RngKey key{seed, 0u, 0u, bounce};
             batch_path<LIST>(b, path, key.pixel, key.sample);
-            trace_unified<false, NESTED, MESHES>(S, o, d, key, w, nullptr, top);
+            trace_unified<false, NESTED, MESHES>(S, o, d, key, w, nullptr);
         }
     FW_EXTEND_EPILOGUE(MAT_NUM_QUEUES)
 }
@@ -241,7 +213,7 @@ template <bool LIST>
 static int launch_extend_t(const ExtendPlan& plan, bool use_bvh, const LinProgram& P, const DeviceScene& S, const PathState& ps,
                            const Batch& b, uint2 seed, uint32_t bounce, cudaStream_t st) {
     const unsigned G = ps.nseg;   // one block per segment
-    if (use_bvh && plan.has_top_mesh && plan.two_pass) {
+    if (use_bvh && plan.has_top_mesh) {   // scenes the mesh walk does not serve
         WalkAux none{};
         if (plan.has_medium_mesh) {
             extend_pass1_kernel<true, false, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, none);
@@ -252,11 +224,9 @@ static int launch_extend_t(const ExtendPlan& plan, bool use_bvh, const LinProgra
         }
         return 2;
     }
-    if (use_bvh) {
+    if (use_bvh) {   // no top-level mesh: a mesh, if any, sits inside a ConstantMedium
         if (plan.has_medium_mesh)
             extend_bvh_simple_kernel<true, true, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
-        else if (plan.has_mesh)
-            extend_bvh_simple_kernel<false, true, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
         else
             extend_bvh_simple_kernel<false, false, LIST><<<G, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce);
     } else if (plan.lin_prog_ok) {
@@ -292,11 +262,6 @@ static void launch_extend_pass1_entries_t(bool small_top, bool nested, const Dev
     if (nested) extend_pass1_kernel<true, true, LIST><<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, aux);
     else extend_pass1_kernel<false, true, LIST><<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, aux);
 }
-template <bool LIST>
-static void launch_extend_debug_t(const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed, uint32_t bounce, uint32_t* steps,
-                                  cudaStream_t st) {
-    extend_bvh_debug_kernel<LIST><<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, b, seed, bounce, steps);
-}
 
 // Batches over a pixel list (b.pixels set: adaptive rounds) run the LIST instantiations.
 int launch_extend(const ExtendPlan& plan, bool use_bvh, const LinProgram& P, const DeviceScene& S, const PathState& ps,
@@ -308,11 +273,6 @@ void launch_extend_pass1_entries(bool small_top, bool nested, const DeviceScene&
                                  const WalkAuxHost& ax, cudaStream_t st) {
     if (b.pixels) launch_extend_pass1_entries_t<true>(small_top, nested, S, ps, b, seed, bounce, ax, st);
     else launch_extend_pass1_entries_t<false>(small_top, nested, S, ps, b, seed, bounce, ax, st);
-}
-void launch_extend_debug(const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed, uint32_t bounce, uint32_t* steps,
-                         cudaStream_t st) {
-    if (b.pixels) launch_extend_debug_t<true>(S, ps, b, seed, bounce, steps, st);
-    else launch_extend_debug_t<false>(S, ps, b, seed, bounce, steps, st);
 }
 
 }  // namespace fw

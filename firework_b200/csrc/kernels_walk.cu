@@ -44,16 +44,9 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_WALK_MIN_BLOCKS) walk_mesh_kernel
     bool has_ray = false, active = false;
     float3 o = f3(0.0f, 0.0f, 0.0f), inv = f3(1.0f, 1.0f, 1.0f);   // the entry's ray in mesh space, permuted to (kx, ky, kz)
     uint32_t near_pack = 0, far_pack = 0;                           // node row offsets for that permutation (walk_rows)
-    float bound0 = FW_FLT_MAX;                                      // FW_WALK_CULL == 0: the bound pass 1 left
     int node = -1, sp = 0;
     uint32_t slot_in = 0;
-#if FW_WALK_SMEM_STACK
-    __shared__ unsigned long long s_stk[FW_WALK_STACK_SMEM_DEPTH][FW_BLOCK];
-    const WalkStack stk{&s_stk[0][threadIdx.x]};
-#else
-    unsigned long long stk_local[FW_WALK_STACK];   // deferred interior children: (cull distance, node)
-    const WalkStack stk{stk_local};
-#endif
+    unsigned long long stk[FW_WALK_STACK];   // deferred interior children: (cull distance, node)
     int npairs = 0;
     bool input_left = true;
 
@@ -128,7 +121,6 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_WALK_MIN_BLOCKS) walk_mesh_kernel
                             walk_rows(su.kz, inv, near_pack, far_pack);
                             W.ox[lane] = o.x; W.oy[lane] = o.y; W.oz[lane] = o.z;
                         }
-                        bound0 = rd.w > 0.0f ? cull_bound(rd.w) : FW_FLT_MAX;   // the pass-1 winner's t travels in d.w (0: none)
                         W.su_k[lane] = su.kz; W.su_x[lane] = su.sx; W.su_y[lane] = su.sy; W.su_z[lane] = su.sz;
                         W.a0[lane] = (uint32_t)m0.y;   // first triangle slot
                         W.a1[lane] = (uint32_t)rank;
@@ -152,11 +144,11 @@ __global__ void __launch_bounds__(FW_BLOCK, FW_WALK_MIN_BLOCKS) walk_mesh_kernel
         bool l0 = false, l1 = false, l2 = false, l3 = false;
         int4 cc = make_int4(0, 0, 0, 0);
         if (active) {
-            const float bnd = FW_WALK_CULL == 0 ? bound0 : key_bound(W.key[lane]);
+            const float bnd = key_bound(W.key[lane]);
             if (node < 0) {
                 for (;;) {
                     if (sp == 0) { active = false; break; }
-                    const unsigned long long e = stk.at(--sp);
+                    const unsigned long long e = stk[--sp];
                     if (!(__uint_as_float((uint32_t)(e >> 32)) > bnd)) { node = (int)(uint32_t)e; break; }
                 }
             }
@@ -206,11 +198,6 @@ void launch_extend_walk_part(int part, const ExtendPlan& plan, const DeviceScene
     if (part == 0) launch_extend_pass1_entries(plan.small_top, plan.has_medium_mesh, S, ps, b, seed, bounce, ax, st);
     else if (part == 1) walk_mesh_kernel<<<G, FW_BLOCK, 0, st>>>(S, ps, bounce, aux);
     else classify_mesh_kernel<<<G, FW_BLOCK, 0, st>>>(S, ps, bounce, aux);
-}
-int launch_extend_walk(const ExtendPlan& plan, const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed,
-                       uint32_t bounce, const WalkAuxHost& ax, cudaStream_t st) {
-    for (int part = 0; part < 3; ++part) launch_extend_walk_part(part, plan, S, ps, b, seed, bounce, ax, st);
-    return 3;
 }
 
 }  // namespace fw

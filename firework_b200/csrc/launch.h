@@ -15,7 +15,6 @@ struct ExtendPlan {
     bool has_mesh = false;          // some object is (or wraps) a TriangleMesh
     bool has_top_mesh = false;      // some render object IS a TriangleMesh
     bool has_medium_mesh = false;   // some ConstantMedium wraps a TriangleMesh
-    bool two_pass = true;           // two-pass extend for BVH scenes with top-level meshes
     bool lin_prog_ok = false;       // the linear-scan program fits kernel-parameter space
     bool lin_generic = false;       // ... and contains LIN_GENERIC items
     int lin_rect_tests = 0;         // AARect::hit calls per ray in the program
@@ -32,19 +31,15 @@ struct WalkAuxHost {
 };
 
 void launch_raygen(const CameraRec& cam, const Batch& b, uint2 seed, const PathState& ps, cudaStream_t st);
-// Returns the number of kernels launched (2 for the two-pass mesh extend).
+// The lock-step and linear-scan extend kernels.  Returns the number of kernels launched (2 for the two-pass mesh extend).
 int launch_extend(const ExtendPlan& plan, bool use_bvh, const LinProgram& prog, const DeviceScene& S, const PathState& ps,
                   const Batch& b, uint2 seed, uint32_t bounce, cudaStream_t st);
-// The same query through the collect / test walk kernels (kernels_walk.cu); returns the number of kernels launched.
-int launch_extend_walk(const ExtendPlan& plan, const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed,
-                       uint32_t bounce, const WalkAuxHost& aux, cudaStream_t st);
-// One of its three kernels on its own (0 = pass 1 with entries, 1 = mesh walk, 2 = classification): FW_DEBUG_SYNC.
+// The same query through the collect / test walk kernels (kernels_walk.cu), one of its three kernels per call:
+// 0 = pass 1 with entries, 1 = mesh walk, 2 = classification.
 void launch_extend_walk_part(int part, const ExtendPlan& plan, const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed,
                              uint32_t bounce, const WalkAuxHost& aux, cudaStream_t st);
 void launch_extend_pass1_entries(bool small_top, bool nested, const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed, uint32_t bounce,
                                  const WalkAuxHost& aux, cudaStream_t st);
-void launch_extend_debug(const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed, uint32_t bounce, uint32_t* steps,
-                         cudaStream_t st);
 void launch_miss(const DeviceScene& S, const PathState& ps, uint32_t bounce, bool black_env, cudaStream_t st);
 void launch_shade_emissive(const DeviceScene& S, const PathState& ps, uint32_t bounce, cudaStream_t st);
 void launch_shade_scatter(int mat, const DeviceScene& S, const PathState& ps, const Batch& b, uint2 seed, uint32_t bounce,

@@ -39,10 +39,6 @@ namespace fw {
 #define FW_WALK_CHECKS 0          // 1 = bounds checks with printf + trap in the walk kernels (debug builds)
 #endif
 #define FW_WALK_CHECK(cond, ...) do { if (FW_WALK_CHECKS && !(cond)) { printf(__VA_ARGS__); __trap(); } } while (0)
-#ifndef FW_WALK_SMEM_STACK
-#define FW_WALK_SMEM_STACK 0      // 1 = the walker's stack lives in shared memory ([level][thread], conflict-free) instead of local
-#endif
-constexpr int FW_WALK_STACK_SMEM_DEPTH = 32;   // 3 per wide level: covers mesh trees up to 9 wide levels (deeper ones: checked at flatten)
 constexpr int FW_WALK_STACK = 64;      // deferred interior children per lane (3 per wide level; checked at flatten)
 constexpr int FW_WALK_RING = 256;      // pair buffer (power of two): < 32 left over + at most 4 new per lane = 159 pending
 constexpr int FW_WALK_SLOTS = 32;      // entry slots per warp: one per lane
@@ -80,29 +76,21 @@ struct WalkAux {
 };
 
 // ---- culling that can not change the winner ---------------------------------------------------------------------
-// FW_WALK_CULL selects the distance a child box is culled (and ordered) by against the best hit so far:
-//   1  the box-entry parameter of the slab test (what the lock-step kernels use).  Fast, but only ALMOST safe: a triangle
-//      seen nearly edge-on is accepted with barycentrics that are rounding noise, and its t = sum(b_i z_i) (mesh.rs:188-196)
-//      can then land anywhere inside the triangle's depth range along the ray's axis kz — below the entry parameter of
-//      its own leaf box.  Such a hit is lost if an unrelated hit culled the leaf first (measured: ~3e-8 of the rays on
-//      suzanne, and WHICH is lost depends on scheduling once warps fetch work dynamically);
-//   2  the entry parameter of the kz-axis slab alone, (near_z - o_z) * (1 / d_z), kz = the axis Triangle::hit permutes to z
-//      (mesh.rs:146-153).  Every accepted hit satisfies t >= min_i z_i up to a few ulp, z_i = (p_i.z - o.z) * (1 / d.z) being
-//      computed from a vertex inside the box with the same subtraction, the same reciprocal and monotonic rounding, so
-//      t >= that slab entry: a box skipped because the entry exceeds best_t + margin can not hold the winner.  The set of
-//      boxes skipped then depends on timing, the winner does not — results are the reference's exhaustive traversal
-//      (bvh.rs:134-146), bit for bit and run to run;
-//   0  no hit-dependent culling inside an entry (reference traversal order of magnitude; for measurements).
+// A child box is culled against the best hit so far by the entry parameter of its kz-axis slab alone,
+// (near_z - o_z) * (1 / d_z), kz = the axis Triangle::hit permutes to z (mesh.rs:146-153).  Every accepted hit satisfies
+// t >= min_i z_i up to a few ulp, z_i = (p_i.z - o.z) * (1 / d.z) being computed from a vertex inside the box with the same
+// subtraction, the same reciprocal and monotonic rounding, so t >= that slab entry: a box skipped because the entry exceeds
+// best_t + margin can not hold the winner.  The set of boxes skipped then depends on timing, the winner does not — results
+// are the reference's exhaustive traversal (bvh.rs:134-146), bit for bit and run to run.
+// The box-entry parameter of the full slab test (what the lock-step kernels cull by) is NOT safe here: a triangle seen
+// nearly edge-on is accepted with barycentrics that are rounding noise, and its t = sum(b_i z_i) (mesh.rs:188-196) can then
+// land anywhere inside the triangle's depth range along kz — below the entry parameter of its own leaf box.  Such a hit is
+// lost if an unrelated hit culled the leaf first (measured: ~3e-8 of the rays on suzanne, and WHICH is lost depends on
+// scheduling once warps fetch work dynamically; profiles/r02_variants.md §2).
 // The slab test itself is axis-order independent (max / min of the same six products), so the walker keeps the ray
 // permuted to (kx, ky, kz) and loads the node rows in that order; the kz product comes out of the test for free.
-#ifndef FW_WALK_CULL
-#define FW_WALK_CULL 2
-#endif
 #ifndef FW_WALK_TEST_AT
 #define FW_WALK_TEST_AT 32   // pairs gathered by a warp before it runs a test phase (fewer: bounds shrink sooner, test lanes idle)
-#endif
-#ifndef FW_WALK_ORDER_BOX
-#define FW_WALK_ORDER_BOX 1   // deferred children ordered by box entry (0: by the kz-slab entry they are culled by); teapot +1.8 %, suzanne 0
 #endif
 
 // One deferred interior child on a lane's stack: (cull distance, node) in one 64-bit word — one local-memory access per
@@ -110,12 +98,6 @@ struct WalkAux {
 FW_DEV unsigned long long stack_entry(float dist, int node) {
     return ((unsigned long long)__float_as_uint(dist) << 32) | (uint32_t)node;
 }
-
-// Where a lane's stack lives: a private (local-memory) array, or one column of a block-wide shared-memory array.
-struct WalkStack {
-    unsigned long long* base;
-    FW_DEV unsigned long long& at(int i) const { return FW_WALK_SMEM_STACK ? base[(size_t)i * FW_BLOCK] : base[i]; }
-};
 
 // Row byte offsets inside a wide node for a ray whose axes are permuted to (kx, ky, kz): near / far plane rows of each
 // permuted axis, one byte each (near plane = max row where the direction is negative, see wide_visit).
@@ -128,9 +110,9 @@ FW_DEV void walk_rows(int kz, float3 inv_perm, uint32_t& near_pack, uint32_t& fa
 
 // One wide-node visit for the walk loop; o / inv are the ray permuted to (kx, ky, kz).  Children that survive the slab test
 // (aabb.rs:30-50 arithmetic) and the cull are split into leaves (returned in l0..l3 for the caller to emit) and interior
-// nodes (nearest becomes `node`, the rest are pushed with their cull distance).
+// nodes (nearest becomes `node`, the rest are pushed onto the lane's stack `stk` with their cull distance).
 FW_DEV void walk_visit(const float4* __restrict__ nodes, int& node, float3 o, float3 inv, uint32_t near_pack, uint32_t far_pack,
-                       float bound, WalkStack stk, int& sp, bool& l0, bool& l1, bool& l2, bool& l3, int4& cc) {
+                       float bound, unsigned long long* stk, int& sp, bool& l0, bool& l1, bool& l2, bool& l3, int4& cc) {
     const float tmin = 0.001f, tmax = 2e9f;   // render.rs:19
     const float4* n = &nodes[8 * node];
     const uintptr_t nb = reinterpret_cast<uintptr_t>(n);   // 128-byte aligned: row offsets are OR-ed in
@@ -152,8 +134,7 @@ FW_DEV void walk_visit(const float4* __restrict__ nodes, int& node, float3 o, fl
     bool h2 = slab(nx.z, ny.z, nz.z, fx.z, fy.z, fz.z, e2, z2);
     bool h3 = slab(nx.w, ny.w, nz.w, fx.w, fy.w, fz.w, e3, z3);
     // cull / order distance (a NaN product, 0 * inf, must not drop the child: fmaxf returns the other operand)
-    float t0 = FW_WALK_CULL == 2 ? fmaxf(z0, -FW_FLT_MAX) : e0, t1 = FW_WALK_CULL == 2 ? fmaxf(z1, -FW_FLT_MAX) : e1;
-    float t2 = FW_WALK_CULL == 2 ? fmaxf(z2, -FW_FLT_MAX) : e2, t3 = FW_WALK_CULL == 2 ? fmaxf(z3, -FW_FLT_MAX) : e3;
+    float t0 = fmaxf(z0, -FW_FLT_MAX), t1 = fmaxf(z1, -FW_FLT_MAX), t2 = fmaxf(z2, -FW_FLT_MAX), t3 = fmaxf(z3, -FW_FLT_MAX);
     h0 = h0 && !(t0 > bound); h1 = h1 && !(t1 > bound); h2 = h2 && !(t2 > bound); h3 = h3 && !(t3 > bound);
     // leaf children; empty slots (code FW_CODE_EXIT, inverted box) are excluded explicitly: a direction with NaN / infinite
     // components (scatter off a near-zero interpolated normal) passes EVERY slab test, f32::max / min ignoring NaN
@@ -164,9 +145,8 @@ FW_DEV void walk_visit(const float4* __restrict__ nodes, int& node, float3 o, fl
     t0 = (h0 && cc.x >= 0) ? t0 : miss; t1 = (h1 && cc.y >= 0) ? t1 : miss;
     t2 = (h2 && cc.z >= 0) ? t2 : miss; t3 = (h3 && cc.w >= 0) ? t3 : miss;
     int c0 = cc.x, c1 = cc.y, c2 = cc.z, c3 = cc.w;
-#if FW_WALK_ORDER_BOX
-    // visit order by the true box entry (all three slabs: a better front-to-back proxy), culling still by the kz slab alone:
-    // the order only decides how soon the bound shrinks, never which hit wins
+    // visit order by the true box entry (all three slabs: a better front-to-back proxy than the kz slab, teapot +1.8 %),
+    // culling still by the kz slab alone: the order only decides how soon the bound shrinks, never which hit wins
     float k0 = t0 < miss ? e0 : miss, k1 = t1 < miss ? e1 : miss, k2 = t2 < miss ? e2 : miss, k3 = t3 < miss ? e3 : miss;
     auto cswap3 = [](float& ka, int& ca, float& da, float& kb, int& cb, float& db) {
         if (kb < ka) { float k = ka; ka = kb; kb = k; int c = ca; ca = cb; cb = c; float d = da; da = db; db = d; }
@@ -175,20 +155,10 @@ FW_DEV void walk_visit(const float4* __restrict__ nodes, int& node, float3 o, fl
     cswap3(k2, c2, t2, k3, c3, t3);
     cswap3(k0, c0, t0, k2, c2, t2);
     FW_WALK_CHECK(sp + 3 <= FW_WALK_STACK, "walk stack overflow sp=%d node=%d\n", sp, node);
-    if (k3 < miss) stk.at(sp++) = stack_entry(t3, c3);
-    if (k2 < miss) stk.at(sp++) = stack_entry(t2, c2);
-    if (k1 < miss) stk.at(sp++) = stack_entry(t1, c1);
+    if (k3 < miss) stk[sp++] = stack_entry(t3, c3);
+    if (k2 < miss) stk[sp++] = stack_entry(t2, c2);
+    if (k1 < miss) stk[sp++] = stack_entry(t1, c1);
     node = (k0 < miss) ? c0 : -1;
-#else
-    cswap(t0, c0, t1, c1);
-    cswap(t2, c2, t3, c3);
-    cswap(t0, c0, t2, c2);   // (t0, c0) = nearest surviving interior child
-    FW_WALK_CHECK(sp + 3 <= FW_WALK_STACK, "walk stack overflow sp=%d node=%d\n", sp, node);
-    if (t3 < miss) stk.at(sp++) = stack_entry(t3, c3);
-    if (t2 < miss) stk.at(sp++) = stack_entry(t2, c2);
-    if (t1 < miss) stk.at(sp++) = stack_entry(t1, c1);
-    node = (t0 < miss) ? c0 : -1;
-#endif
 }
 
 // Appends the leaf children a lane found (l0..l3 of cc) for its entry slot `slot` to the warp's pair ring; returns the new

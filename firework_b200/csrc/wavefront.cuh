@@ -22,19 +22,11 @@ namespace fw {
 // counter per queue was the top stall of both extend and shade: ~2.5 same-sector atomics per warp iteration.)
 // Path-state streams are touched once per kernel: load / store them with the streaming (evict-first) policy so
 // that they do not push the scene tables (nodes, objects, shapes, materials) out of L1.
-#ifndef FW_STREAM_HINTS
-#define FW_STREAM_HINTS 1
-#endif
-FW_DEV float4 ld_stream(const float4* p) { return FW_STREAM_HINTS ? __ldcs(p) : *p; }
-#ifndef FW_PREFETCH
-#define FW_PREFETCH 1
-#endif
+FW_DEV float4 ld_stream(const float4* p) { return __ldcs(p); }
 // The record a shade thread will need in its NEXT iteration is FW_BLOCK slots ahead: ask L2 for it now (no register
-// cost).  Measured: +1-2 % on the latency-bound shade kernels, +0.3 ... +0.6 % on the extend kernels (FW_EXTEND_PREFETCH).
-FW_DEV void prefetch_l2(const void* p) {
-    if (FW_PREFETCH) asm volatile("prefetch.global.L2 [%0];" ::"l"(p));
-}
-FW_DEV void st_stream(float4* p, float4 v) { if (FW_STREAM_HINTS) __stcs(p, v); else *p = v; }
+// cost).  Measured: +1-2 % on the latency-bound shade kernels, +0.3 ... +0.6 % on the extend kernels (profiles/r02_variants.md).
+FW_DEV void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
+FW_DEV void st_stream(float4* p, float4 v) { __stcs(p, v); }
 // Counter rows: material / mesh queues of bounce b live in row b; the extend queue CONSUMED at bounce b lives in
 // row b (raygen fills row 0, the shade kernels of bounce b fill row b + 1).
 FW_DEV uint32_t* counter_row(const PathState& ps, uint32_t row, int queue) {
@@ -114,15 +106,13 @@ FW_DEV void seg_close(const uint32_t* s_fill, const PathState& ps, uint32_t* cou
 }
 // Reserve one slot in queue `mine` of the segment for every lane with 0 <= mine < NQ: one shared-memory atomic per
 // warp per non-empty queue (warp ballot / popc compaction).  Returns the slot (global index); all 32 lanes must call.
-#ifndef FW_RESERVE_MATCH
-#define FW_RESERVE_MATCH 1   // 1 = group the lanes of a warp by queue with one match.any instead of one ballot round per queue
-#endif
+// More than two queues: the lanes of a warp are grouped by queue with one match.any instead of one ballot round per queue.
 template <int NQ>
 FW_DEV uint32_t seg_reserve(uint32_t* s_fill, uint32_t seg_base, int mine) {
     unsigned lane = threadIdx.x & 31u;
     unsigned lt = (1u << lane) - 1u;
     uint32_t slot = 0;
-    if (FW_RESERVE_MATCH && NQ > 2) {
+    if (NQ > 2) {
         const unsigned grp = __match_any_sync(0xffffffffu, mine);   // the lanes that go to the same queue (or to none: mine < 0)
         const int leader = __ffs(grp) - 1;
         uint32_t base = 0;
@@ -158,49 +148,24 @@ FW_DEV int classify_winner(const DeviceScene& S, const Winner& w, int& material)
     if ((meta.x & OBJ_KIND_MASK) == SH_RECT3D) material = winner_material(S, w.obj, w.h.prim);  // faces may carry their own material
     return __ldg(&S.mats[material].kind);
 }
-// Writes the hit record of one ray into slot `slot` of queue K (K is a compile-time constant at every call site, so
-// the queue's pointers are plain kernel parameters).
-template <int K>
-FW_DEV void put_hit(const PathState& ps, uint32_t slot, float3 o, float3 d, uint32_t path, const Winner& w, int material) {
-    if (K == MAT_MISS) {
-        st_stream(&ps.hq[K].d[slot], make_float4(d.x, d.y, d.z, __uint_as_float(path)));
-        return;
-    }
-    st_stream(&ps.hq[K].o[slot], make_float4(o.x, o.y, o.z, __uint_as_float(path)));
-    st_stream(&ps.hq[K].d[slot], make_float4(d.x, d.y, d.z, w.t));
-    st_stream(&ps.hq[K].w[slot], make_float4(__int_as_float(w.obj), __int_as_float(w.h.prim), __int_as_float(material), __int_as_float(w.rank)));
-}
-#ifndef FW_ENQUEUE_INDEXED
-#define FW_ENQUEUE_INDEXED 1   // 1 = pick the queue's stream pointers with a (constant-bank) indexed load: one store sequence for the warp
-#endif
+// Writes the hit record of every lane with 0 <= mine < NQ into its reserved slot of queue `mine`; the queue's stream pointers
+// come from an indexed (constant-bank) load, so the warp runs one store sequence whatever queues its lanes go to.  Returns
+// the global slot index (meaningful for those lanes); all 32 lanes must call.
 template <int NQ>
 FW_DEV uint32_t enqueue_hit(const PathState& ps, uint32_t* s_fill, uint32_t seg_base, int mine, float3 o, float3 d, uint32_t path,
                             const Winner& w, int material) {
     uint32_t slot = seg_reserve<NQ>(s_fill, seg_base, mine);
-    if (FW_ENQUEUE_INDEXED) {
-        if (mine >= 0) {
-            const HitQueue q = ps.hq[mine];   // kernel-parameter space, indexed per lane
-            if (mine == MAT_MISS) {
-                st_stream(&q.d[slot], make_float4(d.x, d.y, d.z, __uint_as_float(path)));
-            } else {
-                st_stream(&q.o[slot], make_float4(o.x, o.y, o.z, __uint_as_float(path)));
-                st_stream(&q.d[slot], make_float4(d.x, d.y, d.z, w.t));
-                st_stream(&q.w[slot], make_float4(__int_as_float(w.obj), __int_as_float(w.h.prim), __int_as_float(material), __int_as_float(w.rank)));
-            }
+    if (mine >= 0) {
+        const HitQueue q = ps.hq[mine];   // kernel-parameter space, indexed per lane
+        if (mine == MAT_MISS) {
+            st_stream(&q.d[slot], make_float4(d.x, d.y, d.z, __uint_as_float(path)));
+        } else {
+            st_stream(&q.o[slot], make_float4(o.x, o.y, o.z, __uint_as_float(path)));
+            st_stream(&q.d[slot], make_float4(d.x, d.y, d.z, w.t));
+            st_stream(&q.w[slot], make_float4(__int_as_float(w.obj), __int_as_float(w.h.prim), __int_as_float(material), __int_as_float(w.rank)));
         }
-        return slot;
     }
-    switch (mine) {   // one arm per queue keeps the queue index a compile-time constant
-        case 0: put_hit<0>(ps, slot, o, d, path, w, material); break;
-        case 1: put_hit<1>(ps, slot, o, d, path, w, material); break;
-        case 2: put_hit<2>(ps, slot, o, d, path, w, material); break;
-        case 3: put_hit<3>(ps, slot, o, d, path, w, material); break;
-        case 4: put_hit<4>(ps, slot, o, d, path, w, material); break;
-        case 5: put_hit<5>(ps, slot, o, d, path, w, material); break;
-        case FW_Q_MESH: if (NQ > FW_Q_MESH) put_hit<FW_Q_MESH>(ps, slot, o, d, path, w, material); break;
-        default: break;
-    }
-    return slot;   // global slot index (meaningful for lanes with 0 <= mine < NQ)
+    return slot;
 }
 // A hit record read back by the kernel that consumes queue K.
 struct HitIn {
@@ -223,11 +188,8 @@ FW_DEV HitIn get_hit(const PathState& ps, uint32_t slot) {
     return h;
 }
 
-// Common shape of the extend kernels: one block per segment, FW_BLOCK rays per iteration.  The body sets `w`
-// for valid lanes; the epilogue sorts the ray into its shade queue.
-#ifndef FW_EXTEND_PREFETCH
-#define FW_EXTEND_PREFETCH 1   // L2 prefetch of the next iteration's ray records: +0.3 ... +0.6 % (profiles/r02_variants.md)
-#endif
+// Common shape of the extend kernels: one block per segment, FW_BLOCK rays per iteration (the next iteration's ray
+// records are prefetched to L2).  The body sets `w` for valid lanes; the epilogue sorts the ray into its shade queue.
 #define FW_EXTEND_PROLOGUE(NQ_OUT)                                                                         \
     __shared__ uint32_t s_fill[FW_NUM_QUEUES];                                                               \
     const uint32_t in_count = counter_row(ps, bounce, FW_Q_EXTEND)[blockIdx.x];                              \
@@ -240,7 +202,7 @@ FW_DEV HitIn get_hit(const PathState& ps, uint32_t slot) {
             const size_t slot_in = (size_t)blockIdx.x * ps.seg_cap + e0 + threadIdx.x;                       \
             float4 ro = ld_stream(&ps.xo[bounce & 1][slot_in]), rd = ld_stream(&ps.xd[bounce & 1][slot_in]);     \
             o = f3(ro); d = f3(rd); path = __float_as_uint(ro.w);                                            \
-            if (FW_EXTEND_PREFETCH && e0 + FW_BLOCK + threadIdx.x < in_count) {                              \
+            if (e0 + FW_BLOCK + threadIdx.x < in_count) {                                                    \
                 prefetch_l2(&ps.xo[bounce & 1][slot_in + FW_BLOCK]); prefetch_l2(&ps.xd[bounce & 1][slot_in + FW_BLOCK]); \
             }                                                                                                \
         }                                                                                                    \

@@ -74,10 +74,33 @@ def test_ragged_image_sizes(w, h, spp):
     _compare(s, w, h, spp, True, min_close=0.99 if w * h > 4 else 1.0)
 
 
+def _mesh_layout(top_meshes, medium_mesh, n_spheres):
+    """A floor, `top_meshes` tetrahedra (4 triangles: an interior mesh root, which the mesh walk needs), optionally one more
+    as the boundary of a ConstantMedium, and `n_spheres` small spheres (over 32 objects: more than 16 top-level leaves)."""
+    s = _base_scene()
+    red = s.add_material(LambertianMat.with_color(Vec3(0.8, 0.2, 0.2)))
+    grey = s.add_material(LambertianMat.with_color(Vec3(0.5, 0.5, 0.5)))
+    s.add_object(RenderObject.new(XZRect(-6.0, 6.0, -6.0, 6.0, 0.0, grey)))
+    v = [[0, 0, 0], [1, 0, 0], [0.5, 0, 0.9], [0.5, 0.9, 0.4]]
+    tet = [0, 2, 1, 0, 1, 3, 1, 2, 3, 2, 0, 3]
+    for k in range(top_meshes):
+        s.add_object(RenderObject.new(TriangleMesh(v, tet, None, None, red)).position(-2.0 + 1.5 * k, 0.1, 0.0)
+                     .rotate(Rotor3.from_rotation_xz(0.3 * k)))
+    if medium_mesh:
+        s.add_volume(RenderObject.new(TriangleMesh(v, tet, None, None, red)).position(1.5, 0.1, 0.5), 2.0,
+                     ConstantTexture(Vec3(0.2, 0.4, 0.9)))
+    for x, z in np.random.default_rng(5).uniform((-4.0, -4.0), (4.0, -1.5), (n_spheres, 2)):
+        s.add_object(RenderObject.new(Sphere(0.15, grey)).position(float(x), 0.15, float(z)))
+    return s
+
+
 @pytest.mark.parametrize("use_bvh", [True, False])
 def test_meshes_small_and_nested_in_media(use_bvh):
     """1- and 2-triangle meshes (Leaf / DoubleLeaf mesh roots), a mesh with normals + uvs, and ConstantMedium
-    wrapping a mesh and a box (volume.rs generic over the boundary shape)."""
+    wrapping a mesh and a box (volume.rs generic over the boundary shape).  Then the other mesh layouts an extend kernel is
+    chosen by: a mesh only inside a medium, and meshes the mesh walk serves, with and without one inside a medium, under a
+    top-level tree of at most and of more than 16 leaves (linear scan: the larger scenes' programs do not fit
+    kernel-parameter space, so the object loop runs)."""
     s = _base_scene()
     red = s.add_material(LambertianMat.with_color(Vec3(0.8, 0.2, 0.2)))
     grey = s.add_material(LambertianMat.with_color(Vec3(0.5, 0.5, 0.5)))
@@ -94,6 +117,8 @@ def test_meshes_small_and_nested_in_media(use_bvh):
     s.add_volume(RenderObject.new(Rect3d.with_size(Vec3(1.0, 1.0, 1.0), grey)).position(-0.5, 0.0, -2.5), 1.5,
                  ConstantTexture(Vec3(0.9, 0.9, 0.9)))
     _compare(s, 96, 64, 4, use_bvh)
+    for top_meshes, medium_mesh, n_spheres in ((0, True, 0), (2, True, 0), (2, True, 100), (2, False, 100)):
+        _compare(_mesh_layout(top_meshes, medium_mesh, n_spheres), 64, 40, 2, use_bvh)
 
 
 @pytest.mark.parametrize("use_bvh", [True, False])
