@@ -15,6 +15,7 @@ inline int run_example(int argc, char** argv, const char* title, const firework:
         if (c == ' ') c = '_';
     float target_error = -1.0f;
     uint32_t min_samples = 16;
+    bool denoise = false;
     for (int i = 1; i < argc; ++i) {
         const std::string a = argv[i];
         auto next = [&]() -> const char* { if (i + 1 >= argc) { fprintf(stderr, "error: %s needs a value\n", a.c_str()); exit(1); } return argv[++i]; };
@@ -26,11 +27,13 @@ inline int run_example(int argc, char** argv, const char* title, const firework:
         else if (a == "--gpus") renderer = renderer.gpus(atoi(next()));
         else if (a == "--target-error") target_error = (float)atof(next());
         else if (a == "--min-samples") min_samples = (uint32_t)atol(next());
+        else if (a == "--denoise") denoise = true;
         else if (a == "--asset-dir") renderer = renderer.asset_dir(next());
         else if (a == "--output" || a == "-o") out = next();
-        else { fprintf(stderr, "usage: %s [--yaml] [-s samples] [--width w] [--height h] [--seed n] [--gpus n] [--target-error e] [--min-samples n] [--asset-dir d] [-o out.png]\n", argv[0]); return 1; }
+        else { fprintf(stderr, "usage: %s [--yaml] [-s samples] [--width w] [--height h] [--seed n] [--gpus n] [--target-error e] [--min-samples n] [--denoise] [--asset-dir d] [-o out.png]\n", argv[0]); return 1; }
     }
     if (target_error >= 0.0f) renderer = renderer.adaptive(target_error, min_samples);
+    if (denoise) renderer = renderer.denoise();
     try {
         const auto start = std::chrono::steady_clock::now();
         const std::vector<firework::Color> render = renderer.render(scene);

@@ -3,7 +3,8 @@
 BVH on.  `-o` writes a PNG (window.rs:59-66 `save_image`); without it the image is written to `<name>.png`
 (there is no window here).  Extra flags: --checkpoint FILE resumes / saves the fp32 sample sums so that a long
 render can be interrupted (the reference's 3.36 h render has no intermediate save, README.md:16); --target-error E renders each
-pixel until its relative standard error is <= E (adaptive sampling, `-s` is the cap per pixel, --min-samples the first round)."""
+pixel until its relative standard error is <= E (adaptive sampling, `-s` is the cap per pixel, --min-samples the first round);
+--denoise filters the render with first-hit albedo / normal / depth as guides (fw_render_denoised, default settings)."""
 import argparse
 import os
 import sys
@@ -29,7 +30,15 @@ def main(argv=None):
     ap.add_argument("--target-error", type=float, default=None,
                     help="adaptive sampling: render each pixel until its relative standard error <= this (-s is the cap)")
     ap.add_argument("--min-samples", type=int, default=16, help="adaptive sampling: samples of the first round (default 16)")
+    ap.add_argument("--denoise", action="store_true",
+                    help="filter the render with first-hit albedo / normal / depth as guides (-s >= 2)")
     opt = ap.parse_args(argv)
+    if opt.denoise:
+        # a denoised render owns its sample range: no chunks, no checkpoint, no adaptive schedule
+        if opt.checkpoint or opt.chunk or opt.target_error is not None:
+            ap.error("--denoise can not be combined with --checkpoint, --chunk or --target-error")
+        if opt.samples < 2:
+            ap.error("--denoise needs --samples >= 2")
     if opt.target_error is not None:
         # an adaptive render owns its sample schedule: it can not be split into chunks or resumed from a checkpoint
         if opt.checkpoint or opt.chunk:
@@ -42,7 +51,10 @@ def main(argv=None):
     renderer = (Renderer.default().width(opt.width).height(opt.height).samples(opt.samples).use_bvh(True)
                 .camera(camera).seed(opt.seed))
     start = time.time()
-    if opt.target_error is not None:
+    if opt.denoise:
+        rgb = renderer.denoise().render(scene)
+        print(f"Finished Rendering in {int(time.time() - start)} s")
+    elif opt.target_error is not None:
         rgb = renderer.adaptive(opt.target_error, opt.min_samples).render(scene)
         st = renderer.last_stats
         print(f"Finished Rendering in {int(time.time() - start)} s")

@@ -37,6 +37,15 @@ class FwAdaptiveResult(C.Structure):
     _fields_ = [("rounds", C.c_uint32), ("samples", C.c_uint64), ("active", C.c_uint32 * 32)]
 
 
+class FwAov(C.Structure):
+    _fields_ = [("albedo", C.c_void_p), ("normal", C.c_void_p), ("depth", C.c_void_p), ("object", C.c_void_p)]
+
+
+class FwDenoise(C.Structure):
+    _fields_ = [("iterations", C.c_uint32), ("aov_samples", C.c_uint32), ("sigma_luminance", C.c_float),
+                ("sigma_depth", C.c_float), ("sigma_albedo", C.c_float)]
+
+
 class FireworkError(RuntimeError):
     def __init__(self, code, msg):
         super().__init__(f"firework_b200 error {code}: {msg}")
@@ -53,6 +62,7 @@ EXPORTS = [
     "fw_device_count", "fw_measure_peaks", "fw_selftest_shared_division", "fw_obj_load", "fw_obj_num_models",
     "fw_obj_model_name", "fw_obj_model_sizes", "fw_obj_model_copy", "fw_obj_destroy", "fw_hdr_load", "fw_hdr_free", "fw_image_load", "fw_image_free", "fw_png_write", "fw_set_profiling", "fw_set_batch_paths", "fw_release_cached_memory", "fw_texture_store_stats",
     "fw_resolve_host", "fw_render_multi", "fw_scene_walk_info", "fw_first_hit_wavefront", "fw_render_adaptive",
+    "fw_render_aov", "fw_denoise_host", "fw_render_denoised",
 ]
 
 _lib = None
@@ -138,6 +148,11 @@ def lib():
         if hasattr(L, "fw_render_adaptive"):        # absent only in older builds used for A/B timing
             L.fw_render_adaptive.argtypes = [C.c_void_p, C.POINTER(FwParams), C.POINTER(FwAdaptive)] + [C.c_void_p] * 4 + \
                                             [C.POINTER(FwStats), C.POINTER(FwAdaptiveResult)]
+        if hasattr(L, "fw_render_denoised"):        # absent only in older builds used for A/B timing
+            L.fw_render_aov.argtypes = [C.c_void_p, C.POINTER(FwParams), C.POINTER(FwAov), C.POINTER(FwStats)]
+            L.fw_denoise_host.argtypes = [C.c_int, C.c_uint32, C.c_uint32] + [C.c_void_p] * 5 + [C.POINTER(FwDenoise), C.c_void_p, C.c_void_p]
+            L.fw_render_denoised.argtypes = [C.c_void_p, C.POINTER(FwParams), C.POINTER(FwDenoise)] + [C.c_void_p] * 4 + \
+                                            [C.POINTER(FwAov), C.POINTER(FwStats)]
         _lib = L
     return _lib
 

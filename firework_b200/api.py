@@ -588,7 +588,8 @@ class Renderer:
     """render.rs:57-107; defaults per render.rs:198-218 (1920x1080, 128 spp, use_bvh=false, gamma 2.2).
 
     Extra (not in the reference): `seed` keys the counter-based RNG, `device` picks the GPU, `gpus` spreads the samples over
-    several GPUs, `adaptive` renders each pixel until its noise estimate meets a target.
+    several GPUs, `adaptive` renders each pixel until its noise estimate meets a target, `denoise` filters the render with
+    first-hit feature buffers as guides.
     """
 
     def __init__(self):
@@ -598,6 +599,7 @@ class Renderer:
         self._seed = 0
         self._gpus, self._reduce = 1, "nccl"
         self._adaptive = None
+        self._denoise = None
         self.last_stats = None
 
     @staticmethod
@@ -626,6 +628,22 @@ class Renderer:
         else:
             from .engine import ADAPTIVE_FLOOR
             self._adaptive = (float(threshold), int(min_samples), ADAPTIVE_FLOOR if floor is None else float(floor))
+        return self
+
+    def denoise(self, iterations=5, aov_samples=4, sigma_luminance=4.0, sigma_depth=0.1, sigma_albedo=0.1):
+        """Extra (not in the reference): a denoised render (fw_render_denoised, DESIGN.md §12).  The image is rendered at
+        `samples` spp (>= 2) as usual, the first-hit albedo, normal and depth of every pixel are averaged over its first
+        `aov_samples` samples, and an edge-aware a-trous filter of `iterations` passes (step 1, 2, 4, ...) averages each pixel
+        with neighbours whose luminance (in standard deviations of the noise estimate, `sigma_luminance`), relative depth
+        (`sigma_depth`) and albedo (`sigma_albedo`) are close, and whose normals agree.  `iterations=None` switches it off.  Single
+        GPU and not together with adaptive(): `render` raises ValueError for those combinations.  last_stats then carries
+        `denoised` (linear fp32), `variance` (of the mean luminance before filtering) and `aov` (albedo, normal, depth,
+        object)."""
+        if iterations is None:
+            self._denoise = None
+        else:
+            self._denoise = {"iterations": int(iterations), "aov_samples": int(aov_samples), "sigma_luminance": float(sigma_luminance),
+                             "sigma_depth": float(sigma_depth), "sigma_albedo": float(sigma_albedo)}
         return self
 
     def width(self, w):
@@ -678,6 +696,19 @@ class Renderer:
     def render(self, scene: Scene) -> np.ndarray:
         """GPU drop-in for `Renderer::render` — returns (height, width, 3) u8, row 0 = top."""
         from .engine import NativeScene, render_scene
+        if self._denoise is not None:
+            if self._gpus > 1:
+                raise ValueError("a denoised render runs on one GPU: gpus(n > 1) and denoise() can not be combined")
+            if self._adaptive is not None:
+                raise ValueError("adaptive() and denoise() can not be combined")
+            ns = NativeScene.from_scene(scene, 0)
+            try:
+                rgb, _sum, den, var, aov, stats = ns.render_denoised(self.params(), want_sum=False, **self._denoise)
+            finally:
+                ns.close()
+            stats["denoised"], stats["variance"], stats["aov"] = den, var, aov
+            self.last_stats = stats
+            return rgb
         if self._adaptive is not None:
             if self._gpus > 1:
                 raise ValueError("adaptive sampling renders on one GPU: gpus(n > 1) and adaptive() can not be combined")

@@ -275,6 +275,7 @@ static void destroy_ctx(RenderCtx* c) {
     fr(c->d_sum); fr(c->d_rgb);
     fr(c->adapt.m1); fr(c->adapt.m2); fr(c->adapt.count); fr(c->adapt.err); fr(c->adapt.list[0]); fr(c->adapt.list[1]);
     fr(c->adapt.keep); fr(c->adapt.block_base);
+    fr(c->aov.nz); fr(c->aov.alb); fr(c->aov.obj); fr(c->dn_cv[0]); fr(c->dn_cv[1]); fr(c->dn_planar); fr(c->dn_var); fr(c->dn_color);
     if (c->h_rays) cudaFreeHost(c->h_rays);
     if (c->h_stage) cudaFreeHost(c->h_stage);
     if (c->d_rays) cudaFree(c->d_rays);
@@ -1119,6 +1120,62 @@ static int run_tiles(fw_scene* sc, const fw_params* p, const CameraRec& cam, uin
     return FW_OK;
 }
 
+// The AOV pass (DESIGN.md §12) over samples [s_begin, s_begin + s_count) of every pixel, with run_tiles' batching: raygen and
+// the bounce-0 extend of each batch, its records collected and added in sample order.  Leaves the means in ctx->aov (and,
+// when `planar` is set, the planar albedo / normal / depth there).
+static int aov_pass(fw_scene* sc, const fw_params* p, const CameraRec& cam, uint2 seed, size_t cap, uint32_t s_begin, uint32_t s_count,
+                    float* planar, cudaStream_t st, RunTotals& tot) {
+    RenderCtx* c = sc->ctx;
+    PathState& ps = c->ps;
+    const size_t npix = (size_t)p->width * p->height;
+    const unsigned grid = grid_for(npix, 256, sc->sm_count * 8);
+    FW_CUDA(cudaMemsetAsync(c->aov.nz, 0, npix * sizeof(float4), st));
+    FW_CUDA(cudaMemsetAsync(c->aov.alb, 0, npix * sizeof(float4), st));
+    const size_t tile = std::min(npix, cap);
+    for (size_t pix0 = 0; pix0 < npix; pix0 += tile) {
+        const size_t np = std::min(tile, npix - pix0);
+        const uint32_t chunk = (uint32_t)std::max<size_t>(1, cap / np);
+        for (uint32_t s = 0; s < s_count; s += chunk) {
+            const Batch b = make_batch((uint32_t)pix0, (uint32_t)np, s_begin + s, std::min(chunk, s_count - s), p->width, p->height, nullptr);
+            segment_geometry(sc, (size_t)b.npix * b.ns, &ps.nseg, &ps.seg_cap);
+            FW_CUDA(cudaMemsetAsync(ps.counters, 0, sizeof(uint32_t) * (FW_MAX_DEPTH + 2) * FW_NUM_QUEUES * (size_t)ps.nseg, st));
+            FW_CUDA(cudaMemsetAsync(ps.poison, 0, sizeof(uint32_t), st));
+            launch_raygen(cam, b, seed, ps, st);
+            int rc = extend_bounce(sc, p->use_bvh != 0, b, seed, 0, st, tot.launches);
+            if (rc != FW_OK) return rc;
+            tot.extend_launches++;
+            launch_aov_collect(sc->dscene, ps, st);
+            launch_aov_accumulate(c->aov, ps, b, s == 0, grid_for(b.npix, 256, sc->sm_count * 8), st);
+            launch_tally(ps, c->d_rays, st);
+            tot.launches += 4;
+            if ((rc = sync_stage(st, "AOV pass", 0)) != FW_OK) return rc;
+        }
+    }
+    launch_aov_finalize(c->aov, (uint32_t)npix, (float)s_count, planar, grid, st);
+    tot.launches++;
+    FW_CUDA(cudaGetLastError());
+    return FW_OK;
+}
+
+// The a-trous iterations over ctx->dn_cv[0] with the guides in ctx->aov; returns the index of the buffer holding the result.
+static int denoise_iterations(const fw_denoise* dn, uint32_t width, uint32_t height, float4* cv[2], const AovState& g, cudaStream_t st,
+                              uint64_t* launches) {
+    const DenoiseSigmas sg{dn->sigma_luminance, dn->sigma_depth, dn->sigma_albedo};
+    int cur = 0;
+    for (uint32_t it = 0; it < dn->iterations; ++it, cur ^= 1) launch_atrous(cv[cur], g.nz, g.alb, width, height, it, sg, cv[cur ^ 1], st);
+    if (launches) *launches += dn->iterations;
+    return cur;
+}
+
+static bool denoise_settings_ok(const fw_denoise* dn) {
+    auto pos = [](float v) { return std::isfinite(v) && v > 0.0f; };
+    if (dn->iterations < 1 || dn->iterations > 10) return set_error(FW_ERR_ARG, "iterations must be in 1..10"), false;
+    if (dn->aov_samples < 1) return set_error(FW_ERR_ARG, "aov_samples must be >= 1"), false;
+    if (!pos(dn->sigma_luminance) || !pos(dn->sigma_depth) || !pos(dn->sigma_albedo))
+        return set_error(FW_ERR_ARG, "sigma_luminance, sigma_depth and sigma_albedo must be finite and > 0"), false;
+    return true;
+}
+
 // Closes the device work of one call (ev_begin was recorded at its start): ray tally, event times -> stats.  Synchronises `st`.
 static int finish_call(fw_scene* sc, cudaStream_t st, RunTotals& tot, uint64_t samples, fw_stats* stats) {
     FW_CUDA(cudaEventRecord(sc->ctx->ev_end, st));
@@ -1194,6 +1251,23 @@ int fw::ensure_adaptive_buffers(fw_scene* sc, size_t npix) {
     FW_CUDA(cudaMalloc(&a.keep, npix));
     FW_CUDA(cudaMalloc(&a.block_base, ((size_t)adaptive_blocks((uint32_t)npix) + 1) * sizeof(uint32_t)));
     c->adapt_pix = npix;
+    return FW_OK;
+}
+int fw::ensure_denoise_buffers(fw_scene* sc, size_t npix) {
+    RenderCtx* c = sc->ctx;
+    if (c->dn_pix >= npix) return FW_OK;
+    auto fr = [](auto*& p) { if (p) { cudaFree(p); p = nullptr; } };
+    fr(c->aov.nz); fr(c->aov.alb); fr(c->aov.obj); fr(c->dn_cv[0]); fr(c->dn_cv[1]); fr(c->dn_planar); fr(c->dn_var); fr(c->dn_color);
+    c->dn_pix = 0;
+    FW_CUDA(cudaMalloc(&c->aov.nz, npix * sizeof(float4)));
+    FW_CUDA(cudaMalloc(&c->aov.alb, npix * sizeof(float4)));
+    FW_CUDA(cudaMalloc(&c->aov.obj, npix * sizeof(int)));
+    FW_CUDA(cudaMalloc(&c->dn_cv[0], npix * sizeof(float4)));
+    FW_CUDA(cudaMalloc(&c->dn_cv[1], npix * sizeof(float4)));
+    FW_CUDA(cudaMalloc(&c->dn_planar, npix * 7 * sizeof(float)));
+    FW_CUDA(cudaMalloc(&c->dn_var, npix * sizeof(float)));
+    FW_CUDA(cudaMalloc(&c->dn_color, npix * 3 * sizeof(float)));
+    c->dn_pix = npix;
     return FW_OK;
 }
 int fw::commit_scene(fw_scene* sc, int device) { return fw_scene_commit(sc, device); }
@@ -1329,6 +1403,141 @@ int fw_render_adaptive(fw_scene* sc, const fw_params* p, const fw_adaptive* ad, 
         if (error_out) FW_CUDA(cudaMemcpyAsync(error_out, A.err, npix * sizeof(float), cudaMemcpyDeviceToHost, st));
         FW_CUDA(cudaStreamSynchronize(st));
         if (result) *result = res;
+        return FW_OK;
+});
+}
+
+// ---- denoised renders (DESIGN.md §12) --------------------------------------------------------------------
+static int check_image(const fw_params* p) {
+    if (p->width == 0 || p->height == 0 || p->samples == 0) return set_error(FW_ERR_ARG, "width, height and samples must be non-zero");
+    if ((uint64_t)p->width * p->height > 0x7fffffffull) return set_error(FW_ERR_ARG, "image too large");
+    return FW_OK;
+}
+static int copy_aov_out(RenderCtx* c, size_t npix, const fw_aov* aov, cudaStream_t st) {
+    if (!aov) return FW_OK;
+    if (aov->albedo) FW_CUDA(cudaMemcpyAsync(aov->albedo, c->dn_planar, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
+    if (aov->normal) FW_CUDA(cudaMemcpyAsync(aov->normal, c->dn_planar + 3 * npix, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
+    if (aov->depth) FW_CUDA(cudaMemcpyAsync(aov->depth, c->dn_planar + 6 * npix, npix * sizeof(float), cudaMemcpyDeviceToHost, st));
+    if (aov->object) FW_CUDA(cudaMemcpyAsync(aov->object, c->aov.obj, npix * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    return FW_OK;
+}
+
+int fw_render_aov(fw_scene* sc, const fw_params* p, const fw_aov* aov, fw_stats* stats) {
+    return guarded([&]() -> int {
+        // every argument check comes before the first CUDA call
+        if (!sc || !p || !aov) return set_error(FW_ERR_ARG, "null argument");
+        int rc = check_image(p);
+        if (rc != FW_OK) return rc;
+        if (p->sample_count == 0) return set_error(FW_ERR_ARG, "sample_count must be >= 1");
+        if (!sc->committed || !sc->ctx) return set_error(FW_ERR_STATE, "fw_scene_commit must be called before rendering");
+        FW_CUDA(cudaSetDevice(sc->device));
+        const size_t npix = (size_t)p->width * p->height;
+        if ((rc = ensure_denoise_buffers(sc, npix)) != FW_OK) return rc;
+        RenderParamsHost hp;
+        memcpy(&hp, p, sizeof(hp));
+        const CameraRec cam = make_camera(hp);
+        const uint2 seed = make_uint2((uint32_t)p->seed, (uint32_t)(p->seed >> 32));
+        size_t cap = 0;
+        if ((rc = prepare_batches(sc, npix * p->sample_count, &cap)) != FW_OK) return rc;
+        RenderCtx* c = sc->ctx;
+        cudaStream_t st = c->stream;
+        RunTotals tot;
+        FW_CUDA(cudaMemsetAsync(c->d_rays, 0, sizeof(unsigned long long), st));
+        FW_CUDA(cudaEventRecord(c->ev_begin, st));
+        if ((rc = aov_pass(sc, p, cam, seed, cap, p->sample_begin, p->sample_count, c->dn_planar, st, tot)) != FW_OK) return rc;
+        if ((rc = finish_call(sc, st, tot, (uint64_t)npix * p->sample_count, stats)) != FW_OK) return rc;
+        if ((rc = copy_aov_out(c, npix, aov, st)) != FW_OK) return rc;
+        FW_CUDA(cudaStreamSynchronize(st));
+        return FW_OK;
+});
+}
+
+int fw_denoise_host(int device, uint32_t width, uint32_t height, const float* color, const float* variance, const float* albedo,
+                    const float* normal, const float* depth, const fw_denoise* dn, float* color_out, float* variance_out) {
+    return guarded([&]() -> int {
+        if (!color || !variance || !albedo || !normal || !depth || !dn || !color_out) return set_error(FW_ERR_ARG, "null argument");
+        if (width == 0 || height == 0) return set_error(FW_ERR_ARG, "width and height must be non-zero");
+        if ((uint64_t)width * height > 0x7fffffffull) return set_error(FW_ERR_ARG, "image too large");
+        if (!denoise_settings_ok(dn)) return FW_ERR_ARG;
+        int ndev = 0;
+        FW_CUDA(cudaGetDeviceCount(&ndev));
+        if (device < 0 || device >= ndev) return set_error(FW_ERR_CUDA, "no such CUDA device " + std::to_string(device));
+        FW_CUDA(cudaSetDevice(device));
+        const size_t npix = (size_t)width * height;
+        DevBuf dc, dv, da, dnrm, dd, cv0, cv1, nz, alb, oc, ov;
+        int rc;
+        if ((rc = dc.put(color, npix * 12)) != FW_OK || (rc = dv.put(variance, npix * 4)) != FW_OK || (rc = da.put(albedo, npix * 12)) != FW_OK ||
+            (rc = dnrm.put(normal, npix * 12)) != FW_OK || (rc = dd.put(depth, npix * 4)) != FW_OK || (rc = cv0.alloc(npix * 16)) != FW_OK ||
+            (rc = cv1.alloc(npix * 16)) != FW_OK || (rc = nz.alloc(npix * 16)) != FW_OK || (rc = alb.alloc(npix * 16)) != FW_OK ||
+            (rc = oc.alloc(npix * 12)) != FW_OK || (rc = ov.alloc(npix * 4)) != FW_OK)
+            return rc;
+        const unsigned grid = grid_for(npix, 256, 148 * 8);
+        launch_denoise_pack(dc.as<float>(), dv.as<float>(), da.as<float>(), dnrm.as<float>(), dd.as<float>(), (uint32_t)npix, cv0.as<float4>(),
+                            nz.as<float4>(), alb.as<float4>(), grid, nullptr);
+        float4* cv[2] = {cv0.as<float4>(), cv1.as<float4>()};
+        AovState g;
+        g.nz = nz.as<float4>(); g.alb = alb.as<float4>();
+        const int cur = denoise_iterations(dn, width, height, cv, g, nullptr, nullptr);
+        launch_denoise_unpack(cv[cur], (uint32_t)npix, oc.as<float>(), ov.as<float>(), grid, nullptr);
+        FW_CUDA(cudaGetLastError());
+        FW_CUDA(cudaDeviceSynchronize());
+        if ((rc = oc.get(color_out, npix * 12)) != FW_OK) return rc;
+        if (variance_out) return ov.get(variance_out, npix * 4);
+        return FW_OK;
+});
+}
+
+int fw_render_denoised(fw_scene* sc, const fw_params* p, const fw_denoise* dn, uint8_t* rgb_out, float* sum_out, float* denoised_out,
+                       float* variance_out, const fw_aov* aov, fw_stats* stats) {
+    return guarded([&]() -> int {
+        // every argument check comes before the first CUDA call
+        if (!sc || !p || !dn) return set_error(FW_ERR_ARG, "null argument");
+        int rc = check_image(p);
+        if (rc != FW_OK) return rc;
+        if (p->sample_begin != 0 || p->sample_count != p->samples || p->samples < 2)
+            return set_error(FW_ERR_ARG, "a denoised render owns the sample range: sample_begin must be 0, sample_count == samples and samples >= 2");
+        if (!denoise_settings_ok(dn)) return FW_ERR_ARG;
+        if (!sc->committed || !sc->ctx) return set_error(FW_ERR_STATE, "fw_scene_commit must be called before rendering");
+        FW_CUDA(cudaSetDevice(sc->device));
+        const size_t npix = (size_t)p->width * p->height;
+        if ((rc = ensure_sum_buffers(sc, npix)) != FW_OK || (rc = ensure_adaptive_buffers(sc, npix)) != FW_OK ||
+            (rc = ensure_denoise_buffers(sc, npix)) != FW_OK)
+            return rc;
+        RenderParamsHost hp;
+        memcpy(&hp, p, sizeof(hp));
+        const CameraRec cam = make_camera(hp);
+        const uint2 seed = make_uint2((uint32_t)p->seed, (uint32_t)(p->seed >> 32));
+        size_t cap = 0;
+        if ((rc = prepare_batches(sc, npix * p->samples, &cap)) != FW_OK) return rc;
+        RenderCtx* c = sc->ctx;
+        const AdaptiveState& A = c->adapt;
+        cudaStream_t st = c->stream;
+        const unsigned grid = grid_for(npix, 256, sc->sm_count * 8);
+        FW_CUDA(cudaMemsetAsync(c->d_sum, 0, npix * 3 * sizeof(float), st));
+        FW_CUDA(cudaMemsetAsync(A.m1, 0, npix * sizeof(double), st));
+        FW_CUDA(cudaMemsetAsync(A.m2, 0, npix * sizeof(double), st));
+        FW_CUDA(cudaMemsetAsync(A.count, 0, npix * sizeof(uint32_t), st));
+        RunTotals tot;
+        size_t ev_next = 0;
+        FW_CUDA(cudaMemsetAsync(c->d_rays, 0, sizeof(unsigned long long), st));
+        FW_CUDA(cudaEventRecord(c->ev_begin, st));
+        if ((rc = run_tiles(sc, p, cam, seed, cap, npix, nullptr, 0, p->samples, c->d_sum, &A, st, tot, ev_next)) != FW_OK) return rc;
+        const uint32_t aov_n = std::min(dn->aov_samples, p->samples);
+        if ((rc = aov_pass(sc, p, cam, seed, cap, 0, aov_n, c->dn_planar, st, tot)) != FW_OK) return rc;
+        launch_denoise_input(c->d_sum, A, (uint32_t)npix, p->samples, c->dn_cv[0], c->dn_var, grid, st);
+        tot.launches++;
+        const int cur = denoise_iterations(dn, p->width, p->height, c->dn_cv, c->aov, st, &tot.launches);
+        launch_denoise_unpack(c->dn_cv[cur], (uint32_t)npix, c->dn_color, nullptr, grid, st);
+        launch_resolve(c->dn_color, (uint32_t)npix, 1.0f, p->gamma, c->d_rgb, grid, st);
+        tot.launches += 2;
+        FW_CUDA(cudaGetLastError());
+        if ((rc = finish_call(sc, st, tot, (uint64_t)npix * p->samples, stats)) != FW_OK) return rc;
+        if (rgb_out) FW_CUDA(cudaMemcpyAsync(rgb_out, c->d_rgb, npix * 3, cudaMemcpyDeviceToHost, st));
+        if (sum_out) FW_CUDA(cudaMemcpyAsync(sum_out, c->d_sum, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
+        if (denoised_out) FW_CUDA(cudaMemcpyAsync(denoised_out, c->dn_color, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
+        if (variance_out) FW_CUDA(cudaMemcpyAsync(variance_out, c->dn_var, npix * sizeof(float), cudaMemcpyDeviceToHost, st));
+        if ((rc = copy_aov_out(c, npix, aov, st)) != FW_OK) return rc;
+        FW_CUDA(cudaStreamSynchronize(st));
         return FW_OK;
 });
 }

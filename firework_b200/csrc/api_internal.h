@@ -47,6 +47,14 @@ struct RenderCtx {
     size_t d_sum_pix = 0;
     AdaptiveState adapt{};       // fw_render_adaptive: moments, counts, active lists (~33 B per pixel), sized on first use
     size_t adapt_pix = 0;
+    // fw_render_aov / fw_render_denoised (~124 B per pixel), sized on first use: the AOV sums / guides, the filter's ping-pong
+    // (colour, variance), the planar AOV, variance and denoised-colour outputs
+    AovState aov{};
+    float4* dn_cv[2] = {nullptr, nullptr};
+    float* dn_planar = nullptr;    // albedo [3 npix], normal [3 npix], depth [npix]
+    float* dn_var = nullptr;       // [npix]
+    float* dn_color = nullptr;     // [3 npix]
+    size_t dn_pix = 0;
     unsigned long long* d_rays = nullptr;   // device-side ray tally of the current render call
     unsigned long long* h_rays = nullptr;   // pinned
     std::vector<cudaEvent_t> ev_pool;
@@ -117,6 +125,7 @@ namespace fw {
 int render_into(fw_scene* sc, const fw_params* p, float* d_sum, cudaStream_t st, fw_stats* stats);
 int ensure_sum_buffers(fw_scene* sc, size_t npix);   // ctx->d_sum / d_rgb sized for npix pixels
 int ensure_adaptive_buffers(fw_scene* sc, size_t npix);   // ctx->adapt sized for npix pixels
+int ensure_denoise_buffers(fw_scene* sc, size_t npix);    // ctx->aov / dn_* sized for npix pixels
 int commit_scene(fw_scene* sc, int device);          // fw_scene_commit
 void destroy_scene(fw_scene* sc);                    // fw_scene_destroy
 unsigned grid_for(size_t n, unsigned threads, unsigned max_blocks);

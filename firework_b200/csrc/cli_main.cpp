@@ -9,7 +9,8 @@
 // the fp32 sums and the number of samples done are saved after every chunk, and a later run with the same arguments continues
 // where the file stops (SURVEY.md §8f row 2; the reference's 3.36 h render had no way to resume).  --target-error E
 // [--min-samples N]: adaptive sampling (fw_render_adaptive), each pixel renders until its relative standard error is <= E,
-// with -s as the cap per pixel; it owns its sample schedule, so it is refused together with --checkpoint, --chunk or --gpus > 1.  The file format is shared
+// with -s as the cap per pixel; it owns its sample schedule, so it is refused together with --checkpoint, --chunk or --gpus > 1.
+// --denoise: a denoised render (fw_render_denoised, default filter settings), refused with the same flags and --target-error.  The file format is shared
 // with `python -m firework_b200 --checkpoint x.fwck` (firework_b200/progressive.py), so either driver finishes what the other began.
 // Links libfirework_b200.a: nothing here goes through Python.
 #include <zlib.h>
@@ -36,7 +37,8 @@ void usage(FILE* f) {
             "        --gpus <n>         render on n GPUs of this box (default 1)\n"
             "        --checkpoint <f>   resume from / save to this file after every chunk\n        --chunk <n>        samples per chunk (default: all)\n"
             "        --target-error <e> adaptive sampling: render each pixel until its relative standard error <= e (-s is the cap)\n"
-            "        --min-samples <n>  adaptive sampling: samples of the first round (default 16)\n    -h, --help\n");
+            "        --min-samples <n>  adaptive sampling: samples of the first round (default 16)\n"
+            "        --denoise          filter the render with first-hit albedo / normal / depth as guides (-s >= 2)\n    -h, --help\n");
 }
 [[noreturn]] void die(const std::string& msg) {
     fprintf(stderr, "error: %s\n", msg.c_str());
@@ -137,7 +139,7 @@ int main(int argc, char** argv) {
     std::string scene_file, name, output, checkpoint;
     long samples = -1, width = 960, height = 540, gpus = 1, chunk = 0, min_samples = 16;
     double target_error = -1.0;   // < 0: uniform render
-    bool adaptive = false;
+    bool adaptive = false, denoise = false;
     unsigned long long seed = 0;
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
@@ -163,6 +165,7 @@ int main(int argc, char** argv) {
         else if (is("--chunk", nullptr)) chunk = atol(value("--chunk").c_str());
         else if (is("--target-error", nullptr)) { target_error = atof(value("--target-error <e>").c_str()); adaptive = true; }
         else if (is("--min-samples", nullptr)) min_samples = atol(value("--min-samples <n>").c_str());
+        else if (a == "--denoise") denoise = true;
         else { usage(stderr); die("Found argument '" + a + "' which wasn't expected"); }
     }
     if (scene_file.empty() || samples < 0) {
@@ -175,6 +178,12 @@ int main(int argc, char** argv) {
         if (!checkpoint.empty() || chunk > 0) die("--target-error can not be combined with --checkpoint or --chunk");
         if (gpus > 1) die("--target-error renders on one GPU: it can not be combined with --gpus > 1");
         if (!(target_error >= 0.0) || !std::isfinite(target_error) || min_samples < 1) die("--target-error must be finite and >= 0, --min-samples >= 1");
+    }
+    if (denoise) {    // a denoised render owns its sample range and needs the moments of one device
+        if (!checkpoint.empty() || chunk > 0) die("--denoise can not be combined with --checkpoint or --chunk");
+        if (gpus > 1) die("--denoise renders on one GPU: it can not be combined with --gpus > 1");
+        if (adaptive) die("--denoise can not be combined with --target-error");
+        if (samples < 2) die("--denoise needs --samples >= 2");
     }
 
     // main.rs:25-26
@@ -222,7 +231,10 @@ int main(int argc, char** argv) {
     };
     fw_adaptive_result ares;
     memset(&ares, 0, sizeof ares);
-    if (adaptive) {
+    if (denoise) {
+        const fw_denoise dn{5, 4, 4.0f, 0.1f, 0.1f};   // engine.DENOISE_DEFAULTS
+        check(fw_render_denoised(scene, &p, &dn, rgb.data(), nullptr, nullptr, nullptr, nullptr, &st), "render");
+    } else if (adaptive) {
         fw_adaptive ad;
         ad.min_samples = (uint32_t)min_samples; ad.threshold = (float)target_error; ad.floor = 0.01f;   // engine.ADAPTIVE_FLOOR
         check(fw_render_adaptive(scene, &p, &ad, rgb.data(), nullptr, nullptr, nullptr, &st, &ares), "render");

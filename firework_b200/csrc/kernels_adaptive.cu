@@ -32,11 +32,13 @@ FW_DEV double relative_error(double A, double B, uint32_t n, double floor) {
     return sqrt(var / dn) / den;
 }
 
-// accumulate_kernel for a round's batch over list entries [pix0, pix0 + npix): the samples of a pixel in sample order into
-// its fp32 sum, and their luminance into its fp64 moments.
+// accumulate_kernel for a round's batch over list entries [pix0, pix0 + npix) (LIST), or over pixels [pix0, pix0 + npix) of the
+// image (the render stage of fw_render_denoised): the samples of a pixel in sample order into its fp32 sum, and their luminance
+// into its fp64 moments.
+template <bool LIST>
 __global__ void __launch_bounds__(256) accumulate_adaptive_kernel(float* __restrict__ sum, AdaptiveState a, PathState ps, Batch b) {
     for (uint32_t pl = blockIdx.x * blockDim.x + threadIdx.x; pl < b.npix; pl += gridDim.x * blockDim.x) {
-        const size_t pix = b.pixels[b.pix0 + pl];
+        const size_t pix = LIST ? (size_t)b.pixels[b.pix0 + pl] : (size_t)b.pix0 + pl;
         float r = sum[3 * pix], g = sum[3 * pix + 1], bl = sum[3 * pix + 2];
         double m1 = a.m1[pix], m2 = a.m2[pix];
         for (uint32_t s = 0; s < b.ns; ++s) {
@@ -145,7 +147,8 @@ __global__ void __launch_bounds__(256) resolve_adaptive_kernel(const float* __re
 
 // ---- launchers -------------------------------------------------------------------------------------------
 void launch_accumulate_adaptive(float* d_sum, const AdaptiveState& a, const PathState& ps, const Batch& b, unsigned blocks, cudaStream_t st) {
-    accumulate_adaptive_kernel<<<blocks, 256, 0, st>>>(d_sum, a, ps, b);
+    if (b.pixels) accumulate_adaptive_kernel<true><<<blocks, 256, 0, st>>>(d_sum, a, ps, b);
+    else accumulate_adaptive_kernel<false><<<blocks, 256, 0, st>>>(d_sum, a, ps, b);
 }
 void launch_adaptive_init(uint32_t* list, uint32_t n, unsigned blocks, cudaStream_t st) {
     adaptive_init_kernel<<<blocks, 256, 0, st>>>(list, n);

@@ -49,7 +49,7 @@ void launch_tally(const PathState& ps, unsigned long long* d_rays, cudaStream_t 
 void launch_resolve(const float* d_sum, uint32_t npix, float samples, float gamma, unsigned char* d_rgb, unsigned blocks,
                     cudaStream_t st);
 
-// Per-pixel state of an adaptive render (kernels_adaptive.cu), in the render context next to d_sum.
+// Per-pixel state of an adaptive or denoised render (kernels_adaptive.cu), in the render context next to d_sum.
 struct AdaptiveState {
     double* m1 = nullptr;           // [npix] sum of the samples' luminance
     double* m2 = nullptr;           // [npix] sum of its squares
@@ -68,6 +68,32 @@ int launch_converge_compact(const AdaptiveState& a, const uint32_t* list_in, uin
                             cudaStream_t st);
 void launch_resolve_adaptive(const float* d_sum, const AdaptiveState& a, uint32_t npix, float gamma, double floor, unsigned char* d_rgb,
                              unsigned blocks, cudaStream_t st);
+
+// First-hit feature buffers and the edge-aware filter (kernels_denoise.cu, DESIGN.md §12).
+struct AovState {
+    float4* nz = nullptr;     // [npix] sum, then mean, of (normal.xyz, depth)
+    float4* alb = nullptr;    // [npix] sum, then mean, of (albedo.rgb, 0)
+    int* obj = nullptr;       // [npix] first-hit object of the range's first sample, -1 on a miss
+};
+// Bounce-0 shade and miss queues -> (albedo, asfloat(object)) into atten row 0 and (normal, depth) into atten row 1, by path.
+void launch_aov_collect(const DeviceScene& S, const PathState& ps, cudaStream_t st);
+// Adds the batch's records into a.nz / a.alb in sample order; `first`: the batch starts at the range's first sample (object ids).
+void launch_aov_accumulate(const AovState& a, const PathState& ps, const Batch& b, bool first, unsigned blocks, cudaStream_t st);
+// Sums -> means (divided by `samples`); `planar` (nullable): albedo [3 npix], normal [3 npix], depth [npix], one after the other.
+void launch_aov_finalize(const AovState& a, uint32_t npix, float samples, float* planar, unsigned blocks, cudaStream_t st);
+struct DenoiseSigmas {
+    float luminance, depth, albedo;
+};
+// Planar colour / variance / guides -> (colour, variance) and the two guide float4 streams.
+void launch_denoise_pack(const float* color, const float* variance, const float* albedo, const float* normal, const float* depth,
+                         uint32_t npix, float4* cv, float4* nz, float4* alb, unsigned blocks, cudaStream_t st);
+// (sum / (float)n, variance of the mean luminance from the moments) per pixel into cv, and the variance to `variance` [npix].
+void launch_denoise_input(const float* d_sum, const AdaptiveState& a, uint32_t npix, uint32_t n, float4* cv, float* variance,
+                          unsigned blocks, cudaStream_t st);
+// One a-trous iteration at step 2^iteration.
+void launch_atrous(const float4* cv_in, const float4* nz, const float4* alb, uint32_t width, uint32_t height, uint32_t iteration,
+                   const DenoiseSigmas& sg, float4* cv_out, cudaStream_t st);
+void launch_denoise_unpack(const float4* cv, uint32_t npix, float* color, float* variance, unsigned blocks, cudaStream_t st);
 
 // probes (tests/ parity gates)
 void launch_primary_rays_probe(const CameraRec& cam, uint32_t width, uint32_t height, uint32_t sample, uint2 seed,

@@ -19,6 +19,25 @@ from .assets import load_asset
 # stop instead of chasing a relative error their displayed value can not show.
 ADAPTIVE_FLOOR = 0.01
 
+# Settings of the edge-aware a-trous filter (fw_denoise, DESIGN.md §12): iterations (step 2^i at iteration i, 1..10), the AOV
+# samples of a denoised render, and the luminance (SVGF's value), relative depth and albedo edge-stopping scales.
+DENOISE_DEFAULTS = {"iterations": 5, "aov_samples": 4, "sigma_luminance": 4.0, "sigma_depth": 0.1, "sigma_albedo": 0.1}
+
+
+def _denoise_settings(settings) -> N.FwDenoise:
+    unknown = set(settings) - set(DENOISE_DEFAULTS)
+    if unknown:
+        raise TypeError(f"unknown denoise settings: {sorted(unknown)}")
+    s = dict(DENOISE_DEFAULTS, **settings)
+    return N.FwDenoise(int(s["iterations"]), int(s["aov_samples"]), float(s["sigma_luminance"]), float(s["sigma_depth"]),
+                       float(s["sigma_albedo"]))
+
+
+def _aov_arrays(h, w):
+    aov = {"albedo": np.empty((h, w, 3), np.float32), "normal": np.empty((h, w, 3), np.float32),
+           "depth": np.empty((h, w), np.float32), "object": np.empty((h, w), np.int32)}
+    return aov, N.FwAov(*(N.ptr(aov[k]) for k in ("albedo", "normal", "depth", "object")))
+
 
 class NativeScene:
     """A committed fw_scene on one GPU."""
@@ -159,6 +178,31 @@ class NativeScene:
         d["active"] = [int(res.active[r]) for r in range(min(res.rounds, 32))]
         return rgb, s, counts, err, d
 
+    def render_aov(self, params: N.FwParams):
+        """fw_render_aov: per-pixel means over the params' sample range of what the primary rays hit first.  Returns
+        ({albedo (H,W,3), normal (H,W,3), depth (H,W) f32, object (H,W) i32 of the range's first sample}, stats dict)."""
+        aov, fa = _aov_arrays(params.height, params.width)
+        st = N.FwStats()
+        N.check(N.lib().fw_render_aov(self._h, C.byref(params), C.byref(fa), C.byref(st)))
+        return aov, st.as_dict()
+
+    def render_denoised(self, params: N.FwParams, want_rgb=True, want_sum=True, **settings):
+        """fw_render_denoised: a render of samples [0, params.samples) (params must cover that whole range, samples >= 2), the AOV
+        pass over the first `aov_samples` of them and the a-trous filter; `settings` override DENOISE_DEFAULTS.  Returns
+        (rgb (H,W,3) u8 of the denoised image | None, sum (H,W,3) f32 | None, denoised (H,W,3) f32 linear, variance (H,W) f32 of
+        the mean luminance before filtering, aov dict as render_aov, stats dict)."""
+        h, w = params.height, params.width
+        rgb = np.empty((h, w, 3), np.uint8) if want_rgb else None
+        s = np.empty((h, w, 3), np.float32) if want_sum else None
+        den = np.empty((h, w, 3), np.float32)
+        var = np.empty((h, w), np.float32)
+        aov, fa = _aov_arrays(h, w)
+        st = N.FwStats()
+        N.check(N.lib().fw_render_denoised(self._h, C.byref(params), C.byref(_denoise_settings(settings)),
+                                           N.ptr(rgb) if want_rgb else None, N.ptr(s) if want_sum else None, N.ptr(den), N.ptr(var),
+                                           C.byref(fa), C.byref(st)))
+        return rgb, s, den, var, aov, st.as_dict()
+
     def render_multi(self, params: N.FwParams, n_gpus: int, devices=None, reduce="nccl", want_rgb=True, want_sum=True):
         """fw_render_multi: the call's sample range split over `n_gpus` devices of this box (single process), sums
         combined on this scene's device by one NCCL reduce (`reduce="nccl"`) or by the fused peer-memory
@@ -288,6 +332,27 @@ def resolve_host(sums: np.ndarray, samples: int, gamma: float, device: int = 0) 
     out = np.empty(s.shape, np.uint8)
     N.check(N.lib().fw_resolve_host(device, N.ptr(s), s.size // 3, int(samples), C.c_float(gamma), N.ptr(out)))
     return out
+
+
+def denoise(color, variance, albedo, normal, depth, device: int = 0, **settings):
+    """fw_denoise_host: the a-trous filter of DESIGN.md §12 on host arrays — color (H,W,3) linear, variance (H,W) of the mean
+    luminance, albedo (H,W,3), normal (H,W,3), depth (H,W); `settings` override DENOISE_DEFAULTS (`aov_samples` is checked but
+    unused).  Returns (filtered colour (H,W,3), filtered variance (H,W)), float32."""
+    c = np.ascontiguousarray(color, np.float32)
+    if c.ndim != 3 or c.shape[2] != 3:
+        raise ValueError("color must be (height, width, 3)")
+    h, w = c.shape[:2]
+    v = np.ascontiguousarray(variance, np.float32)
+    a = np.ascontiguousarray(albedo, np.float32)
+    n = np.ascontiguousarray(normal, np.float32)
+    z = np.ascontiguousarray(depth, np.float32)
+    if v.shape != (h, w) or a.shape != c.shape or n.shape != c.shape or z.shape != (h, w):
+        raise ValueError("variance and depth must be (height, width), albedo and normal (height, width, 3)")
+    out_c = np.empty_like(c)
+    out_v = np.empty((h, w), np.float32)
+    N.check(N.lib().fw_denoise_host(int(device), w, h, N.ptr(c), N.ptr(v), N.ptr(a), N.ptr(n), N.ptr(z),
+                                    C.byref(_denoise_settings(settings)), N.ptr(out_c), N.ptr(out_v)))
+    return out_c, out_v
 
 
 def render_scene(scene, renderer, device: int = 0):

@@ -490,6 +490,17 @@ public:
     Renderer adaptive(float threshold, uint32_t min_samples = 16, float floor = 0.01f) const {
         Renderer c = *this; c.threshold_ = threshold; c.min_samples_ = min_samples; c.floor_ = floor; return c;
     }
+    // denoised render (fw_render_denoised, DESIGN.md §12): the render at samples_ spp (>= 2), first-hit albedo / normal / depth
+    // over its first aov_samples samples and an edge-aware a-trous filter; defaults as the Python mirror's Renderer.denoise
+    // (engine.DENOISE_DEFAULTS).  Single GPU and not with adaptive(): render() throws for those combinations.
+    Renderer denoise(uint32_t iterations = 5, uint32_t aov_samples = 4, float sigma_luminance = 4.0f, float sigma_depth = 0.1f,
+                     float sigma_albedo = 0.1f) const {
+        Renderer c = *this;
+        c.denoise_on_ = true;
+        c.denoise_.iterations = iterations; c.denoise_.aov_samples = aov_samples; c.denoise_.sigma_luminance = sigma_luminance;
+        c.denoise_.sigma_depth = sigma_depth; c.denoise_.sigma_albedo = sigma_albedo;
+        return c;
+    }
 
     fw_params params() const {
         fw_params p;
@@ -531,7 +542,11 @@ public:
         detail::check(fw_scene_commit(h, 0), "commit");
         const fw_params p = params();
         std::vector<uint8_t> rgb(width_ * height_ * 3);
-        if (threshold_ >= 0.0f) {
+        if (denoise_on_) {
+            if (gpus_ > 1) throw Error("a denoised render runs on one GPU: gpus(n > 1) and denoise() can not be combined");
+            if (threshold_ >= 0.0f) throw Error("adaptive() and denoise() can not be combined");
+            detail::check(fw_render_denoised(h, &p, &denoise_, rgb.data(), nullptr, nullptr, nullptr, nullptr, nullptr), "render");
+        } else if (threshold_ >= 0.0f) {
             if (gpus_ > 1) throw Error("adaptive sampling renders on one GPU: gpus(n > 1) and adaptive() can not be combined");
             fw_adaptive ad;
             ad.min_samples = min_samples_; ad.threshold = threshold_; ad.floor = floor_;
@@ -561,6 +576,8 @@ private:
     int gpus_ = 1;
     float threshold_ = -1.0f, floor_ = 0.01f;
     uint32_t min_samples_ = 16;
+    bool denoise_on_ = false;
+    fw_denoise denoise_{5, 4, 4.0f, 0.1f, 0.1f};
     std::string asset_dir_ = ".";
 };
 

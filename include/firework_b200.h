@@ -138,6 +138,54 @@ typedef struct fw_adaptive_result {
 int fw_render_adaptive(fw_scene* scene, const fw_params* params, const fw_adaptive* adaptive, uint8_t* rgb_out, float* sum_out,
                        uint32_t* count_out, float* error_out, fw_stats* stats, fw_adaptive_result* result);
 
+/* ---- denoised renders (no reference counterpart) ----------------------------------------------------------
+ * First-hit feature buffers (AOVs) and an edge-aware a-trous filter (the spatial filter of SVGF, Schied et al. 2017); the
+ * definitions, the filter's exact operation order and the measured results are in DESIGN.md §12.  Single GPU.
+ *
+ * fw_render_aov traces the primary ray of every (pixel, sample) of the sample range [sample_begin, sample_begin + sample_count)
+ * through the scene's own bounce-0 extend kernels and averages, per pixel and in sample order in fp32, what it hits:
+ *   albedo : the attenuation the first vertex applies, bit for bit what fw_render's shade kernel writes at bounce 0 (Lambertian
+ *            and isotropic: the texture at the hit; metal: its albedo; dielectric, emissive and a miss: (1, 1, 1));
+ *   normal : the normalised shading normal of the hit, (0, 0, 0) on a miss; the mean is not renormalised;
+ *   depth  : t * |d| along the (unnormalised) camera ray, 0 on a miss;
+ *   object : the object hit by sample sample_begin, -1 on a miss.
+ * The RNG is keyed by (pixel, sample, bounce): the AOV of sample s describes the first vertex of fw_render's path for sample s.
+ * Each fw_aov pointer is nullable: albedo / normal width*height*3 fp32, depth width*height fp32, object width*height int32. */
+typedef struct fw_aov {
+    float* albedo;
+    float* normal;
+    float* depth;
+    int32_t* object;
+} fw_aov;
+/* Filter settings; every field is checked: iterations 1..10 (step 2^i at iteration i), aov_samples >= 1 (the AOV samples of
+ * fw_render_denoised), each sigma finite and > 0.  Defaults (DESIGN.md §12): 5, 4, 4.0, 0.1, 0.1. */
+typedef struct fw_denoise {
+    uint32_t iterations;
+    uint32_t aov_samples;
+    float sigma_luminance;   /* luminance edge-stopping scale, in standard deviations of the 3x3-filtered variance */
+    float sigma_depth;       /* relative depth difference scale                                                    */
+    float sigma_albedo;      /* albedo difference scale                                                            */
+} fw_denoise;
+int fw_render_aov(fw_scene* scene, const fw_params* params, const fw_aov* aov, fw_stats* stats);
+/* The filter on host buffers (width*height pixels, row 0 = top), on `device`, needs no scene: color fp32 x3 (linear), variance
+ * fp32 (of the mean luminance), albedo x3, normal x3, depth.  color_out x3 receives the filtered colour, variance_out (nullable)
+ * the filtered variance.  Argument errors are reported before any CUDA call. */
+int fw_denoise_host(int device, uint32_t width, uint32_t height, const float* color, const float* variance, const float* albedo,
+                    const float* normal, const float* depth, const fw_denoise* settings, float* color_out, float* variance_out);
+/* A render followed by the AOV pass and the filter.  The call owns the sample range: sample_begin must be 0, sample_count ==
+ * samples and samples >= 2 (else FW_ERR_ARG).
+ *   1. every pixel renders samples [0, samples) with the kernels fw_render launches: sum_out equals fw_render's sums bit for
+ *      bit; per pixel the luminance moments A = sum Y, B = sum Y^2 (fp64, Y as in fw_render_adaptive) give the variance of the
+ *      mean v = max(0, (B - A (A / n)) / (n - 1)) / n, computed in fp64 and stored as fp32 (variance_out);
+ *   2. fw_render_aov over samples [0, min(aov_samples, samples));
+ *   3. fw_denoise_host's filter on (sum / (float)samples, v, the AOVs) -> denoised_out (linear fp32 x3); rgb_out u8 x3 is its
+ *      resolve at samples = 1 with params->gamma.
+ * Outputs are nullable; stats covers the whole call.  Argument errors (null scene / params / settings, the settings' ranges, the
+ * sample range) are reported before any CUDA call; fw_render_aov and fw_render_denoised give FW_ERR_STATE for an uncommitted
+ * scene. */
+int fw_render_denoised(fw_scene* scene, const fw_params* params, const fw_denoise* settings, uint8_t* rgb_out, float* sum_out,
+                       float* denoised_out, float* variance_out, const fw_aov* aov, fw_stats* stats);
+
 /* Device-resident variant for multi-GPU sharding: ADDS the sample range into d_sum (device pointer,
  * width*height*3 fp32, on the scene's device) on `cuda_stream` (a cudaStream_t, or NULL for the scene's own
  * stream) and returns once the work is enqueued and statistics are read back. */
