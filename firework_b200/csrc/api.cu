@@ -252,30 +252,47 @@ static int upload(fw_scene* sc, const std::vector<T>& host, const T** dev) {
     return FW_OK;
 }
 
-static void free_path_state(PathState& ps) {
-    auto fr = [](auto*& p) { if (p) { cudaFree(p); p = nullptr; } };
-    for (int i = 0; i < 2; ++i) { fr(ps.xo[i]); fr(ps.xd[i]); }
-    for (HitQueue& q : ps.hq) { fr(q.o); fr(q.d); fr(q.w); }
-    fr(ps.atten); fr(ps.radiance); fr(ps.counters); fr(ps.poison);
+// Each family of render-context buffers has one function that frees it; destroy_ctx and the ensure_* that grow a family
+// both call it, so a buffer added to a family is freed on both paths.
+template <class T>
+static void dev_free(T*& p) {
+    if (p) { cudaFree(p); p = nullptr; }
 }
-static void free_walk(RenderCtx* c) {
-    if (c->walk.tkey) cudaFree(c->walk.tkey);
-    if (c->walk.entries) cudaFree(c->walk.entries);
+// The path-state streams and the walk buffers sized with them.
+static void free_path_state(RenderCtx* c) {
+    PathState& ps = c->ps;
+    for (int i = 0; i < 2; ++i) { dev_free(ps.xo[i]); dev_free(ps.xd[i]); }
+    for (HitQueue& q : ps.hq) { dev_free(q.o); dev_free(q.d); dev_free(q.w); }
+    dev_free(ps.atten); dev_free(ps.radiance); dev_free(ps.counters); dev_free(ps.poison);
+    dev_free(c->walk.tkey); dev_free(c->walk.entries);
     c->walk = WalkAuxHost{};
     c->walk_key_cap = c->walk_ent_total = 0;
+    c->ps_cap = 0;
+}
+static void free_sums(RenderCtx* c) {
+    dev_free(c->d_sum); dev_free(c->d_rgb);
+    c->d_sum_pix = 0;
+}
+static void free_adaptive(RenderCtx* c) {
+    AdaptiveState& a = c->adapt;
+    dev_free(a.m1); dev_free(a.m2); dev_free(a.count); dev_free(a.err); dev_free(a.list[0]); dev_free(a.list[1]); dev_free(a.keep);
+    dev_free(a.block_base);
+    c->adapt_pix = 0;
+}
+static void free_denoise(RenderCtx* c) {
+    dev_free(c->aov.nz); dev_free(c->aov.alb); dev_free(c->aov.obj); dev_free(c->dn_cv[0]); dev_free(c->dn_cv[1]); dev_free(c->dn_planar);
+    dev_free(c->dn_var); dev_free(c->dn_color);
+    c->dn_pix = 0;
 }
 static void destroy_ctx(RenderCtx* c) {
     if (!c) return;
     cudaSetDevice(c->device);
-    auto fr = [](auto*& p) { if (p) { cudaFree(p); p = nullptr; } };
-    free_path_state(c->ps);
-    free_walk(c);
+    free_path_state(c);
     if (c->arena) cudaFree(c->arena);
     for (void* p : c->arena_retired) cudaFree(p);
-    fr(c->d_sum); fr(c->d_rgb);
-    fr(c->adapt.m1); fr(c->adapt.m2); fr(c->adapt.count); fr(c->adapt.err); fr(c->adapt.list[0]); fr(c->adapt.list[1]);
-    fr(c->adapt.keep); fr(c->adapt.block_base);
-    fr(c->aov.nz); fr(c->aov.alb); fr(c->aov.obj); fr(c->dn_cv[0]); fr(c->dn_cv[1]); fr(c->dn_planar); fr(c->dn_var); fr(c->dn_color);
+    free_sums(c);
+    free_adaptive(c);
+    free_denoise(c);
     if (c->h_rays) cudaFreeHost(c->h_rays);
     if (c->h_stage) cudaFreeHost(c->h_stage);
     if (c->d_rays) cudaFree(c->d_rays);
@@ -366,6 +383,26 @@ struct DevBuf {  // tiny RAII helper for probe staging buffers
         return FW_OK;
     }
     template <class T> T* as() { return reinterpret_cast<T*>(p); }
+};
+// The seven per-ray outputs of the first-hit probes (FirstHitOut) and their copy back to the caller.
+struct FirstHitBufs {
+    DevBuf buf[7];   // obj, prim, material, t, point, normal, uv
+    static constexpr size_t kBytes[7] = {4, 4, 4, 4, 12, 12, 8};   // per ray
+    int alloc(uint32_t n) {
+        for (int i = 0; i < 7; ++i)
+            if (int rc = buf[i].alloc(n * kBytes[i]); rc != FW_OK) return rc;
+        return FW_OK;
+    }
+    FirstHitOut out(unsigned long long* counters) {
+        return FirstHitOut{buf[0].as<int>(), buf[1].as<int>(), buf[2].as<int>(), buf[3].as<float>(), buf[4].as<float>(), buf[5].as<float>(),
+                           buf[6].as<float>(), counters};
+    }
+    int get(uint32_t n, int32_t* obj, int32_t* prim, int32_t* material, float* t, float* point, float* normal, float* uv) {
+        void* dst[7] = {obj, prim, material, t, point, normal, uv};
+        for (int i = 0; i < 7; ++i)
+            if (int rc = buf[i].get(dst[i], n * kBytes[i]); rc != FW_OK) return rc;
+        return FW_OK;
+    }
 };
 }  // namespace
 
@@ -792,17 +829,19 @@ int fw_camera(const fw_params* p, float out[24]) {
     return FW_OK;
 }
 // Idle render contexts keep their path state (gigabytes each) for the next scene; when an allocation fails they are the first
-// thing to give back.  Returns how many were destroyed.
+// thing to give back.  Returns how many were destroyed; the caller's current device stays current.
 static size_t destroy_idle_contexts() {
     std::lock_guard<std::mutex> lk(g_ctx_mutex);
-    std::vector<RenderCtx*> keep;
-    size_t n = 0;
-    for (RenderCtx* c : g_ctx_cache) {
-        if (c->in_use) keep.push_back(c);
-        else { destroy_ctx(c); ++n; }
-    }
+    std::vector<RenderCtx*> keep, idle;
+    for (RenderCtx* c : g_ctx_cache) (c->in_use ? keep : idle).push_back(c);
     g_ctx_cache.swap(keep);
-    return n;
+    if (!idle.empty()) {
+        int cur = 0;
+        cudaGetDevice(&cur);
+        for (RenderCtx* c : idle) destroy_ctx(c);   // each on its own device
+        cudaSetDevice(cur);
+    }
+    return idle.size();
 }
 int fw_release_cached_memory(void) {
     destroy_idle_contexts();
@@ -865,11 +904,7 @@ static int ensure_path_state(fw_scene* sc, size_t cap) {
     RenderCtx* ctx = sc->ctx;
     const size_t nseg_max = (size_t)sc->sm_count * FW_SEG_PER_SM_MAX;
     PathState& ps = ctx->ps;
-    if (ctx->ps_cap < cap || ctx->ps_nseg_max < nseg_max) {
-        free_path_state(ps);
-        free_walk(ctx);
-        ctx->ps_cap = 0;
-    }
+    if (ctx->ps_cap < cap || ctx->ps_nseg_max < nseg_max) free_path_state(ctx);
     cap = std::max(cap, ctx->ps_cap);   // streams added later for another scene get the context's full size
     // queue regions: nseg * seg_cap <= n + nseg * FW_TILE slots for any batch of n <= cap paths
     const size_t qcap = cap + (nseg_max + 1) * FW_TILE;
@@ -893,20 +928,20 @@ static int ensure_path_state(fw_scene* sc, size_t cap) {
         NEED(ps.hq[k].w, qcap);
     }
 #undef NEED
-    if (sc->plan.walk && sc->flat.has_top_mesh) {
-        // walk kernels on a scene with top-level meshes: one 64-bit key per queue slot, and an entry queue with room for
-        // every (ray, mesh) combination of a segment (n_top_meshes <= 8 is part of walk_ok)
+    if (sc->plan.walk) {
+        // walk kernels (only scenes with top-level meshes get them): one 64-bit key per queue slot, and an entry queue with
+        // room for every (ray, mesh) combination of a segment (n_top_meshes <= 8 is part of walk_ok)
         const size_t ent_per_seg_max = (size_t)sc->flat.n_top_meshes;
         const size_t ent_total = qcap * ent_per_seg_max;
         if (ctx->walk_key_cap < qcap) {
-            if (ctx->walk.tkey) cudaFree(ctx->walk.tkey);
-            ctx->walk.tkey = nullptr; ctx->walk_key_cap = 0;
+            dev_free(ctx->walk.tkey);
+            ctx->walk_key_cap = 0;
             FW_CUDA(cudaMalloc(&ctx->walk.tkey, qcap * sizeof(unsigned long long)));
             ctx->walk_key_cap = qcap;
         }
         if (ctx->walk_ent_total < ent_total) {
-            if (ctx->walk.entries) cudaFree(ctx->walk.entries);
-            ctx->walk.entries = nullptr; ctx->walk_ent_total = 0;
+            dev_free(ctx->walk.entries);
+            ctx->walk_ent_total = 0;
             FW_CUDA(cudaMalloc(&ctx->walk.entries, ent_total * sizeof(uint4)));
             ctx->walk_ent_total = ent_total;
         }
@@ -920,9 +955,24 @@ static int ensure_path_state(fw_scene* sc, size_t cap) {
     return FW_OK;
 }
 
-struct RunTotals {
-    uint64_t rays = 0, launches = 0, extend_launches = 0;
-    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> extend_events;
+// One render call of `p` on `sc`: what its batches share, and the totals that finish_call turns into fw_stats.  The camera and
+// seed are built here alone, for every render entry point and fw_primary_rays.
+struct CallFrame {
+    fw_scene* sc;
+    const fw_params* p;
+    CameraRec cam;
+    uint2 seed;
+    cudaStream_t st;
+    size_t cap = 0;        // paths per batch (begin_call)
+    uint64_t launches = 0, extend_launches = 0;
+    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> extend_events;   // fw_set_profiling: one pair per extend of run_batch
+    size_t ev_next = 0;    // next free event of the context's pool
+    CallFrame(fw_scene* s, const fw_params* q, cudaStream_t stream) : sc(s), p(q), st(stream) {
+        RenderParamsHost hp;
+        memcpy(&hp, q, sizeof(hp));
+        cam = make_camera(hp);
+        seed = make_uint2((uint32_t)q->seed, (uint32_t)(q->seed >> 32));
+    }
 };
 
 static int get_event(fw_scene* sc, size_t& next, cudaEvent_t* ev) {
@@ -972,60 +1022,65 @@ static int extend_bounce(fw_scene* sc, bool use_bvh, const Batch& b, uint2 seed,
     return FW_OK;
 }
 
-// One batch: raygen, up to FW_MAX_DEPTH+1 extend/shade rounds, accumulate into d_sum (and, for a round of an adaptive render,
+// Segment geometry of a batch of `paths` paths, its queue counters and the poison word zeroed.
+static int begin_batch(fw_scene* sc, size_t paths, cudaStream_t st) {
+    PathState& ps = sc->ctx->ps;
+    segment_geometry(sc, paths, &ps.nseg, &ps.seg_cap);
+    FW_CUDA(cudaMemsetAsync(ps.counters, 0, sizeof(uint32_t) * (FW_MAX_DEPTH + 2) * FW_NUM_QUEUES * (size_t)ps.nseg, st));
+    FW_CUDA(cudaMemsetAsync(ps.poison, 0, sizeof(uint32_t), st));
+    return FW_OK;
+}
+
+// One batch: raygen, up to FW_MAX_DEPTH+1 extend/shade rounds, accumulate into d_sum (and, for an adaptive or denoised render,
 // into the moments and counts of `adapt`).
-static int run_batch(fw_scene* sc, const CameraRec& cam, const Batch& b, uint2 seed, bool use_bvh, float* d_sum,
-                     const AdaptiveState* adapt, cudaStream_t st, RunTotals& tot, size_t& ev_next) {
+static int run_batch(CallFrame& f, const Batch& b, float* d_sum, const AdaptiveState* adapt) {
+    fw_scene* sc = f.sc;
+    const cudaStream_t st = f.st;
     PathState& ps = sc->ctx->ps;
     const DeviceScene& S = sc->dscene;
-    uint32_t N = b.npix * b.ns;
-    segment_geometry(sc, N, &ps.nseg, &ps.seg_cap);
-    const size_t counter_bytes = sizeof(uint32_t) * (FW_MAX_DEPTH + 2) * FW_NUM_QUEUES * (size_t)ps.nseg;
-    FW_CUDA(cudaMemsetAsync(ps.counters, 0, counter_bytes, st));
-    FW_CUDA(cudaMemsetAsync(ps.poison, 0, sizeof(uint32_t), st));
+    int rc = begin_batch(sc, (size_t)b.npix * b.ns, st);
+    if (rc != FW_OK) return rc;
     unsigned sm = (unsigned)sc->sm_count;
-    launch_raygen(cam, b, seed, ps, st);
-    tot.launches++;
+    launch_raygen(f.cam, b, f.seed, ps, st);
+    f.launches++;
     FW_STAGE("raygen", 0);
     for (uint32_t bounce = 0; bounce <= (uint32_t)FW_MAX_DEPTH; ++bounce) {
         cudaEvent_t e0 = nullptr, e1 = nullptr;
         if (sc->profiling) {
-            int rc;
-            if ((rc = get_event(sc, ev_next, &e0)) != FW_OK || (rc = get_event(sc, ev_next, &e1)) != FW_OK) return rc;
+            if ((rc = get_event(sc, f.ev_next, &e0)) != FW_OK || (rc = get_event(sc, f.ev_next, &e1)) != FW_OK) return rc;
             FW_CUDA(cudaEventRecord(e0, st));
         }
-        const int rc = extend_bounce(sc, use_bvh, b, seed, bounce, st, tot.launches);
-        if (rc != FW_OK) return rc;
+        if ((rc = extend_bounce(sc, f.p->use_bvh != 0, b, f.seed, bounce, st, f.launches)) != FW_OK) return rc;
         if (sc->profiling) {
             FW_CUDA(cudaEventRecord(e1, st));
-            tot.extend_events.emplace_back(e0, e1);
+            f.extend_events.emplace_back(e0, e1);
         }
-        tot.extend_launches++;
+        f.extend_launches++;
         FW_STAGE("extend", bounce);
         if (!sc->miss_is_zero) {
             launch_miss(S, ps, bounce, sc->env_black, st);
-            tot.launches++;
+            f.launches++;
             FW_STAGE("miss", bounce);
         }
         if (sc->mat_present[MAT_EMISSIVE]) {
             launch_shade_emissive(S, ps, bounce, st);
-            tot.launches++;
+            f.launches++;
             FW_STAGE("shade emissive", bounce);
         }
         if (bounce < (uint32_t)FW_MAX_DEPTH) {
             for (int mat : {MAT_LAMBERTIAN, MAT_METAL, MAT_DIELECTRIC, MAT_ISOTROPIC})
                 if (sc->mat_present[mat]) {
-                    launch_shade_scatter(mat, S, ps, b, seed, bounce, st);
-                    tot.launches++;
+                    launch_shade_scatter(mat, S, ps, b, f.seed, bounce, st);
+                    f.launches++;
                     FW_STAGE(mat == MAT_LAMBERTIAN ? "shade lambertian" : mat == MAT_METAL ? "shade metal" : mat == MAT_DIELECTRIC ? "shade dielectric" : "shade isotropic", bounce);
                 }
         }
     }
     if (adapt) launch_accumulate_adaptive(d_sum, *adapt, ps, b, grid_for(b.npix, 256, sm * 8), st);
     else launch_accumulate(d_sum, ps, b, grid_for(b.npix, 256, sm * 8), st);
-    tot.launches++;
+    f.launches++;
     launch_tally(ps, sc->ctx->d_rays, st);
-    tot.launches++;
+    f.launches++;
     FW_STAGE("accumulate / tally", 0);
 #undef FW_STAGE
     FW_CUDA(cudaGetLastError());
@@ -1053,15 +1108,10 @@ static int prepare_batches(fw_scene* sc, size_t paths, size_t* cap_out) {
         size_t free_b = 0, total_b = 0;
         FW_CUDA(cudaMemGetInfo(&free_b, &total_b));
         double budget = 0.8 * ((double)free_b + (double)sc->ctx->ps_cap * per_path);
-        if ((double)cap * per_path > budget) {   // idle contexts of earlier scenes hold path state nobody is using
-            int cur = 0;
-            cudaGetDevice(&cur);
-            const size_t n_freed = destroy_idle_contexts();
-            cudaSetDevice(cur);
-            if (n_freed) {
-                FW_CUDA(cudaMemGetInfo(&free_b, &total_b));
-                budget = 0.8 * ((double)free_b + (double)sc->ctx->ps_cap * per_path);
-            }
+        // idle contexts of earlier scenes hold path state nobody is using
+        if ((double)cap * per_path > budget && destroy_idle_contexts() > 0) {
+            FW_CUDA(cudaMemGetInfo(&free_b, &total_b));
+            budget = 0.8 * ((double)free_b + (double)sc->ctx->ps_cap * per_path);
         }
         while (cap > ((size_t)1 << 22) && (double)cap * per_path > budget) cap >>= 1;
     }
@@ -1069,16 +1119,10 @@ static int prepare_batches(fw_scene* sc, size_t paths, size_t* cap_out) {
         rc = ensure_path_state(sc, cap);
         if (rc == FW_OK || cudaPeekAtLastError() != cudaErrorMemoryAllocation) break;
         cudaGetLastError();
-        free_path_state(sc->ctx->ps);
-        free_walk(sc->ctx);
-        sc->ctx->ps_cap = 0;
+        free_path_state(sc->ctx);
         if (!freed_idle) {
             freed_idle = true;
-            int cur = 0;
-            cudaGetDevice(&cur);
-            const size_t n = destroy_idle_contexts();
-            cudaSetDevice(cur);
-            if (n > 0) continue;   // same size again
+            if (destroy_idle_contexts() > 0) continue;   // same size again
         }
         if (cap <= ((size_t)1 << 20)) break;
         cap >>= 1;
@@ -1101,58 +1145,67 @@ static Batch make_batch(uint32_t pix0, uint32_t npix, uint32_t s0, uint32_t ns, 
     return b;
 }
 
+// Opens the device work of a call of `paths` paths in all: the batch cap and path state (prepare_batches), the ray tally
+// zeroed and ev_begin recorded.  finish_call closes it.
+static int begin_call(CallFrame& f, size_t paths) {
+    const int rc = prepare_batches(f.sc, paths, &f.cap);
+    if (rc != FW_OK) return rc;
+    FW_CUDA(cudaMemsetAsync(f.sc->ctx->d_rays, 0, sizeof(unsigned long long), f.st));
+    FW_CUDA(cudaEventRecord(f.sc->ctx->ev_begin, f.st));
+    return FW_OK;
+}
+
 // Samples [s_begin, s_begin + s_count) of `npix` pixels — the image's pixels 0 .. npix-1, or the first npix entries of a pixel
-// list — in batches of at most `cap` paths: pixel tiles outer, sample chunks inner, so every pixel's samples are accumulated
-// in sample order.
-static int run_tiles(fw_scene* sc, const fw_params* p, const CameraRec& cam, uint2 seed, size_t cap, size_t npix, const uint32_t* pixels,
-                     uint32_t s_begin, uint32_t s_count, float* d_sum, const AdaptiveState* adapt, cudaStream_t st, RunTotals& tot,
-                     size_t& ev_next) {
-    int rc;
-    size_t tile = std::min(npix, cap);
+// list — in batches of at most f.cap paths: pixel tiles outer, sample chunks inner, so every pixel's samples are accumulated
+// in sample order.  body(batch, first) runs each batch; `first`: the batch starts at sample s_begin.
+template <class Body>
+static int for_each_batch(const CallFrame& f, size_t npix, const uint32_t* pixels, uint32_t s_begin, uint32_t s_count, Body&& body) {
+    const size_t tile = std::min(npix, f.cap);
     for (size_t pix0 = 0; pix0 < npix; pix0 += tile) {
-        size_t np = std::min(tile, npix - pix0);
-        uint32_t chunk = (uint32_t)std::max<size_t>(1, cap / np);
+        const size_t np = std::min(tile, npix - pix0);
+        const uint32_t chunk = (uint32_t)std::max<size_t>(1, f.cap / np);
         for (uint32_t s = 0; s < s_count; s += chunk) {
-            const Batch b = make_batch((uint32_t)pix0, (uint32_t)np, s_begin + s, std::min(chunk, s_count - s), p->width, p->height, pixels);
-            if ((rc = run_batch(sc, cam, b, seed, p->use_bvh != 0, d_sum, adapt, st, tot, ev_next)) != FW_OK) return rc;
+            const Batch b = make_batch((uint32_t)pix0, (uint32_t)np, s_begin + s, std::min(chunk, s_count - s), f.p->width, f.p->height, pixels);
+            const int rc = body(b, s == 0);
+            if (rc != FW_OK) return rc;
         }
     }
     return FW_OK;
 }
 
-// The AOV pass (DESIGN.md §12) over samples [s_begin, s_begin + s_count) of every pixel, with run_tiles' batching: raygen and
+// run_batch over every batch of those samples.
+static int run_tiles(CallFrame& f, size_t npix, const uint32_t* pixels, uint32_t s_begin, uint32_t s_count, float* d_sum,
+                     const AdaptiveState* adapt) {
+    return for_each_batch(f, npix, pixels, s_begin, s_count, [&](const Batch& b, bool) { return run_batch(f, b, d_sum, adapt); });
+}
+
+// The AOV pass (DESIGN.md §12) over samples [s_begin, s_begin + s_count) of every pixel, with the render's batching: raygen and
 // the bounce-0 extend of each batch, its records collected and added in sample order.  Leaves the means in ctx->aov (and,
 // when `planar` is set, the planar albedo / normal / depth there).
-static int aov_pass(fw_scene* sc, const fw_params* p, const CameraRec& cam, uint2 seed, size_t cap, uint32_t s_begin, uint32_t s_count,
-                    float* planar, cudaStream_t st, RunTotals& tot) {
+static int aov_pass(CallFrame& f, uint32_t s_begin, uint32_t s_count, float* planar) {
+    fw_scene* sc = f.sc;
     RenderCtx* c = sc->ctx;
     PathState& ps = c->ps;
-    const size_t npix = (size_t)p->width * p->height;
+    const cudaStream_t st = f.st;
+    const size_t npix = (size_t)f.p->width * f.p->height;
     const unsigned grid = grid_for(npix, 256, sc->sm_count * 8);
     FW_CUDA(cudaMemsetAsync(c->aov.nz, 0, npix * sizeof(float4), st));
     FW_CUDA(cudaMemsetAsync(c->aov.alb, 0, npix * sizeof(float4), st));
-    const size_t tile = std::min(npix, cap);
-    for (size_t pix0 = 0; pix0 < npix; pix0 += tile) {
-        const size_t np = std::min(tile, npix - pix0);
-        const uint32_t chunk = (uint32_t)std::max<size_t>(1, cap / np);
-        for (uint32_t s = 0; s < s_count; s += chunk) {
-            const Batch b = make_batch((uint32_t)pix0, (uint32_t)np, s_begin + s, std::min(chunk, s_count - s), p->width, p->height, nullptr);
-            segment_geometry(sc, (size_t)b.npix * b.ns, &ps.nseg, &ps.seg_cap);
-            FW_CUDA(cudaMemsetAsync(ps.counters, 0, sizeof(uint32_t) * (FW_MAX_DEPTH + 2) * FW_NUM_QUEUES * (size_t)ps.nseg, st));
-            FW_CUDA(cudaMemsetAsync(ps.poison, 0, sizeof(uint32_t), st));
-            launch_raygen(cam, b, seed, ps, st);
-            int rc = extend_bounce(sc, p->use_bvh != 0, b, seed, 0, st, tot.launches);
-            if (rc != FW_OK) return rc;
-            tot.extend_launches++;
-            launch_aov_collect(sc->dscene, ps, st);
-            launch_aov_accumulate(c->aov, ps, b, s == 0, grid_for(b.npix, 256, sc->sm_count * 8), st);
-            launch_tally(ps, c->d_rays, st);
-            tot.launches += 4;
-            if ((rc = sync_stage(st, "AOV pass", 0)) != FW_OK) return rc;
-        }
-    }
+    const int rc = for_each_batch(f, npix, nullptr, s_begin, s_count, [&](const Batch& b, bool first) {
+        int rc = begin_batch(sc, (size_t)b.npix * b.ns, st);
+        if (rc != FW_OK) return rc;
+        launch_raygen(f.cam, b, f.seed, ps, st);
+        if ((rc = extend_bounce(sc, f.p->use_bvh != 0, b, f.seed, 0, st, f.launches)) != FW_OK) return rc;
+        f.extend_launches++;
+        launch_aov_collect(sc->dscene, ps, st);
+        launch_aov_accumulate(c->aov, ps, b, first, grid_for(b.npix, 256, sc->sm_count * 8), st);
+        launch_tally(ps, c->d_rays, st);
+        f.launches += 4;
+        return sync_stage(st, "AOV pass", 0);
+    });
+    if (rc != FW_OK) return rc;
     launch_aov_finalize(c->aov, (uint32_t)npix, (float)s_count, planar, grid, st);
-    tot.launches++;
+    f.launches++;
     FW_CUDA(cudaGetLastError());
     return FW_OK;
 }
@@ -1176,23 +1229,23 @@ static bool denoise_settings_ok(const fw_denoise* dn) {
     return true;
 }
 
-// Closes the device work of one call (ev_begin was recorded at its start): ray tally, event times -> stats.  Synchronises `st`.
-static int finish_call(fw_scene* sc, cudaStream_t st, RunTotals& tot, uint64_t samples, fw_stats* stats) {
-    FW_CUDA(cudaEventRecord(sc->ctx->ev_end, st));
-    FW_CUDA(cudaMemcpyAsync(sc->ctx->h_rays, sc->ctx->d_rays, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    FW_CUDA(cudaStreamSynchronize(st));
-    tot.rays = *sc->ctx->h_rays;
+// Closes the device work of a call opened by begin_call: ray tally, event times -> stats.  Synchronises the call's stream.
+static int finish_call(CallFrame& f, uint64_t samples, fw_stats* stats) {
+    RenderCtx* c = f.sc->ctx;
+    FW_CUDA(cudaEventRecord(c->ev_end, f.st));
+    FW_CUDA(cudaMemcpyAsync(c->h_rays, c->d_rays, sizeof(unsigned long long), cudaMemcpyDeviceToHost, f.st));
+    FW_CUDA(cudaStreamSynchronize(f.st));
     if (stats) {
         memset(stats, 0, sizeof(*stats));
         stats->samples = samples;
-        stats->rays = tot.rays;
-        stats->launches = tot.launches;
-        stats->extend_launches = tot.extend_launches;
+        stats->rays = *c->h_rays;
+        stats->launches = f.launches;
+        stats->extend_launches = f.extend_launches;
         float ms = 0;
-        FW_CUDA(cudaEventElapsedTime(&ms, sc->ctx->ev_begin, sc->ctx->ev_end));
+        FW_CUDA(cudaEventElapsedTime(&ms, c->ev_begin, c->ev_end));
         stats->ms_device = ms;
         double me = 0;
-        for (auto& pr : tot.extend_events) {
+        for (auto& pr : f.extend_events) {
             float m = 0;
             FW_CUDA(cudaEventElapsedTime(&m, pr.first, pr.second));
             me += m;
@@ -1202,46 +1255,49 @@ static int finish_call(fw_scene* sc, cudaStream_t st, RunTotals& tot, uint64_t s
     return FW_OK;
 }
 
+// Width, height and samples non-zero and fewer than 2^31 pixels: the image checks of every render entry point.
+static int check_image(const fw_params* p) {
+    if (!p || p->width == 0 || p->height == 0 || p->samples == 0) return set_error(FW_ERR_ARG, "width, height and samples must be non-zero");
+    if ((uint64_t)p->width * p->height > 0x7fffffffull) return set_error(FW_ERR_ARG, "image too large");
+    return FW_OK;
+}
+
+// d_sum and the luminance moments and sample counts of `npix` pixels zeroed: the start of an adaptive or denoised render.
+static int zero_moments(RenderCtx* c, size_t npix, cudaStream_t st) {
+    FW_CUDA(cudaMemsetAsync(c->d_sum, 0, npix * 3 * sizeof(float), st));
+    FW_CUDA(cudaMemsetAsync(c->adapt.m1, 0, npix * sizeof(double), st));
+    FW_CUDA(cudaMemsetAsync(c->adapt.m2, 0, npix * sizeof(double), st));
+    FW_CUDA(cudaMemsetAsync(c->adapt.count, 0, npix * sizeof(uint32_t), st));
+    return FW_OK;
+}
+
 int fw::render_into(fw_scene* sc, const fw_params* p, float* d_sum, cudaStream_t st, fw_stats* stats) {
     if (!sc->committed) return set_error(FW_ERR_STATE, "fw_scene_commit must be called before rendering");
-    if (!p || p->width == 0 || p->height == 0 || p->samples == 0)
-        return set_error(FW_ERR_ARG, "width, height and samples must be non-zero");
-    if ((uint64_t)p->width * p->height > 0x7fffffffull) return set_error(FW_ERR_ARG, "image too large");
-    FW_CUDA(cudaSetDevice(sc->device));
-    RenderParamsHost hp;
-    memcpy(&hp, p, sizeof(hp));
-    CameraRec cam = make_camera(hp);
-    uint2 seed = make_uint2((uint32_t)p->seed, (uint32_t)(p->seed >> 32));
-    size_t npix = (size_t)p->width * p->height;
-    size_t cap = 0;
-    int rc = prepare_batches(sc, npix * std::max<uint32_t>(p->sample_count, 1), &cap);
+    int rc = check_image(p);
     if (rc != FW_OK) return rc;
-    RunTotals tot;
-    size_t ev_next = 0;
-    FW_CUDA(cudaMemsetAsync(sc->ctx->d_rays, 0, sizeof(unsigned long long), st));
-    FW_CUDA(cudaEventRecord(sc->ctx->ev_begin, st));
-    if ((rc = run_tiles(sc, p, cam, seed, cap, npix, nullptr, p->sample_begin, p->sample_count, d_sum, nullptr, st, tot, ev_next)) != FW_OK)
+    FW_CUDA(cudaSetDevice(sc->device));
+    const size_t npix = (size_t)p->width * p->height;
+    CallFrame f(sc, p, st);
+    if ((rc = begin_call(f, npix * std::max<uint32_t>(p->sample_count, 1))) != FW_OK ||
+        (rc = run_tiles(f, npix, nullptr, p->sample_begin, p->sample_count, d_sum, nullptr)) != FW_OK)
         return rc;
-    return finish_call(sc, st, tot, (uint64_t)npix * p->sample_count, stats);
+    return finish_call(f, (uint64_t)npix * p->sample_count, stats);
 }
 
 int fw::ensure_sum_buffers(fw_scene* sc, size_t npix) {
-    if (sc->ctx->d_sum_pix >= npix) return FW_OK;
-    if (sc->ctx->d_sum) cudaFree(sc->ctx->d_sum);
-    if (sc->ctx->d_rgb) cudaFree(sc->ctx->d_rgb);
-    sc->ctx->d_sum = nullptr; sc->ctx->d_rgb = nullptr; sc->ctx->d_sum_pix = 0;
-    FW_CUDA(cudaMalloc(&sc->ctx->d_sum, npix * 3 * sizeof(float)));
-    FW_CUDA(cudaMalloc(&sc->ctx->d_rgb, npix * 3));
-    sc->ctx->d_sum_pix = npix;
+    RenderCtx* c = sc->ctx;
+    if (c->d_sum_pix >= npix) return FW_OK;
+    free_sums(c);
+    FW_CUDA(cudaMalloc(&c->d_sum, npix * 3 * sizeof(float)));
+    FW_CUDA(cudaMalloc(&c->d_rgb, npix * 3));
+    c->d_sum_pix = npix;
     return FW_OK;
 }
 int fw::ensure_adaptive_buffers(fw_scene* sc, size_t npix) {
     RenderCtx* c = sc->ctx;
     if (c->adapt_pix >= npix) return FW_OK;
     AdaptiveState& a = c->adapt;
-    auto fr = [](auto*& p) { if (p) { cudaFree(p); p = nullptr; } };
-    fr(a.m1); fr(a.m2); fr(a.count); fr(a.err); fr(a.list[0]); fr(a.list[1]); fr(a.keep); fr(a.block_base);
-    c->adapt_pix = 0;
+    free_adaptive(c);
     FW_CUDA(cudaMalloc(&a.m1, npix * sizeof(double)));
     FW_CUDA(cudaMalloc(&a.m2, npix * sizeof(double)));
     FW_CUDA(cudaMalloc(&a.count, npix * sizeof(uint32_t)));
@@ -1256,9 +1312,7 @@ int fw::ensure_adaptive_buffers(fw_scene* sc, size_t npix) {
 int fw::ensure_denoise_buffers(fw_scene* sc, size_t npix) {
     RenderCtx* c = sc->ctx;
     if (c->dn_pix >= npix) return FW_OK;
-    auto fr = [](auto*& p) { if (p) { cudaFree(p); p = nullptr; } };
-    fr(c->aov.nz); fr(c->aov.alb); fr(c->aov.obj); fr(c->dn_cv[0]); fr(c->dn_cv[1]); fr(c->dn_planar); fr(c->dn_var); fr(c->dn_color);
-    c->dn_pix = 0;
+    free_denoise(c);
     FW_CUDA(cudaMalloc(&c->aov.nz, npix * sizeof(float4)));
     FW_CUDA(cudaMalloc(&c->aov.alb, npix * sizeof(float4)));
     FW_CUDA(cudaMalloc(&c->aov.obj, npix * sizeof(int)));
@@ -1270,8 +1324,6 @@ int fw::ensure_denoise_buffers(fw_scene* sc, size_t npix) {
     c->dn_pix = npix;
     return FW_OK;
 }
-int fw::commit_scene(fw_scene* sc, int device) { return fw_scene_commit(sc, device); }
-void fw::destroy_scene(fw_scene* sc) { fw_scene_destroy(sc); }
 
 extern "C" {
 
@@ -1341,8 +1393,8 @@ int fw_render_adaptive(fw_scene* sc, const fw_params* p, const fw_adaptive* ad, 
     return guarded([&]() -> int {
         // every argument check comes before the first CUDA call
         if (!sc || !p || !ad) return set_error(FW_ERR_ARG, "null argument");
-        if (p->width == 0 || p->height == 0 || p->samples == 0) return set_error(FW_ERR_ARG, "width, height and samples must be non-zero");
-        if ((uint64_t)p->width * p->height > 0x7fffffffull) return set_error(FW_ERR_ARG, "image too large");
+        int rc = check_image(p);
+        if (rc != FW_OK) return rc;
         if (p->sample_begin != 0 || p->sample_count != p->samples)
             return set_error(FW_ERR_ARG, "an adaptive render owns the sample range: sample_begin must be 0 and sample_count == samples (the cap)");
         if (ad->min_samples == 0) return set_error(FW_ERR_ARG, "min_samples must be >= 1");
@@ -1351,40 +1403,28 @@ int fw_render_adaptive(fw_scene* sc, const fw_params* p, const fw_adaptive* ad, 
         if (!sc->committed || !sc->ctx) return set_error(FW_ERR_STATE, "fw_scene_commit must be called before rendering");
         FW_CUDA(cudaSetDevice(sc->device));
         const size_t npix = (size_t)p->width * p->height;
-        int rc;
-        if ((rc = ensure_sum_buffers(sc, npix)) != FW_OK || (rc = ensure_adaptive_buffers(sc, npix)) != FW_OK) return rc;
-        RenderParamsHost hp;
-        memcpy(&hp, p, sizeof(hp));
-        const CameraRec cam = make_camera(hp);
-        const uint2 seed = make_uint2((uint32_t)p->seed, (uint32_t)(p->seed >> 32));
-        size_t cap = 0;
-        if ((rc = prepare_batches(sc, npix * p->samples, &cap)) != FW_OK) return rc;
         RenderCtx* c = sc->ctx;
         const AdaptiveState& A = c->adapt;
-        cudaStream_t st = c->stream;
+        CallFrame f(sc, p, c->stream);
+        const cudaStream_t st = f.st;
+        if ((rc = ensure_sum_buffers(sc, npix)) != FW_OK || (rc = ensure_adaptive_buffers(sc, npix)) != FW_OK ||
+            (rc = zero_moments(c, npix, st)) != FW_OK || (rc = begin_call(f, npix * p->samples)) != FW_OK)
+            return rc;
         const unsigned grid = grid_for(npix, 256, sc->sm_count * 8);
         const double threshold = ad->threshold, floor = ad->floor;
-        FW_CUDA(cudaMemsetAsync(c->d_sum, 0, npix * 3 * sizeof(float), st));
-        FW_CUDA(cudaMemsetAsync(A.m1, 0, npix * sizeof(double), st));
-        FW_CUDA(cudaMemsetAsync(A.m2, 0, npix * sizeof(double), st));
-        FW_CUDA(cudaMemsetAsync(A.count, 0, npix * sizeof(uint32_t), st));
-        RunTotals tot;
-        size_t ev_next = 0;
-        FW_CUDA(cudaMemsetAsync(c->d_rays, 0, sizeof(unsigned long long), st));
-        FW_CUDA(cudaEventRecord(c->ev_begin, st));
         launch_adaptive_init(A.list[0], (uint32_t)npix, grid, st);
-        tot.launches++;
+        f.launches++;
         fw_adaptive_result res;
         memset(&res, 0, sizeof(res));
         uint32_t active = (uint32_t)npix, n_prev = 0, n = std::min(ad->min_samples, p->samples);
         int cur = 0;
         for (;;) {
-            if ((rc = run_tiles(sc, p, cam, seed, cap, active, A.list[cur], n_prev, n - n_prev, c->d_sum, &A, st, tot, ev_next)) != FW_OK) return rc;
+            if ((rc = run_tiles(f, active, A.list[cur], n_prev, n - n_prev, c->d_sum, &A)) != FW_OK) return rc;
             if (res.rounds < 32) res.active[res.rounds] = active;
             res.rounds++;
             res.samples += (uint64_t)active * (n - n_prev);
             if (n == p->samples) break;   // the cap: nothing left to decide
-            tot.launches += launch_converge_compact(A, A.list[cur], active, threshold, floor, A.list[cur ^ 1], st);
+            f.launches += launch_converge_compact(A, A.list[cur], active, threshold, floor, A.list[cur ^ 1], st);
             FW_CUDA(cudaGetLastError());
             FW_CUDA(cudaMemcpyAsync(&active, A.block_base + adaptive_blocks(active), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
             FW_CUDA(cudaStreamSynchronize(st));
@@ -1395,8 +1435,8 @@ int fw_render_adaptive(fw_scene* sc, const fw_params* p, const fw_adaptive* ad, 
         }
         launch_resolve_adaptive(c->d_sum, A, (uint32_t)npix, p->gamma, floor, c->d_rgb, grid, st);
         FW_CUDA(cudaGetLastError());
-        tot.launches++;
-        if ((rc = finish_call(sc, st, tot, res.samples, stats)) != FW_OK) return rc;
+        f.launches++;
+        if ((rc = finish_call(f, res.samples, stats)) != FW_OK) return rc;
         if (rgb_out) FW_CUDA(cudaMemcpyAsync(rgb_out, c->d_rgb, npix * 3, cudaMemcpyDeviceToHost, st));
         if (sum_out) FW_CUDA(cudaMemcpyAsync(sum_out, c->d_sum, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
         if (count_out) FW_CUDA(cudaMemcpyAsync(count_out, A.count, npix * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
@@ -1408,11 +1448,6 @@ int fw_render_adaptive(fw_scene* sc, const fw_params* p, const fw_adaptive* ad, 
 }
 
 // ---- denoised renders (DESIGN.md §12) --------------------------------------------------------------------
-static int check_image(const fw_params* p) {
-    if (p->width == 0 || p->height == 0 || p->samples == 0) return set_error(FW_ERR_ARG, "width, height and samples must be non-zero");
-    if ((uint64_t)p->width * p->height > 0x7fffffffull) return set_error(FW_ERR_ARG, "image too large");
-    return FW_OK;
-}
 static int copy_aov_out(RenderCtx* c, size_t npix, const fw_aov* aov, cudaStream_t st) {
     if (!aov) return FW_OK;
     if (aov->albedo) FW_CUDA(cudaMemcpyAsync(aov->albedo, c->dn_planar, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
@@ -1432,22 +1467,14 @@ int fw_render_aov(fw_scene* sc, const fw_params* p, const fw_aov* aov, fw_stats*
         if (!sc->committed || !sc->ctx) return set_error(FW_ERR_STATE, "fw_scene_commit must be called before rendering");
         FW_CUDA(cudaSetDevice(sc->device));
         const size_t npix = (size_t)p->width * p->height;
-        if ((rc = ensure_denoise_buffers(sc, npix)) != FW_OK) return rc;
-        RenderParamsHost hp;
-        memcpy(&hp, p, sizeof(hp));
-        const CameraRec cam = make_camera(hp);
-        const uint2 seed = make_uint2((uint32_t)p->seed, (uint32_t)(p->seed >> 32));
-        size_t cap = 0;
-        if ((rc = prepare_batches(sc, npix * p->sample_count, &cap)) != FW_OK) return rc;
         RenderCtx* c = sc->ctx;
-        cudaStream_t st = c->stream;
-        RunTotals tot;
-        FW_CUDA(cudaMemsetAsync(c->d_rays, 0, sizeof(unsigned long long), st));
-        FW_CUDA(cudaEventRecord(c->ev_begin, st));
-        if ((rc = aov_pass(sc, p, cam, seed, cap, p->sample_begin, p->sample_count, c->dn_planar, st, tot)) != FW_OK) return rc;
-        if ((rc = finish_call(sc, st, tot, (uint64_t)npix * p->sample_count, stats)) != FW_OK) return rc;
-        if ((rc = copy_aov_out(c, npix, aov, st)) != FW_OK) return rc;
-        FW_CUDA(cudaStreamSynchronize(st));
+        CallFrame f(sc, p, c->stream);
+        if ((rc = ensure_denoise_buffers(sc, npix)) != FW_OK || (rc = begin_call(f, npix * p->sample_count)) != FW_OK ||
+            (rc = aov_pass(f, p->sample_begin, p->sample_count, c->dn_planar)) != FW_OK)
+            return rc;
+        if ((rc = finish_call(f, (uint64_t)npix * p->sample_count, stats)) != FW_OK || (rc = copy_aov_out(c, npix, aov, f.st)) != FW_OK)
+            return rc;
+        FW_CUDA(cudaStreamSynchronize(f.st));
         return FW_OK;
 });
 }
@@ -1500,38 +1527,25 @@ int fw_render_denoised(fw_scene* sc, const fw_params* p, const fw_denoise* dn, u
         if (!sc->committed || !sc->ctx) return set_error(FW_ERR_STATE, "fw_scene_commit must be called before rendering");
         FW_CUDA(cudaSetDevice(sc->device));
         const size_t npix = (size_t)p->width * p->height;
-        if ((rc = ensure_sum_buffers(sc, npix)) != FW_OK || (rc = ensure_adaptive_buffers(sc, npix)) != FW_OK ||
-            (rc = ensure_denoise_buffers(sc, npix)) != FW_OK)
-            return rc;
-        RenderParamsHost hp;
-        memcpy(&hp, p, sizeof(hp));
-        const CameraRec cam = make_camera(hp);
-        const uint2 seed = make_uint2((uint32_t)p->seed, (uint32_t)(p->seed >> 32));
-        size_t cap = 0;
-        if ((rc = prepare_batches(sc, npix * p->samples, &cap)) != FW_OK) return rc;
         RenderCtx* c = sc->ctx;
-        const AdaptiveState& A = c->adapt;
-        cudaStream_t st = c->stream;
+        CallFrame f(sc, p, c->stream);
+        const cudaStream_t st = f.st;
+        if ((rc = ensure_sum_buffers(sc, npix)) != FW_OK || (rc = ensure_adaptive_buffers(sc, npix)) != FW_OK ||
+            (rc = ensure_denoise_buffers(sc, npix)) != FW_OK || (rc = zero_moments(c, npix, st)) != FW_OK ||
+            (rc = begin_call(f, npix * p->samples)) != FW_OK)
+            return rc;
+        if ((rc = run_tiles(f, npix, nullptr, 0, p->samples, c->d_sum, &c->adapt)) != FW_OK ||
+            (rc = aov_pass(f, 0, std::min(dn->aov_samples, p->samples), c->dn_planar)) != FW_OK)
+            return rc;
         const unsigned grid = grid_for(npix, 256, sc->sm_count * 8);
-        FW_CUDA(cudaMemsetAsync(c->d_sum, 0, npix * 3 * sizeof(float), st));
-        FW_CUDA(cudaMemsetAsync(A.m1, 0, npix * sizeof(double), st));
-        FW_CUDA(cudaMemsetAsync(A.m2, 0, npix * sizeof(double), st));
-        FW_CUDA(cudaMemsetAsync(A.count, 0, npix * sizeof(uint32_t), st));
-        RunTotals tot;
-        size_t ev_next = 0;
-        FW_CUDA(cudaMemsetAsync(c->d_rays, 0, sizeof(unsigned long long), st));
-        FW_CUDA(cudaEventRecord(c->ev_begin, st));
-        if ((rc = run_tiles(sc, p, cam, seed, cap, npix, nullptr, 0, p->samples, c->d_sum, &A, st, tot, ev_next)) != FW_OK) return rc;
-        const uint32_t aov_n = std::min(dn->aov_samples, p->samples);
-        if ((rc = aov_pass(sc, p, cam, seed, cap, 0, aov_n, c->dn_planar, st, tot)) != FW_OK) return rc;
-        launch_denoise_input(c->d_sum, A, (uint32_t)npix, p->samples, c->dn_cv[0], c->dn_var, grid, st);
-        tot.launches++;
-        const int cur = denoise_iterations(dn, p->width, p->height, c->dn_cv, c->aov, st, &tot.launches);
+        launch_denoise_input(c->d_sum, c->adapt, (uint32_t)npix, p->samples, c->dn_cv[0], c->dn_var, grid, st);
+        f.launches++;
+        const int cur = denoise_iterations(dn, p->width, p->height, c->dn_cv, c->aov, st, &f.launches);
         launch_denoise_unpack(c->dn_cv[cur], (uint32_t)npix, c->dn_color, nullptr, grid, st);
         launch_resolve(c->dn_color, (uint32_t)npix, 1.0f, p->gamma, c->d_rgb, grid, st);
-        tot.launches += 2;
+        f.launches += 2;
         FW_CUDA(cudaGetLastError());
-        if ((rc = finish_call(sc, st, tot, (uint64_t)npix * p->samples, stats)) != FW_OK) return rc;
+        if ((rc = finish_call(f, (uint64_t)npix * p->samples, stats)) != FW_OK) return rc;
         if (rgb_out) FW_CUDA(cudaMemcpyAsync(rgb_out, c->d_rgb, npix * 3, cudaMemcpyDeviceToHost, st));
         if (sum_out) FW_CUDA(cudaMemcpyAsync(sum_out, c->d_sum, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
         if (denoised_out) FW_CUDA(cudaMemcpyAsync(denoised_out, c->dn_color, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
@@ -1550,13 +1564,11 @@ int fw_primary_rays(fw_scene* sc, const fw_params* p, uint32_t sample, uint32_t 
     if (!sc || !p || !origins || !dirs) return set_error(FW_ERR_ARG, "null argument");
     if (!sc->committed) return set_error(FW_ERR_STATE, "scene not committed");
     FW_CUDA(cudaSetDevice(sc->device));
-    RenderParamsHost hp;
-    memcpy(&hp, p, sizeof(hp));
-    CameraRec cam = make_camera(hp);
+    const CallFrame f(sc, p, sc->ctx->stream);   // the rays of a render call of `p`
     DevBuf o, d;
     TRY(o.alloc((size_t)n * 12)); TRY(d.alloc((size_t)n * 12));
-    launch_primary_rays_probe(cam, p->width, p->height, sample, make_uint2((uint32_t)p->seed, (uint32_t)(p->seed >> 32)), pix_begin, n,
-                              o.as<float>(), d.as<float>(), grid_for(n, 256, 4096), sc->ctx->stream);
+    launch_primary_rays_probe(f.cam, p->width, p->height, sample, f.seed, pix_begin, n, o.as<float>(), d.as<float>(), grid_for(n, 256, 4096),
+                              f.st);
     FW_CUDA(cudaGetLastError());
     FW_CUDA(cudaStreamSynchronize(sc->ctx->stream));
     TRY(o.get(origins, (size_t)n * 12)); TRY(d.get(dirs, (size_t)n * 12));
@@ -1570,26 +1582,23 @@ int fw_first_hit(fw_scene* sc, int use_bvh, uint64_t seed, uint32_t n, const flo
         return set_error(FW_ERR_ARG, "null argument");
     if (!sc->committed) return set_error(FW_ERR_STATE, "scene not committed");
     FW_CUDA(cudaSetDevice(sc->device));
-    DevBuf dO, dD, dP, dS, dB, oObj, oPrim, oMat, oT, oPt, oN, oUv, oC;
+    DevBuf dO, dD, dP, dS, dB, oC;
+    FirstHitBufs hit;
     TRY(dO.put(origins, (size_t)n * 12)); TRY(dD.put(dirs, (size_t)n * 12));
     if (pixel) TRY(dP.put(pixel, (size_t)n * 4));
     if (sample) TRY(dS.put(sample, (size_t)n * 4));
     if (bounce) TRY(dB.put(bounce, (size_t)n * 4));
-    TRY(oObj.alloc((size_t)n * 4)); TRY(oPrim.alloc((size_t)n * 4)); TRY(oMat.alloc((size_t)n * 4)); TRY(oT.alloc((size_t)n * 4));
-    TRY(oPt.alloc((size_t)n * 12)); TRY(oN.alloc((size_t)n * 12)); TRY(oUv.alloc((size_t)n * 8)); TRY(oC.alloc(16));
+    TRY(hit.alloc(n)); TRY(oC.alloc(16));
     FW_CUDA(cudaMemset(oC.p, 0, 16));
-    FirstHitOut out{oObj.as<int>(), oPrim.as<int>(), oMat.as<int>(), oT.as<float>(), oPt.as<float>(), oN.as<float>(),
-                    oUv.as<float>(), oC.as<unsigned long long>()};
     uint2 sd = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
     unsigned g = grid_for(n, 128, 8192);
     int mode = use_bvh ? 1 : (sc->lin_prog_ok ? (sc->flat.lin_generic ? 2 : 3) : 0);
     launch_first_hit_probe(mode, sc->lin_prog, sc->dscene, sd, n, dO.as<float>(), dD.as<float>(), pixel ? dP.as<uint32_t>() : nullptr,
-                           sample ? dS.as<uint32_t>() : nullptr, bounce ? dB.as<uint32_t>() : nullptr, out, g, sc->ctx->stream);
+                           sample ? dS.as<uint32_t>() : nullptr, bounce ? dB.as<uint32_t>() : nullptr, hit.out(oC.as<unsigned long long>()), g,
+                           sc->ctx->stream);
     FW_CUDA(cudaGetLastError());
     FW_CUDA(cudaStreamSynchronize(sc->ctx->stream));
-    TRY(oObj.get(obj, (size_t)n * 4)); TRY(oPrim.get(prim, (size_t)n * 4)); TRY(oMat.get(material, (size_t)n * 4));
-    TRY(oT.get(t, (size_t)n * 4)); TRY(oPt.get(point, (size_t)n * 12)); TRY(oN.get(normal, (size_t)n * 12));
-    TRY(oUv.get(uv, (size_t)n * 8));
+    TRY(hit.get(n, obj, prim, material, t, point, normal, uv));
     if (counters) TRY(oC.get(counters, 16));
     return FW_OK;
 }
@@ -1605,28 +1614,22 @@ int fw_first_hit_wavefront(fw_scene* sc, int use_bvh, uint64_t seed, uint32_t n,
     FW_CUDA(cudaSetDevice(sc->device));
     int rc = ensure_path_state(sc, std::max<size_t>(n, 32));
     if (rc != FW_OK) return rc;
-    DevBuf dO, dD, oObj, oPrim, oMat, oT, oPt, oN, oUv;
+    DevBuf dO, dD;
+    FirstHitBufs hit;
     TRY(dO.put(origins, (size_t)n * 12)); TRY(dD.put(dirs, (size_t)n * 12));
-    TRY(oObj.alloc((size_t)n * 4)); TRY(oPrim.alloc((size_t)n * 4)); TRY(oMat.alloc((size_t)n * 4)); TRY(oT.alloc((size_t)n * 4));
-    TRY(oPt.alloc((size_t)n * 12)); TRY(oN.alloc((size_t)n * 12)); TRY(oUv.alloc((size_t)n * 8));
-    FirstHitOut out{oObj.as<int>(), oPrim.as<int>(), oMat.as<int>(), oT.as<float>(), oPt.as<float>(), oN.as<float>(), oUv.as<float>(), nullptr};
+    TRY(hit.alloc(n));
     cudaStream_t st = sc->ctx->stream;
-    PathState& ps = sc->ctx->ps;
-    segment_geometry(sc, n, &ps.nseg, &ps.seg_cap);
-    FW_CUDA(cudaMemsetAsync(ps.counters, 0, sizeof(uint32_t) * (FW_MAX_DEPTH + 2) * FW_NUM_QUEUES * (size_t)ps.nseg, st));
-    FW_CUDA(cudaMemsetAsync(ps.poison, 0, sizeof(uint32_t), st));
+    const PathState& ps = sc->ctx->ps;
+    TRY(begin_batch(sc, n, st));
     const Batch b = make_batch(0, n, sample, 1, n, 1, nullptr);   // ray i = path i = "pixel" i of a one-sample batch: RNG key (pixel i, sample, bounce)
     const uint2 sd = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
     launch_probe_fill(ps, n, dO.as<float>(), dD.as<float>(), bounce, st);
     uint64_t launches = 0;
     TRY(extend_bounce(sc, use_bvh != 0, b, sd, bounce, st, launches));
-    launch_probe_collect(sc->dscene, ps, bounce, out, st);
+    launch_probe_collect(sc->dscene, ps, bounce, hit.out(nullptr), st);
     FW_CUDA(cudaGetLastError());
     FW_CUDA(cudaStreamSynchronize(st));
-    TRY(oObj.get(obj, (size_t)n * 4)); TRY(oPrim.get(prim, (size_t)n * 4)); TRY(oMat.get(material, (size_t)n * 4));
-    TRY(oT.get(t, (size_t)n * 4)); TRY(oPt.get(point, (size_t)n * 12)); TRY(oN.get(normal, (size_t)n * 12));
-    TRY(oUv.get(uv, (size_t)n * 8));
-    return FW_OK;
+    return hit.get(n, obj, prim, material, t, point, normal, uv);
 }
 
 int fw_scatter_step(fw_scene* sc, uint32_t n, const int32_t* material, const float* ray_o, const float* ray_d,

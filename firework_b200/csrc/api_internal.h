@@ -126,7 +126,5 @@ int render_into(fw_scene* sc, const fw_params* p, float* d_sum, cudaStream_t st,
 int ensure_sum_buffers(fw_scene* sc, size_t npix);   // ctx->d_sum / d_rgb sized for npix pixels
 int ensure_adaptive_buffers(fw_scene* sc, size_t npix);   // ctx->adapt sized for npix pixels
 int ensure_denoise_buffers(fw_scene* sc, size_t npix);    // ctx->aov / dn_* sized for npix pixels
-int commit_scene(fw_scene* sc, int device);          // fw_scene_commit
-void destroy_scene(fw_scene* sc);                    // fw_scene_destroy
 unsigned grid_for(size_t n, unsigned threads, unsigned max_blocks);
 }  // namespace fw

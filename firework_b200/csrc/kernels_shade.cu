@@ -1,4 +1,4 @@
-// Ray generation, shading, miss, accumulation and resolve kernels.
+// Ray generation, shading, miss, accumulation and resolve kernels (and fw_render_multi's fused peer reduce + resolve).
 #include "launch.h"
 #include "wavefront.cuh"
 
@@ -205,6 +205,18 @@ __global__ void __launch_bounds__(256) resolve_kernel(const float* __restrict__ 
     }
 }
 
+// resolve_kernel over the sum of src.n per-device buffers, read in place through peer mappings (rank order).
+__global__ void __launch_bounds__(256) peer_reduce_resolve_kernel(PeerSums src, float* __restrict__ total, uint32_t n_values,
+                                                                   float samples, float gamma, unsigned char* __restrict__ rgb) {
+    const float inv_gamma = 1.0f / gamma;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_values; i += gridDim.x * blockDim.x) {
+        float s = src.p[0][i];
+        for (int k = 1; k < src.n; ++k) s += __ldcs(&src.p[k][i]);   // peer memory: read once, streaming
+        total[i] = s;
+        if (rgb) rgb[i] = quantise(s / samples, inv_gamma);
+    }
+}
+
 // ---- launchers -------------------------------------------------------------------------------------------
 void launch_raygen(const CameraRec& cam, const Batch& b, uint2 seed, const PathState& ps, cudaStream_t st) {
     if (b.pixels) raygen_kernel<true><<<ps.nseg, FW_BLOCK, 0, st>>>(cam, b, seed, ps);   // a pixel list (adaptive rounds)
@@ -243,6 +255,10 @@ void launch_tally(const PathState& ps, unsigned long long* d_rays, cudaStream_t 
 void launch_resolve(const float* d_sum, uint32_t npix, float samples, float gamma, unsigned char* d_rgb, unsigned blocks,
                     cudaStream_t st) {
     resolve_kernel<<<blocks, 256, 0, st>>>(d_sum, npix, samples, gamma, d_rgb);
+}
+void launch_peer_reduce_resolve(const PeerSums& src, float* total, uint32_t n_values, float samples, float gamma, unsigned char* rgb,
+                                unsigned blocks, cudaStream_t st) {
+    peer_reduce_resolve_kernel<<<blocks, 256, 0, st>>>(src, total, n_values, samples, gamma, rgb);
 }
 
 }  // namespace fw

@@ -48,6 +48,15 @@ void launch_accumulate(float* d_sum, const PathState& ps, const Batch& b, unsign
 void launch_tally(const PathState& ps, unsigned long long* d_rays, cudaStream_t st);
 void launch_resolve(const float* d_sum, uint32_t npix, float samples, float gamma, unsigned char* d_rgb, unsigned blocks,
                     cudaStream_t st);
+// fw_render_multi's peer reduce: the per-device sum buffers of up to kMaxPeers devices, read in place through peer mappings.
+constexpr int kMaxPeers = 16;
+struct PeerSums {
+    const float* p[kMaxPeers];
+    int n;
+};
+// total = the sum of the n_values floats of src.p[0 .. n) in rank order; rgb (nullable) = its resolve, as launch_resolve does.
+void launch_peer_reduce_resolve(const PeerSums& src, float* total, uint32_t n_values, float samples, float gamma, unsigned char* rgb,
+                                unsigned blocks, cudaStream_t st);
 
 // Per-pixel state of an adaptive or denoised render (kernels_adaptive.cu), in the render context next to d_sum.
 struct AdaptiveState {

@@ -103,42 +103,14 @@ int replica_on(fw_scene* sc, int device, fw_scene** out) {
     r->built = sc->built;
     r->asset_src = sc;
     r->batch_paths = sc->batch_paths;
-    int rc = commit_scene(r, device);
-    if (rc != FW_OK) { destroy_scene(r); return rc; }
+    int rc = fw_scene_commit(r, device);
+    if (rc != FW_OK) { fw_scene_destroy(r); return rc; }
     sc->replicas.push_back(r);
     *out = r;
     return FW_OK;
 }
 
-constexpr int kMaxPeers = 16;
-struct PeerSums {
-    const float* p[kMaxPeers];
-    int n;
-};
-
 }  // namespace
-
-namespace fw {
-// render.rs:184-189 over the sum of n per-device buffers, read in place through peer mappings (rank order).
-__device__ __forceinline__ unsigned char quantise_u8(float mean, float inv_gamma) {
-    float x = powf(mean, inv_gamma);
-    if (x < 0.0f) x = 0.0f;
-    if (x > 1.0f) x = 1.0f;
-    float y = x * 255.99f;
-    if (!(y == y)) return 0;
-    return (unsigned char)fminf(fmaxf(truncf(y), 0.0f), 255.0f);
-}
-__global__ void __launch_bounds__(256) peer_reduce_resolve_kernel(PeerSums src, float* __restrict__ total, uint32_t n_values,
-                                                                   float samples, float gamma, unsigned char* __restrict__ rgb) {
-    const float inv_gamma = 1.0f / gamma;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_values; i += gridDim.x * blockDim.x) {
-        float s = src.p[0][i];
-        for (int k = 1; k < src.n; ++k) s += __ldcs(&src.p[k][i]);   // peer memory: read once, streaming
-        total[i] = s;
-        if (rgb) rgb[i] = quantise_u8(s / samples, inv_gamma);
-    }
-}
-}  // namespace fw
 
 extern "C" int fw_render_multi(fw_scene* sc, const fw_params* p, int n_gpus, const int* devices, int reduce_mode,
                                uint8_t* rgb_out, float* sum_out, fw_stats* stats, double* ms_reduce) {
@@ -226,8 +198,8 @@ extern "C" int fw_render_multi(fw_scene* sc, const fw_params* p, int n_gpus, con
             if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
             else if (e != cudaSuccess) return set_error(FW_ERR_CUDA, std::string("cudaDeviceEnablePeerAccess: ") + cudaGetErrorString(e));
         }
-        peer_reduce_resolve_kernel<<<grid_for(n_values, 256, sc->sm_count * 8), 256, 0, c0->stream>>>(
-            src, c0->d_sum, n_values, (float)p->samples, p->gamma, rgb_out ? c0->d_rgb : nullptr);
+        launch_peer_reduce_resolve(src, c0->d_sum, n_values, (float)p->samples, p->gamma, rgb_out ? c0->d_rgb : nullptr,
+                                   grid_for(n_values, 256, sc->sm_count * 8), c0->stream);
         FW_CUDA(cudaGetLastError());
         resolved = true;
     } else if (n_gpus > 1) {
