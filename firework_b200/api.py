@@ -731,3 +731,26 @@ class Renderer:
             rgb, _sum, stats = render_scene(scene, self)
         self.last_stats = stats
         return rgb
+
+    def trace_rays(self, scene: Scene, origins, directions, keys=None) -> np.ndarray:
+        """Extra (not in the reference): path-trace caller-supplied rays instead of the camera's (fw_trace_rays, DESIGN.md §13), with
+        this renderer's `samples`, `seed` and `use_bvh`.  `origins` / `directions` of shape (N, 3) are re-traced for every sample;
+        of shape (samples, N, 3) they give one ray per sample.  Ray i is keyed as pixel keys[i] (uint32, default i): the same
+        (key, sample) draws the same random numbers in every call.  Returns the per-ray mean radiance sum / samples, (N, 3) float32;
+        last_stats carries `sum`.  Single GPU and not together with adaptive() or denoise(): those raise ValueError."""
+        from .engine import NativeScene
+        if self._gpus > 1:
+            raise ValueError("tracing rays runs on one GPU: gpus(n > 1) and trace_rays can not be combined")
+        if self._adaptive is not None:
+            raise ValueError("adaptive() and trace_rays can not be combined")
+        if self._denoise is not None:
+            raise ValueError("denoise() and trace_rays can not be combined")
+        ns = NativeScene.from_scene(scene, 0)
+        try:
+            s, stats = ns.trace_rays(np.asarray(origins, F), np.asarray(directions, F), sample_count=self._samples, seed=self._seed,
+                                     use_bvh=self._use_bvh, keys=None if keys is None else np.asarray(keys, np.uint32))
+        finally:
+            ns.close()
+        stats["sum"] = s
+        self.last_stats = stats
+        return s / F(self._samples)

@@ -956,10 +956,12 @@ static int ensure_path_state(fw_scene* sc, size_t cap) {
 }
 
 // One render call of `p` on `sc`: what its batches share, and the totals that finish_call turns into fw_stats.  The camera and
-// seed are built here alone, for every render entry point and fw_primary_rays.
+// seed are built here alone, for every render entry point and fw_primary_rays.  A trace call (fw_trace_rays) sets `rays`
+// instead: its params only carry the ray count as the width (height 1), the seed and use_bvh, and it has no camera.
 struct CallFrame {
     fw_scene* sc;
     const fw_params* p;
+    const RaySource* rays;
     CameraRec cam;
     uint2 seed;
     cudaStream_t st;
@@ -967,10 +969,13 @@ struct CallFrame {
     uint64_t launches = 0, extend_launches = 0;
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> extend_events;   // fw_set_profiling: one pair per extend of run_batch
     size_t ev_next = 0;    // next free event of the context's pool
-    CallFrame(fw_scene* s, const fw_params* q, cudaStream_t stream) : sc(s), p(q), st(stream) {
-        RenderParamsHost hp;
-        memcpy(&hp, q, sizeof(hp));
-        cam = make_camera(hp);
+    CallFrame(fw_scene* s, const fw_params* q, cudaStream_t stream, const RaySource* r = nullptr) : sc(s), p(q), rays(r), st(stream) {
+        memset(&cam, 0, sizeof(cam));
+        if (!rays) {
+            RenderParamsHost hp;
+            memcpy(&hp, q, sizeof(hp));
+            cam = make_camera(hp);
+        }
         seed = make_uint2((uint32_t)q->seed, (uint32_t)(q->seed >> 32));
     }
 };
@@ -1031,8 +1036,8 @@ static int begin_batch(fw_scene* sc, size_t paths, cudaStream_t st) {
     return FW_OK;
 }
 
-// One batch: raygen, up to FW_MAX_DEPTH+1 extend/shade rounds, accumulate into d_sum (and, for an adaptive or denoised render,
-// into the moments and counts of `adapt`).
+// One batch: raygen (from the camera, or from the call's rays), up to FW_MAX_DEPTH+1 extend/shade rounds, accumulate into d_sum
+// (and, for an adaptive or denoised render, into the moments and counts of `adapt`).
 static int run_batch(CallFrame& f, const Batch& b, float* d_sum, const AdaptiveState* adapt) {
     fw_scene* sc = f.sc;
     const cudaStream_t st = f.st;
@@ -1041,7 +1046,8 @@ static int run_batch(CallFrame& f, const Batch& b, float* d_sum, const AdaptiveS
     int rc = begin_batch(sc, (size_t)b.npix * b.ns, st);
     if (rc != FW_OK) return rc;
     unsigned sm = (unsigned)sc->sm_count;
-    launch_raygen(f.cam, b, f.seed, ps, st);
+    if (f.rays) launch_raygen_rays(*f.rays, b, ps, st);
+    else launch_raygen(f.cam, b, f.seed, ps, st);
     f.launches++;
     FW_STAGE("raygen", 0);
     for (uint32_t bounce = 0; bounce <= (uint32_t)FW_MAX_DEPTH; ++bounce) {
@@ -1553,6 +1559,73 @@ int fw_render_denoised(fw_scene* sc, const fw_params* p, const fw_denoise* dn, u
         if ((rc = copy_aov_out(c, npix, aov, st)) != FW_OK) return rc;
         FW_CUDA(cudaStreamSynchronize(st));
         return FW_OK;
+});
+}
+
+// ---- caller-supplied rays (DESIGN.md §13) ----------------------------------------------------------------
+// The argument checks of both trace entry points; none of them makes a CUDA call.
+static int check_trace(const fw_scene* sc, uint64_t n, const float* origins, const float* dirs, uint32_t sample_begin,
+                       uint32_t sample_count, const float* sum) {
+    if (!sc || !origins || !dirs || !sum) return set_error(FW_ERR_ARG, "null argument");
+    if (n == 0 || n > 0x7fffffffull) return set_error(FW_ERR_ARG, "the number of rays must be in 1 .. 2^31 - 1");
+    if (sample_count == 0) return set_error(FW_ERR_ARG, "sample_count must be >= 1");
+    if ((uint64_t)sample_begin + sample_count > 0x100000000ull) return set_error(FW_ERR_ARG, "sample_begin + sample_count must be <= 2^32");
+    if (!sc->committed || !sc->ctx) return set_error(FW_ERR_STATE, "fw_scene_commit must be called before tracing");
+    return FW_OK;
+}
+
+// Adds samples [rs.sample_begin, rs.sample_begin + sample_count) of every ray of `rs`, ray i keyed as pixel d_keys[i] (or i when
+// d_keys is null), into d_sum[3i .. 3i+2] on `st`: the render's batch loop with the rays as a one-row image of rs.n pixels.
+static int trace_into(fw_scene* sc, const RaySource& rs, const uint32_t* d_keys, uint32_t sample_count, uint64_t seed, int use_bvh,
+                      float* d_sum, cudaStream_t st, fw_stats* stats) {
+    fw_params p;
+    memset(&p, 0, sizeof(p));
+    p.width = rs.n; p.height = 1;
+    p.samples = p.sample_count = sample_count; p.sample_begin = rs.sample_begin;
+    p.use_bvh = use_bvh != 0;
+    p.seed = seed;
+    CallFrame f(sc, &p, st, &rs);
+    int rc;
+    if ((rc = begin_call(f, (size_t)rs.n * sample_count)) != FW_OK ||
+        (rc = run_tiles(f, rs.n, d_keys, rs.sample_begin, sample_count, d_sum, nullptr)) != FW_OK)
+        return rc;
+    return finish_call(f, (uint64_t)rs.n * sample_count, stats);
+}
+
+int fw_trace_rays(fw_scene* sc, uint64_t n, const float* origins, const float* dirs, const uint32_t* keys, int per_sample,
+                  uint32_t sample_begin, uint32_t sample_count, uint64_t seed, int use_bvh, float* sum_out, fw_stats* stats) {
+    return guarded([&]() -> int {
+        int rc = check_trace(sc, n, origins, dirs, sample_begin, sample_count, sum_out);
+        if (rc != FW_OK) return rc;
+        FW_CUDA(cudaSetDevice(sc->device));
+        RenderCtx* c = sc->ctx;
+        const cudaStream_t st = c->stream;
+        const size_t ray_bytes = (size_t)n * (per_sample ? sample_count : 1) * 12;
+        DevBuf dO, dD, dK;
+        if ((rc = dO.alloc(ray_bytes)) != FW_OK || (rc = dD.alloc(ray_bytes)) != FW_OK || (keys && (rc = dK.alloc(n * 4)) != FW_OK) ||
+            (rc = ensure_sum_buffers(sc, n)) != FW_OK)
+            return rc;
+        FW_CUDA(cudaMemcpyAsync(dO.p, origins, ray_bytes, cudaMemcpyHostToDevice, st));
+        FW_CUDA(cudaMemcpyAsync(dD.p, dirs, ray_bytes, cudaMemcpyHostToDevice, st));
+        if (keys) FW_CUDA(cudaMemcpyAsync(dK.p, keys, n * 4, cudaMemcpyHostToDevice, st));
+        FW_CUDA(cudaMemsetAsync(c->d_sum, 0, n * 3 * sizeof(float), st));
+        const RaySource rs{dO.as<float>(), dD.as<float>(), (uint32_t)n, sample_begin, per_sample != 0};
+        if ((rc = trace_into(sc, rs, keys ? dK.as<uint32_t>() : nullptr, sample_count, seed, use_bvh, c->d_sum, st, stats)) != FW_OK) return rc;
+        FW_CUDA(cudaMemcpyAsync(sum_out, c->d_sum, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
+        FW_CUDA(cudaStreamSynchronize(st));
+        return FW_OK;
+});
+}
+
+int fw_trace_rays_device(fw_scene* sc, uint64_t n, const float* d_origins, const float* d_dirs, const uint32_t* d_keys, int per_sample,
+                         uint32_t sample_begin, uint32_t sample_count, uint64_t seed, int use_bvh, float* d_sum, void* cuda_stream,
+                         fw_stats* stats) {
+    return guarded([&]() -> int {
+        int rc = check_trace(sc, n, d_origins, d_dirs, sample_begin, sample_count, d_sum);
+        if (rc != FW_OK) return rc;
+        FW_CUDA(cudaSetDevice(sc->device));
+        const RaySource rs{d_origins, d_dirs, (uint32_t)n, sample_begin, per_sample != 0};
+        return trace_into(sc, rs, d_keys, sample_count, seed, use_bvh, d_sum, cuda_stream ? (cudaStream_t)cuda_stream : sc->ctx->stream, stats);
 });
 }
 

@@ -36,6 +36,38 @@ __global__ void __launch_bounds__(FW_BLOCK) raygen_kernel(CameraRec cam, Batch b
     if (threadIdx.x == 0) counter_row(ps, 0, FW_Q_EXTEND)[seg] = s_count;
 }
 
+// raygen_kernel for caller-supplied rays (fw_trace_rays): the same segment and tile mapping, so every later kernel sees the
+// queue layout of a render.  Path p is list position pix0 + p % npix at sample s0 + p / npix; the ray is read from that list
+// position, not from the key b.pixels maps it to, and no random number is drawn.  The key only matters to the later kernels,
+// which read it through their LIST instances.
+template <bool PER_SAMPLE>
+__global__ void __launch_bounds__(FW_BLOCK) raygen_rays_kernel(RaySource rs, Batch b, PathState ps) {
+    const uint32_t total = b.npix * b.ns;
+    const uint32_t seg = blockIdx.x;
+    const size_t base = (size_t)seg * ps.seg_cap;
+    uint32_t count = 0;
+    for (uint32_t e = threadIdx.x; e < ps.seg_cap; e += FW_BLOCK) {
+        uint32_t p = ((e / FW_TILE) * ps.nseg + seg) * FW_TILE + (e % FW_TILE);
+        if (p >= total) break;   // p grows with e: the valid entries are a prefix
+        uint32_t q, r;
+        div_magic(p, b.npix, b.npix_magic, q, r);
+        size_t i = (size_t)b.pix0 + r;
+        if (PER_SAMPLE) i += (size_t)(b.s0 + q - rs.sample_begin) * rs.n;   // sample_count x n can pass 2^32
+        const float* o = rs.origins + 3 * i;
+        const float* d = rs.dirs + 3 * i;
+        st_stream(&ps.xo[0][base + e], make_float4(__ldcs(o), __ldcs(o + 1), __ldcs(o + 2), __uint_as_float(p)));
+        st_stream(&ps.xd[0][base + e], make_float4(__ldcs(d), __ldcs(d + 1), __ldcs(d + 2), 0.0f));
+        st_stream(&ps.radiance[p], make_float4(0.0f, 0.0f, 0.0f, 0.0f));
+        count = e + 1;
+    }
+    __shared__ uint32_t s_count;
+    if (threadIdx.x == 0) s_count = 0;
+    __syncthreads();
+    if (count) atomicMax(&s_count, count);
+    __syncthreads();
+    if (threadIdx.x == 0) counter_row(ps, 0, FW_Q_EXTEND)[seg] = s_count;
+}
+
 // render.rs:23 evaluated without recursion: colour = a0 * (a1 * (... (a_{k-1} * terminal))) with the same
 // right-nested association as `emit + attenuation * color(...)`; emit is zero at every scattering vertex
 // (material.rs:13-15), so the chain of attenuations is all that is needed.
@@ -221,6 +253,10 @@ __global__ void __launch_bounds__(256) peer_reduce_resolve_kernel(PeerSums src, 
 void launch_raygen(const CameraRec& cam, const Batch& b, uint2 seed, const PathState& ps, cudaStream_t st) {
     if (b.pixels) raygen_kernel<true><<<ps.nseg, FW_BLOCK, 0, st>>>(cam, b, seed, ps);   // a pixel list (adaptive rounds)
     else raygen_kernel<false><<<ps.nseg, FW_BLOCK, 0, st>>>(cam, b, seed, ps);
+}
+void launch_raygen_rays(const RaySource& rs, const Batch& b, const PathState& ps, cudaStream_t st) {
+    if (rs.per_sample) raygen_rays_kernel<true><<<ps.nseg, FW_BLOCK, 0, st>>>(rs, b, ps);
+    else raygen_rays_kernel<false><<<ps.nseg, FW_BLOCK, 0, st>>>(rs, b, ps);
 }
 void launch_miss(const DeviceScene& S, const PathState& ps, uint32_t bounce, bool black_env, cudaStream_t st) {
     if (black_env) miss_kernel<true><<<ps.nseg, FW_BLOCK, 0, st>>>(S, ps, bounce);

@@ -31,6 +31,8 @@ struct WalkAuxHost {
 };
 
 void launch_raygen(const CameraRec& cam, const Batch& b, uint2 seed, const PathState& ps, cudaStream_t st);
+// raygen from the caller's rays (fw_trace_rays): entry e of the bounce-0 queue gets the ray of its path, as launch_raygen lays it out.
+void launch_raygen_rays(const RaySource& rs, const Batch& b, const PathState& ps, cudaStream_t st);
 // The lock-step and linear-scan extend kernels.  Returns the number of kernels launched (2 for the two-pass mesh extend).
 int launch_extend(const ExtendPlan& plan, bool use_bvh, const LinProgram& prog, const DeviceScene& S, const PathState& ps,
                   const Batch& b, uint2 seed, uint32_t bounce, cudaStream_t st);

@@ -44,6 +44,15 @@ struct Batch {
     uint32_t width_magic;  // the same for `width` (pixel -> column / row in raygen)
     const uint32_t* pixels;   // null: pixel = pix0 + p % npix.  Else a pixel list (adaptive rounds): pixel = pixels[pix0 + p % npix]
 };
+// Caller-supplied rays of a trace call (fw_trace_rays, DESIGN.md §13), device pointers to fp32 x3 per ray.  The ray of list
+// position i and sample s is entry i (shared layout) or entry (s - sample_begin) * n + i (per-sample layout).
+struct RaySource {
+    const float* origins;
+    const float* dirs;
+    uint32_t n;
+    uint32_t sample_begin;
+    bool per_sample;
+};
 
 struct FirstHitOut {
     int *obj, *prim, *material;

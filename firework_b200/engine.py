@@ -39,6 +39,22 @@ def _aov_arrays(h, w):
     return aov, N.FwAov(*(N.ptr(aov[k]) for k in ("albedo", "normal", "depth", "object")))
 
 
+def _ray_layout(origins, dirs, sample_count, keys):
+    """(number of rays, per-sample layout?) of trace_rays' inputs: (N, 3) shared, (sample_count, N, 3) per sample."""
+    shape = tuple(origins.shape)
+    if tuple(dirs.shape) != shape:
+        raise ValueError(f"origins {shape} and dirs {tuple(dirs.shape)} must have the same shape")
+    if len(shape) == 2 and shape[1] == 3:
+        n, per_sample = shape[0], False
+    elif len(shape) == 3 and shape[2] == 3 and shape[0] == sample_count:
+        n, per_sample = shape[1], True
+    else:
+        raise ValueError(f"rays must be (N, 3) or (sample_count={sample_count}, N, 3), got {shape}")
+    if keys is not None and tuple(keys.shape) != (n,):
+        raise ValueError(f"keys must be ({n},), got {tuple(keys.shape)}")
+    return int(n), per_sample
+
+
 class NativeScene:
     """A committed fw_scene on one GPU."""
 
@@ -225,6 +241,47 @@ class NativeScene:
         st = N.FwStats()
         N.check(N.lib().fw_render_accumulate_device(self._h, C.byref(params), C.c_void_p(d_sum_ptr),
                                                     C.c_void_p(stream_ptr) if stream_ptr else None, C.byref(st)))
+        return st.as_dict()
+
+    def trace_rays(self, origins, dirs, sample_count=1, sample_begin=0, seed=0, use_bvh=False, keys=None):
+        """fw_trace_rays (DESIGN.md §13): path-traces samples [sample_begin, sample_begin + sample_count) of caller-supplied rays.
+        `origins` / `dirs` of shape (N, 3) are re-traced for every sample (shared layout); of shape (sample_count, N, 3) they give
+        one ray per sample (per-sample layout).  Ray i is keyed as pixel keys[i] (uint32, default i).  numpy arrays: returns
+        (sum (N, 3) f32, stats dict).  torch CUDA tensors on this scene's device: runs fw_trace_rays_device into a new torch
+        buffer on a stream of its own and returns (sum tensor (N, 3) f32, stats dict)."""
+        n, per_sample = _ray_layout(origins, dirs, sample_count, keys)
+        if type(origins).__module__.startswith("torch"):
+            import torch
+            dev = torch.device("cuda", self.device)
+            o = origins.to(dev, torch.float32).contiguous()
+            d = dirs.to(dev, torch.float32).contiguous()
+            k = None if keys is None else keys.to(dev, torch.int64).to(torch.int32).contiguous()   # uint32 bit patterns
+            out = torch.zeros((n, 3), dtype=torch.float32, device=dev)
+            # torch's default stream has handle 0, which the C ABI reads as the scene's own stream: use an explicit one
+            stream = torch.cuda.Stream(device=dev)
+            stream.wait_stream(torch.cuda.current_stream(dev))
+            st = self.trace_rays_device(o.data_ptr(), d.data_ptr(), n, out.data_ptr(), stream.cuda_stream, per_sample, sample_count,
+                                        sample_begin, seed, use_bvh, 0 if k is None else k.data_ptr())
+            torch.cuda.current_stream(dev).wait_stream(stream)
+            return out, st
+        o = np.ascontiguousarray(origins, np.float32)
+        d = np.ascontiguousarray(dirs, np.float32)
+        k = None if keys is None else np.ascontiguousarray(keys, np.uint32)
+        s = np.empty((n, 3), np.float32)
+        st = N.FwStats()
+        N.check(N.lib().fw_trace_rays(self._h, n, N.ptr(o), N.ptr(d), None if k is None else N.ptr(k), int(per_sample),
+                                      int(sample_begin), int(sample_count), int(seed), 1 if use_bvh else 0, N.ptr(s), C.byref(st)))
+        return s, st.as_dict()
+
+    def trace_rays_device(self, d_origins_ptr: int, d_dirs_ptr: int, n: int, d_sum_ptr: int, stream_ptr: int, per_sample=False,
+                          sample_count=1, sample_begin=0, seed=0, use_bvh=False, d_keys_ptr: int = 0):
+        """fw_trace_rays_device: ADDS the per-ray sums into a device fp32 (n, 3) buffer (e.g. a torch tensor's data_ptr()) on
+        `stream_ptr` (0: the scene's own stream)."""
+        st = N.FwStats()
+        N.check(N.lib().fw_trace_rays_device(self._h, int(n), C.c_void_p(d_origins_ptr), C.c_void_p(d_dirs_ptr),
+                                             C.c_void_p(d_keys_ptr) if d_keys_ptr else None, 1 if per_sample else 0, int(sample_begin),
+                                             int(sample_count), int(seed), 1 if use_bvh else 0, C.c_void_p(d_sum_ptr),
+                                             C.c_void_p(stream_ptr) if stream_ptr else None, C.byref(st)))
         return st.as_dict()
 
     def resolve_device(self, d_sum_ptr: int, npix: int, samples: int, gamma: float, d_rgb_ptr: int, stream_ptr: int = 0):

@@ -519,27 +519,9 @@ public:
     // Renderer::render (render.rs:109): same inputs, same Vec<Color> (row 0 = top)
     std::vector<Color> render(const Scene& scene) const { return render_yaml(scene.to_yaml()); }
     std::vector<Color> render_yaml(const std::string& yaml) const {
-        fw_scene* h = nullptr;
-        detail::check(fw_scene_from_yaml(yaml.data(), yaml.size(), &h), "scene");
-        struct Guard { fw_scene* h; ~Guard() { fw_scene_destroy(h); } } guard{h};
-        for (int i = 0; i < fw_scene_num_assets(h); ++i) {
-            const std::string path = find_asset(fw_scene_asset_path(h, i));
-            uint32_t w = 0, ht = 0;
-            if (fw_scene_asset_kind(h, i) == 0) {
-                uint8_t* px = nullptr;
-                detail::check(fw_image_load(path.c_str(), &w, &ht, &px), "ImageTexture");
-                int rc = fw_scene_set_image(h, i, w, ht, px);
-                fw_image_free(px);
-                detail::check(rc, "ImageTexture");
-            } else {
-                float* px = nullptr;
-                detail::check(fw_hdr_load(path.c_str(), &w, &ht, &px), "HdrEnvironment");
-                int rc = fw_scene_set_hdr(h, i, w, ht, px);
-                fw_hdr_free(px);
-                detail::check(rc, "HdrEnvironment");
-            }
-        }
-        detail::check(fw_scene_commit(h, 0), "commit");
+        SceneHandle guard;
+        open_scene(yaml, guard);
+        fw_scene* h = guard.h;
         const fw_params p = params();
         std::vector<uint8_t> rgb(width_ * height_ * 3);
         if (denoise_on_) {
@@ -561,7 +543,62 @@ public:
         return out;
     }
 
+    // extra (not in the reference): path-trace n caller-supplied rays instead of the camera's (fw_trace_rays, DESIGN.md §13) with
+    // samples_, seed_ and use_bvh_.  origins / directions hold 3n floats (every sample re-traces the same rays) or samples_ * 3n
+    // (sample-major, one ray per sample); ray i is keyed as pixel keys[i] (empty: i).  Returns the per-ray mean radiance
+    // sum / samples, 3n floats.  Single GPU and not with adaptive() or denoise(): those combinations throw.
+    std::vector<float> trace_rays(const Scene& scene, size_t n, const std::vector<float>& origins, const std::vector<float>& directions,
+                                  const std::vector<uint32_t>& keys = {}) const {
+        return trace_rays_yaml(scene.to_yaml(), n, origins, directions, keys);
+    }
+    std::vector<float> trace_rays_yaml(const std::string& yaml, size_t n, const std::vector<float>& origins,
+                                       const std::vector<float>& directions, const std::vector<uint32_t>& keys = {}) const {
+        if (gpus_ > 1) throw Error("tracing rays runs on one GPU: gpus(n > 1) and trace_rays can not be combined");
+        if (threshold_ >= 0.0f) throw Error("adaptive() and trace_rays can not be combined");
+        if (denoise_on_) throw Error("denoise() and trace_rays can not be combined");
+        const bool per_sample = origins.size() != 3 * n;
+        if (origins.size() != (per_sample ? samples_ : 1) * 3 * n || directions.size() != origins.size())
+            throw Error("trace_rays: origins and directions must hold 3 n or samples * 3 n floats each");
+        if (!keys.empty() && keys.size() != n) throw Error("trace_rays: keys must hold n entries");
+        SceneHandle guard;
+        open_scene(yaml, guard);
+        std::vector<float> out(3 * n);
+        detail::check(fw_trace_rays(guard.h, n, origins.data(), directions.data(), keys.empty() ? nullptr : keys.data(), per_sample ? 1 : 0,
+                                    0, (uint32_t)samples_, seed_, use_bvh_ ? 1 : 0, out.data(), nullptr),
+                      "trace_rays");
+        const float s = (float)samples_;
+        for (float& v : out) v = v / s;
+        return out;
+    }
+
 private:
+    struct SceneHandle {
+        fw_scene* h = nullptr;
+        ~SceneHandle() { fw_scene_destroy(h); }
+    };
+    // The document's scene, its assets handed over, committed on device 0, into `g` (destroyed with it, also when this throws).
+    void open_scene(const std::string& yaml, SceneHandle& g) const {
+        detail::check(fw_scene_from_yaml(yaml.data(), yaml.size(), &g.h), "scene");
+        fw_scene* h = g.h;
+        for (int i = 0; i < fw_scene_num_assets(h); ++i) {
+            const std::string path = find_asset(fw_scene_asset_path(h, i));
+            uint32_t w = 0, ht = 0;
+            if (fw_scene_asset_kind(h, i) == 0) {
+                uint8_t* px = nullptr;
+                detail::check(fw_image_load(path.c_str(), &w, &ht, &px), "ImageTexture");
+                int rc = fw_scene_set_image(h, i, w, ht, px);
+                fw_image_free(px);
+                detail::check(rc, "ImageTexture");
+            } else {
+                float* px = nullptr;
+                detail::check(fw_hdr_load(path.c_str(), &w, &ht, &px), "HdrEnvironment");
+                int rc = fw_scene_set_hdr(h, i, w, ht, px);
+                fw_hdr_free(px);
+                detail::check(rc, "HdrEnvironment");
+            }
+        }
+        detail::check(fw_scene_commit(h, 0), "commit");
+    }
     std::string find_asset(const std::string& path) const {
         const std::string base = path.substr(path.find_last_of('/') == std::string::npos ? 0 : path.find_last_of('/') + 1);
         const std::string cands[] = {path, asset_dir_ + "/" + path, asset_dir_ + "/" + base, asset_dir_ + "/assets/" + base};

@@ -186,6 +186,31 @@ int fw_denoise_host(int device, uint32_t width, uint32_t height, const float* co
 int fw_render_denoised(fw_scene* scene, const fw_params* params, const fw_denoise* settings, uint8_t* rgb_out, float* sum_out,
                        float* denoised_out, float* variance_out, const fw_aov* aov, fw_stats* stats);
 
+/* ---- path tracing of caller-supplied rays (no reference counterpart; DESIGN.md §13) ------------------------------------
+ * For every ray i < n and every sample s of [sample_begin, sample_begin + sample_count), one path of render.rs:12-33 `color()`
+ * (t_min 0.001, depth cap 10, every material, texture, medium and environment) starts at that ray, keyed as
+ * (pixel = keys ? keys[i] : i, sample s); its radiances are added in sample order in fp32, exactly as a render adds the samples of
+ * a pixel, into sum[3i .. 3i+2].  Rays are traced as given: not normalised, non-finite values not rejected (a NaN direction follows
+ * DESIGN.md §5).  Single GPU.
+ *   origins, dirs : fp32 x3 per ray.  per_sample = 0 (shared layout): n rays, each re-traced for every sample, so the samples of a
+ *                   ray differ only in their scatter and medium draws.  per_sample != 0: sample_count * n rays, sample-major, the ray
+ *                   of (i, s) at entry (s - sample_begin) * n + i — fw_primary_rays' rays in this layout give fw_render's sums bit
+ *                   for bit.
+ *   keys          : nullable, uint32 per ray.
+ * Two calls that use the same (key, sample) pairs draw the same random numbers: work split over several calls needs disjoint keys
+ * or disjoint sample ranges.  Argument errors (null scene / rays / sum, n == 0 or n >= 2^31, sample_count == 0,
+ * sample_begin + sample_count > 2^32) are reported before any CUDA call; an uncommitted scene gives FW_ERR_STATE.
+ *
+ * fw_trace_rays : host buffers; sum_out receives n*3 fp32 sums; synchronous; stats->samples = n * sample_count.
+ * fw_trace_rays_device : device pointers on the scene's device; ADDS into d_sum (n*3 fp32) on `cuda_stream` (a cudaStream_t, or
+ *                 NULL for the scene's own stream) and returns once the work is enqueued and statistics are read back, as
+ *                 fw_render_accumulate_device does. */
+int fw_trace_rays(fw_scene* scene, uint64_t n, const float* origins, const float* dirs, const uint32_t* keys, int per_sample,
+                  uint32_t sample_begin, uint32_t sample_count, uint64_t seed, int use_bvh, float* sum_out, fw_stats* stats);
+int fw_trace_rays_device(fw_scene* scene, uint64_t n, const float* d_origins, const float* d_dirs, const uint32_t* d_keys, int per_sample,
+                         uint32_t sample_begin, uint32_t sample_count, uint64_t seed, int use_bvh, float* d_sum, void* cuda_stream,
+                         fw_stats* stats);
+
 /* Device-resident variant for multi-GPU sharding: ADDS the sample range into d_sum (device pointer,
  * width*height*3 fp32, on the scene's device) on `cuda_stream` (a cudaStream_t, or NULL for the scene's own
  * stream) and returns once the work is enqueued and statistics are read back. */
