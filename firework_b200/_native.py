@@ -58,7 +58,7 @@ EXPORTS = [
     "fw_scene_asset_kind", "fw_scene_set_image", "fw_scene_set_hdr", "fw_scene_build_host", "fw_scene_commit", "fw_scene_num_objects",
     "fw_scene_num_nodes", "fw_scene_device_bytes", "fw_scene_top_leaf_order", "fw_scene_object_aabb", "fw_scene_mesh_leaf_order", "fw_scene_linear_program", "fw_scene_bvh_nodes", "fw_render",
     "fw_render_accumulate_device", "fw_resolve_device", "fw_primary_rays", "fw_first_hit", "fw_scatter_step",
-    "fw_env_sample", "fw_texture_sample", "fw_material_texture", "fw_camera", "fw_last_error", "fw_version",
+    "fw_scatter_step_keyed",    "fw_env_sample", "fw_texture_sample", "fw_material_texture", "fw_camera", "fw_last_error", "fw_version",
     "fw_device_count", "fw_measure_peaks", "fw_selftest_shared_division", "fw_obj_load", "fw_obj_num_models",
     "fw_obj_model_name", "fw_obj_model_sizes", "fw_obj_model_copy", "fw_obj_destroy", "fw_hdr_load", "fw_hdr_free", "fw_image_load", "fw_image_free", "fw_png_write", "fw_set_profiling", "fw_set_batch_paths", "fw_release_cached_memory", "fw_texture_store_stats",
     "fw_resolve_host", "fw_render_multi", "fw_scene_walk_info", "fw_first_hit_wavefront", "fw_render_adaptive",
@@ -134,6 +134,7 @@ def lib():
         L.fw_first_hit.argtypes = [C.c_void_p, C.c_int, C.c_uint64, C.c_uint32] + [C.c_void_p] * 13
         L.fw_first_hit_wavefront.argtypes = [C.c_void_p, C.c_int, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32] + [C.c_void_p] * 7
         L.fw_scatter_step.argtypes = [C.c_void_p, C.c_uint32] + [C.c_void_p] * 8 + [C.c_uint32] + [C.c_void_p] * 6
+        L.fw_scatter_step_keyed.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32] + [C.c_void_p] * 16
         L.fw_env_sample.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]
         L.fw_texture_sample.argtypes = [C.c_void_p, C.c_int, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]
         L.fw_material_texture.argtypes = [C.c_void_p, C.c_int]

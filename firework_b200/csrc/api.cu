@@ -1705,32 +1705,55 @@ int fw_first_hit_wavefront(fw_scene* sc, int use_bvh, uint64_t seed, uint32_t n,
     return hit.get(n, obj, prim, material, t, point, normal, uv);
 }
 
-int fw_scatter_step(fw_scene* sc, uint32_t n, const int32_t* material, const float* ray_o, const float* ray_d,
-                    const float* hit_t, const float* hit_point, const float* hit_normal, const float* hit_uv,
-                    const float* uniforms, uint32_t nu, float* emit, int32_t* scattered, float* atten, float* out_o,
-                    float* out_d, int32_t* consumed) {
-    if (!sc || !material || !ray_o || !ray_d || !hit_t || !hit_point || !hit_normal || !hit_uv || !uniforms || !emit ||
-        !scattered || !atten || !out_o || !out_d || !consumed)
+// fw_scatter_step (uniforms != nullptr) and fw_scatter_step_keyed (pixel / sample / bounce keys) share everything else.
+static int scatter_probe(fw_scene* sc, uint32_t n, const int32_t* material, const float* ray_o, const float* ray_d,
+                         const float* hit_t, const float* hit_point, const float* hit_normal, const float* hit_uv,
+                         const float* uniforms, uint32_t nu, uint64_t seed, const uint32_t* pixel, const uint32_t* sample,
+                         const uint32_t* bounce, float* emit, int32_t* scattered, float* atten, float* out_o, float* out_d,
+                         int32_t* consumed) {
+    if (!sc || !material || !ray_o || !ray_d || !hit_t || !hit_point || !hit_normal || !hit_uv || !emit || !scattered ||
+        !atten || !out_o || !out_d || !consumed || (!uniforms && (!pixel || !sample || !bounce)))
         return set_error(FW_ERR_ARG, "null argument");
     if (!sc->committed) return set_error(FW_ERR_STATE, "scene not committed");
     for (uint32_t i = 0; i < n; ++i)
         if (material[i] < 0 || material[i] >= (int)sc->desc.mats.size()) return set_error(FW_ERR_ARG, "material index out of range");
     FW_CUDA(cudaSetDevice(sc->device));
-    DevBuf m, ro, rd, ht, hp, hn, hu, un, e, s, a, oo, od, c;
+    DevBuf m, ro, rd, ht, hp, hn, hu, un, kp, ks, kb, e, s, a, oo, od, c;
     TRY(m.put(material, (size_t)n * 4)); TRY(ro.put(ray_o, (size_t)n * 12)); TRY(rd.put(ray_d, (size_t)n * 12));
     TRY(ht.put(hit_t, (size_t)n * 4)); TRY(hp.put(hit_point, (size_t)n * 12)); TRY(hn.put(hit_normal, (size_t)n * 12));
-    TRY(hu.put(hit_uv, (size_t)n * 8)); TRY(un.put(uniforms, (size_t)n * nu * 4));
+    TRY(hu.put(hit_uv, (size_t)n * 8));
+    if (uniforms) {
+        TRY(un.put(uniforms, (size_t)n * nu * 4));
+    } else {
+        TRY(kp.put(pixel, (size_t)n * 4)); TRY(ks.put(sample, (size_t)n * 4)); TRY(kb.put(bounce, (size_t)n * 4));
+    }
     TRY(e.alloc((size_t)n * 12)); TRY(s.alloc((size_t)n * 4)); TRY(a.alloc((size_t)n * 12)); TRY(oo.alloc((size_t)n * 12));
     TRY(od.alloc((size_t)n * 12)); TRY(c.alloc((size_t)n * 4));
     ScatterProbeIO io{m.as<int>(), ro.as<float>(), rd.as<float>(), ht.as<float>(), hp.as<float>(), hn.as<float>(),
-                      hu.as<float>(), un.as<float>(), nu, e.as<float>(), s.as<int>(), a.as<float>(), oo.as<float>(),
-                      od.as<float>(), c.as<int>()};
+                      hu.as<float>(), uniforms ? un.as<float>() : nullptr, nu,
+                      make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)), kp.as<uint32_t>(), ks.as<uint32_t>(), kb.as<uint32_t>(),
+                      e.as<float>(), s.as<int>(), a.as<float>(), oo.as<float>(), od.as<float>(), c.as<int>()};
     launch_scatter_step_probe(sc->dscene, n, io, grid_for(n, 128, 4096), sc->ctx->stream);
     FW_CUDA(cudaGetLastError());
     FW_CUDA(cudaStreamSynchronize(sc->ctx->stream));
     TRY(e.get(emit, (size_t)n * 12)); TRY(s.get(scattered, (size_t)n * 4)); TRY(a.get(atten, (size_t)n * 12));
     TRY(oo.get(out_o, (size_t)n * 12)); TRY(od.get(out_d, (size_t)n * 12)); TRY(c.get(consumed, (size_t)n * 4));
     return FW_OK;
+}
+int fw_scatter_step(fw_scene* sc, uint32_t n, const int32_t* material, const float* ray_o, const float* ray_d,
+                    const float* hit_t, const float* hit_point, const float* hit_normal, const float* hit_uv,
+                    const float* uniforms, uint32_t nu, float* emit, int32_t* scattered, float* atten, float* out_o,
+                    float* out_d, int32_t* consumed) {
+    if (!uniforms) return set_error(FW_ERR_ARG, "null argument");
+    return scatter_probe(sc, n, material, ray_o, ray_d, hit_t, hit_point, hit_normal, hit_uv, uniforms, nu, 0, nullptr, nullptr,
+                         nullptr, emit, scattered, atten, out_o, out_d, consumed);
+}
+int fw_scatter_step_keyed(fw_scene* sc, uint64_t seed, uint32_t n, const int32_t* material, const float* ray_o,
+                          const float* ray_d, const float* hit_t, const float* hit_point, const float* hit_normal,
+                          const float* hit_uv, const uint32_t* pixel, const uint32_t* sample, const uint32_t* bounce,
+                          float* emit, int32_t* scattered, float* atten, float* out_o, float* out_d, int32_t* consumed) {
+    return scatter_probe(sc, n, material, ray_o, ray_d, hit_t, hit_point, hit_normal, hit_uv, nullptr, 0, seed, pixel, sample,
+                         bounce, emit, scattered, atten, out_o, out_d, consumed);
 }
 
 int fw_env_sample(fw_scene* sc, uint32_t n, const float* dirs, float* out) {

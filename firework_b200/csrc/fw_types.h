@@ -30,6 +30,9 @@ enum MatKind : int {  // material.rs; MAT_MISS is a queue id only
     MAT_NUM_QUEUES = 6
 };
 enum TexKind : int { TEX_CONSTANT = 0, TEX_CHECKER = 1, TEX_PERLIN = 2, TEX_TURBULENCE = 3, TEX_MARBLE = 4, TEX_IMAGE = 5 };
+// Textures on the longest root-to-leaf path of one texture tree (CheckerTextures nest): texture_sample follows at most this many
+// links, and the loader refuses deeper trees.
+constexpr int FW_MAX_TEXTURE_DEPTH = 64;
 enum EnvKind : int { ENV_COLOR = 0, ENV_SKY = 1, ENV_HDR = 2 };
 
 // Linear-scan program (Renderer.use_bvh == false, scene.rs:137-149).  The scene's objects, in scene order, are

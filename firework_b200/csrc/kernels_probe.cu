@@ -68,6 +68,22 @@ __global__ void first_hit_prog_probe(const __grid_constant__ LinProgram P, Devic
     atomicAdd(&out.counters[0], cnt.node_tests);
     atomicAdd(&out.counters[1], cnt.prim_tests);
 }
+// One emit + scatter step per item.  Stream = ArrayStream: explicit uniforms; Stream = PhiloxStream: the keyed stream
+// scatter_segment draws from, so the production sampler (random_in_unit_sphere_fresh) runs.
+template <class Stream>
+FW_DEV Stream scatter_probe_stream(const ScatterProbeIO& io, uint32_t i);
+template <>
+FW_DEV ArrayStream scatter_probe_stream<ArrayStream>(const ScatterProbeIO& io, uint32_t i) {
+    return ArrayStream(io.uniforms + (size_t)i * io.nu, (int)io.nu);
+}
+template <>
+FW_DEV PhiloxStream scatter_probe_stream<PhiloxStream>(const ScatterProbeIO& io, uint32_t i) {
+    return PhiloxStream(RngKey{io.seed, io.pixel[i], io.sample[i], io.bounce[i]}, STREAM_SCATTER);
+}
+FW_DEV int scatter_probe_consumed(const ArrayStream& rng) { return rng.overrun ? -1 : rng.i; }
+FW_DEV int scatter_probe_consumed(const PhiloxStream& rng) { return (int)rng.idx; }
+
+template <class Stream>
 __global__ void scatter_step_probe(DeviceScene S, uint32_t n, ScatterProbeIO io) {
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         int mat = io.material[i];
@@ -78,7 +94,7 @@ __global__ void scatter_step_probe(DeviceScene S, uint32_t n, ScatterProbeIO io)
         float3 point = f3(io.hit_point[3 * i], io.hit_point[3 * i + 1], io.hit_point[3 * i + 2]);
         float3 normal = f3(io.hit_normal[3 * i], io.hit_normal[3 * i + 1], io.hit_normal[3 * i + 2]);
         float2 uv = make_float2(io.hit_uv[2 * i], io.hit_uv[2 * i + 1]);
-        ArrayStream rng(io.uniforms + (size_t)i * io.nu, (int)io.nu);
+        Stream rng = scatter_probe_stream<Stream>(io, i);
         ScatterOut out;
         out.scattered = false;
         out.attenuation = out.origin = out.dir = f3(0.0f, 0.0f, 0.0f);
@@ -96,7 +112,7 @@ __global__ void scatter_step_probe(DeviceScene S, uint32_t n, ScatterProbeIO io)
         io.atten[3 * i] = out.attenuation.x; io.atten[3 * i + 1] = out.attenuation.y; io.atten[3 * i + 2] = out.attenuation.z;
         io.out_o[3 * i] = out.origin.x; io.out_o[3 * i + 1] = out.origin.y; io.out_o[3 * i + 2] = out.origin.z;
         io.out_d[3 * i] = out.dir.x; io.out_d[3 * i + 1] = out.dir.y; io.out_d[3 * i + 2] = out.dir.z;
-        io.consumed[i] = rng.overrun ? -1 : rng.i;
+        io.consumed[i] = scatter_probe_consumed(rng);
     }
 }
 
@@ -240,7 +256,8 @@ void launch_first_hit_probe(int mode, const LinProgram& prog, const DeviceScene&
     }
 }
 void launch_scatter_step_probe(const DeviceScene& S, uint32_t n, const ScatterProbeIO& io, unsigned blocks, cudaStream_t st) {
-    scatter_step_probe<<<blocks, 128, 0, st>>>(S, n, io);
+    if (io.uniforms) scatter_step_probe<ArrayStream><<<blocks, 128, 0, st>>>(S, n, io);
+    else scatter_step_probe<PhiloxStream><<<blocks, 128, 0, st>>>(S, n, io);
 }
 void launch_env_sample_probe(const DeviceScene& S, uint32_t n, const float* dirs, float* out, unsigned blocks, cudaStream_t st) {
     env_sample_probe<<<blocks, 256, 0, st>>>(S, n, dirs, out);

@@ -113,10 +113,15 @@ struct Loader {
         return (int)sc.assets.size() - 1;
     }
 
-    // texture.rs — returns texture index or -1
-    int texture(const Node* n) {
+    // texture.rs — returns texture index or -1.  `level` is the texture's place on its root-to-leaf path (the root is 1).
+    int texture(const Node* n, int level = 1) {
         if (!n) return -1;
         if (n->kind != Node::MAP) { fail(n, "expected a texture mapping"); return -1; }
+        if (level > FW_MAX_TEXTURE_DEPTH) {
+            fail(n, "texture tree deeper than " + std::to_string(FW_MAX_TEXTURE_DEPTH) + " levels: the renderer follows at most " +
+                        std::to_string(FW_MAX_TEXTURE_DEPTH - 1) + " nested CheckerTextures over a leaf texture");
+            return -1;
+        }
         std::string tag;
         if (!as_str(req(*n, "texture"), tag)) return -1;
         TexRec t;
@@ -126,8 +131,8 @@ struct Loader {
             if (!as_v3(req(*n, "color"), t.color)) return -1;
         } else if (tag == "CheckerTexture") {
             t.kind = TEX_CHECKER;
-            t.a = texture(req(*n, "odd"));
-            t.b = texture(req(*n, "even"));
+            t.a = texture(req(*n, "odd"), level + 1);
+            t.b = texture(req(*n, "even"), level + 1);
             if (t.a < 0 || t.b < 0) return -1;
             if (!as_f32(req(*n, "scale"), t.scale)) return -1;
         } else if (tag == "PerlinNoiseTexture") {
@@ -784,7 +789,7 @@ bool flatten_scene(const SceneDesc& desc, HostFlat& out, std::string& err) {
     {
         // uv is read only by ImageTexture::sample (texture.rs:296-309); checker forwards it to its children
         std::function<bool(int, int)> reads_uv = [&](int t, int depth) -> bool {
-            if (t < 0 || t >= (int)desc.texs.size() || depth > 64) return false;
+            if (t < 0 || t >= (int)desc.texs.size() || depth >= FW_MAX_TEXTURE_DEPTH) return false;
             const TexRec& r = desc.texs[t];
             if (r.kind == TEX_IMAGE) return true;
             if (r.kind == TEX_CHECKER) return reads_uv(r.a, depth + 1) || reads_uv(r.b, depth + 1);

@@ -38,6 +38,9 @@ FW_DEV float perlin_grad(unsigned hash, float x, float y, float z) {      // tex
 FW_DEV float perlin_lerp(float t, float a, float b) { return a + t * (b - a); }  // texture.rs:184-186
 // `floor(x) as usize & 255`: the Rust cast saturates (negatives and NaN -> 0, huge -> usize::MAX -> 255)
 FW_DEV unsigned perlin_cell(float f) { return (unsigned)(__float2ull_rz(f) & 255ull); }
+// Rust `f as u64` / `f as u32`: saturating, NaN -> 0.  The hardware conversion saturates but does not map NaN to 0.
+FW_DEV unsigned long long f32_as_u64(float f) { return f == f ? __float2ull_rz(f) : 0ull; }
+FW_DEV uint32_t f32_as_u32(float f) { return f == f ? __float2uint_rz(f) : 0u; }
 FW_DEV float perlin_noise(float3 p) {  // texture.rs:113-158
     float fx = floorf(p.x), fy = floorf(p.y), fz = floorf(p.z);
     unsigned x0 = perlin_cell(fx), y0 = perlin_cell(fy), z0 = perlin_cell(fz);
@@ -74,7 +77,7 @@ FW_DEV float turbulence(int depth, float3 point) {  // texture.rs:206-217 — no
 }
 
 FW_DEV float3 texture_sample(const DeviceScene& S, int tex, float2 uv, float3 point) {
-    for (int guard = 0; guard < 64; ++guard) {
+    for (int guard = 0; guard < FW_MAX_TEXTURE_DEPTH; ++guard) {
         const float4* q = reinterpret_cast<const float4*>(&S.texs[tex]);
         float4 q0 = __ldg(q), q1 = __ldg(q + 1);
         int kind = __float_as_int(q0.x);
@@ -83,11 +86,20 @@ FW_DEV float3 texture_sample(const DeviceScene& S, int tex, float2 uv, float3 po
             case TEX_CONSTANT:  // texture.rs:31-33
                 return f3(q1.y, q1.z, q1.w);
             case TEX_CHECKER: {  // texture.rs:59-72 — product().is_sign_positive()
+                float ax = scale * point.x, ay = scale * point.y, az = scale * point.z;
                 float prod = 1.0f;
-                prod = prod * sinf(scale * point.x);
-                prod = prod * sinf(scale * point.y);
-                prod = prod * sinf(scale * point.z);
-                tex = signbit(prod) ? __float_as_int(q0.y) : __float_as_int(q0.z);  // odd : even
+                prod = prod * sinf(ax);
+                prod = prod * sinf(ay);
+                prod = prod * sinf(az);
+                bool odd = signbit(prod);
+                if (prod != prod) {
+                    // The reference's NaN sign is x86's (DESIGN.md §3): the first axis whose sin is NaN decides; that NaN is
+                    // the coordinate's own, or the negative default NaN of sin(±inf) / 0 * inf.  Device arithmetic yields
+                    // only the positive canonical NaN, so the sign is decided here.
+                    float c = isfinite(ax) ? (isfinite(ay) ? point.z : point.y) : point.x;
+                    odd = !(c != c) || signbit(c);
+                }
+                tex = odd ? __float_as_int(q0.y) : __float_as_int(q0.z);  // odd : even
                 continue;
             }
             case TEX_PERLIN: {  // texture.rs:160-167
@@ -108,8 +120,8 @@ FW_DEV float3 texture_sample(const DeviceScene& S, int tex, float2 uv, float3 po
                 uint32_t w = im->w, h = im->h;
                 float fi = uv.x * (float)w;
                 float fj = (1.0f - uv.y) * (float)h;
-                uint32_t i = min(__float2uint_rz(fi), w - 1);  // saturating like Rust `as u32`
-                uint32_t j = min(__float2uint_rz(fj), h - 1);
+                uint32_t i = min(f32_as_u32(fi), w - 1);
+                uint32_t j = min(f32_as_u32(fj), h - 1);
                 uchar4 c = tex2D<uchar4>(im->tex, (float)i + 0.5f, (float)j + 0.5f);
                 return f3((float)c.x, (float)c.y, (float)c.z) / 255.0f;
             }
@@ -136,9 +148,9 @@ FW_DEV float3 environment_sample(const EnvRec& env, float3 raw_dir) {
     float u = 1.0f - (phi + FW_PI) / (2.0f * FW_PI);
     float v = (theta + FW_PI / 2.0f) / FW_PI;
     float width = (float)env.w, height = (float)env.h;
-    unsigned long long x = __float2ull_rz(u * width);
-    unsigned long long y = __float2ull_rz((1.0f - v) * height);
-    unsigned long long idx = __float2ull_rz((float)y * width) + x;
+    unsigned long long x = f32_as_u64(u * width);
+    unsigned long long y = f32_as_u64((1.0f - v) * height);
+    unsigned long long idx = f32_as_u64((float)y * width) + x;
     // DEVIATION (documented in DESIGN.md): the reference panics on an out-of-range index (dir.y == -1);
     // here the index is clamped to the last texel.
     unsigned long long n = (unsigned long long)env.w * env.h;

@@ -63,6 +63,9 @@ struct ScatterProbeIO {
     const int* material;
     const float *ray_o, *ray_d, *hit_t, *hit_point, *hit_normal, *hit_uv, *uniforms;
     uint32_t nu;
+    // keyed probe (uniforms == nullptr): item i draws from PhiloxStream({seed, pixel[i], sample[i], bounce[i]}, STREAM_SCATTER)
+    uint2 seed;
+    const uint32_t *pixel, *sample, *bounce;
     float* emit;
     int* scattered;
     float *atten, *out_o, *out_d;

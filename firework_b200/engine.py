@@ -339,6 +339,20 @@ class NativeScene:
                                         N.ptr(res["atten"]), N.ptr(res["o"]), N.ptr(res["d"]), N.ptr(res["consumed"])))
         return res
 
+    def scatter_step_keyed(self, material, ray_o, ray_d, hit_t, hit_point, hit_normal, hit_uv, seed, pixel, sample, bounce):
+        """scatter_step drawing from the render's keyed Philox stream; "consumed" counts the uniforms drawn."""
+        n = len(material)
+        material = np.ascontiguousarray(material, np.int32)
+        arrs = [np.ascontiguousarray(a, np.float32) for a in (ray_o, ray_d, hit_t, hit_point, hit_normal, hit_uv)]
+        keys = [np.ascontiguousarray(np.broadcast_to(k, (n,)), np.uint32) for k in (pixel, sample, bounce)]
+        res = {"emit": np.zeros((n, 3), np.float32), "scattered": np.zeros(n, np.int32),
+               "atten": np.zeros((n, 3), np.float32), "o": np.zeros((n, 3), np.float32),
+               "d": np.zeros((n, 3), np.float32), "consumed": np.zeros(n, np.int32)}
+        N.check(N.lib().fw_scatter_step_keyed(self._h, C.c_uint64(seed), n, N.ptr(material), *[N.ptr(a) for a in arrs],
+                                              *[N.ptr(k) for k in keys], N.ptr(res["emit"]), N.ptr(res["scattered"]),
+                                              N.ptr(res["atten"]), N.ptr(res["o"]), N.ptr(res["d"]), N.ptr(res["consumed"])))
+        return res
+
     def env_sample(self, dirs):
         d = np.ascontiguousarray(dirs, np.float32)
         out = np.zeros_like(d)

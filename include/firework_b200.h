@@ -246,6 +246,9 @@ int fw_render_multi(fw_scene* scene, const fw_params* params, int n_gpus, const 
  *                   the ConstantMedium draw (may be NULL: pixel = i, sample = bounce = 0).
  *                   counters (nullable) receives {node tests, primitive tests}.
  * fw_scatter_step : render.rs:20-22 emit + scatter with EXPLICIT uniforms (nu per item, consumed in order).
+ * fw_scatter_step_keyed : the same step drawing from the render's own stream, Philox keyed by (seed, pixel[i],
+ *                   sample[i], bounce[i]) and the scatter stream kind, through the samplers the shade kernels use;
+ *                   consumed[i] = uniforms drawn.
  * fw_env_sample / fw_texture_sample : render.rs:31 / texture.rs lookups.                                 */
 int fw_primary_rays(fw_scene* scene, const fw_params* params, uint32_t sample, uint32_t pix_begin, uint32_t n,
                     float* origins, float* dirs);
@@ -263,6 +266,10 @@ int fw_scatter_step(fw_scene* scene, uint32_t n, const int32_t* material, const 
                     const float* hit_t, const float* hit_point, const float* hit_normal, const float* hit_uv,
                     const float* uniforms, uint32_t nu, float* emit, int32_t* scattered, float* atten, float* out_o,
                     float* out_d, int32_t* consumed);
+int fw_scatter_step_keyed(fw_scene* scene, uint64_t seed, uint32_t n, const int32_t* material, const float* ray_o,
+                          const float* ray_d, const float* hit_t, const float* hit_point, const float* hit_normal,
+                          const float* hit_uv, const uint32_t* pixel, const uint32_t* sample, const uint32_t* bounce,
+                          float* emit, int32_t* scattered, float* atten, float* out_o, float* out_d, int32_t* consumed);
 int fw_env_sample(fw_scene* scene, uint32_t n, const float* dirs, float* out);
 int fw_texture_sample(fw_scene* scene, int texture, uint32_t n, const float* uv, const float* point, float* out);
 int fw_material_texture(const fw_scene* scene, int material);  /* texture index of a material, or -1 */

@@ -810,10 +810,14 @@ struct CheckerTexture : Texture {  // texture.rs:57-73
     float scale;
     Vec3 sample(Vec2 uv, const Vec3& point) const override {
         // iter().map(|x| (scale*x).sin()).product::<f32>() : fold starting at 1.0
+        float sx = std::sin(scale * point.x), sy = std::sin(scale * point.y), sz = std::sin(scale * point.z);
         float prod = 1.0f;
-        prod = prod * std::sin(scale * point.x);
-        prod = prod * std::sin(scale * point.y);
-        prod = prod * std::sin(scale * point.z);
+        prod = prod * sx;
+        prod = prod * sy;
+        prod = prod * sz;
+        // A product of two NaNs is one of them, chosen by the operand order of the multiply instruction, which the
+        // compiler picks (this file's -O2 and -O3 builds differ).  Pin it: the first NaN factor in x, y, z order decides.
+        if (std::isnan(prod)) prod = std::isnan(sx) ? sx : (std::isnan(sy) ? sy : sz);
         if (!std::signbit(prod)) return even->sample(uv, point);
         return odd->sample(uv, point);
     }
@@ -1556,9 +1560,33 @@ void orc_first_hit(void* sp, int use_bvh, uint64_t seed, uint32_t n, const float
     if (stats) { stats->rays = n; stats->aabb_tests = aabb; stats->prim_tests = prim; stats->samples = 0; }
 }
 
-// One scatter step (render.rs:20-22) with EXPLICIT uniforms consumed in order:
-// in:  material id, ray (o,d), hit (t, point, normal, uv), uniforms[nu]
-// out: emit[3], scattered flag, attenuation[3], new ray o[3], d[3], uniforms consumed
+// One scatter step (render.rs:20-22) of item i:
+// in:  material id, ray (o,d), hit (t, point, normal, uv), the item's random stream
+// out: emit[3], scattered flag, attenuation[3], new ray o[3], d[3]
+static void scatter_one(Scene* s, uint32_t i, const int32_t* material, const float* ray_o, const float* ray_d,
+                        const float* hit_t, const float* hit_point, const float* hit_normal, const float* hit_uv, Rng& rng,
+                        float* emit, int32_t* scattered, float* atten, float* out_o, float* out_d) {
+    Ray r{v3(ray_o[3 * i], ray_o[3 * i + 1], ray_o[3 * i + 2]), v3(ray_d[3 * i], ray_d[3 * i + 1], ray_d[3 * i + 2])};
+    RaycastHit h;
+    h.t = hit_t[i];
+    h.point = v3(hit_point[3 * i], hit_point[3 * i + 1], hit_point[3 * i + 2]);
+    h.normal = v3(hit_normal[3 * i], hit_normal[3 * i + 1], hit_normal[3 * i + 2]);
+    h.uv = Vec2{hit_uv[2 * i], hit_uv[2 * i + 1]};
+    h.material = material[i];
+    const Material& m = *s->materials.at(material[i]);
+    Vec3 e = m.emit(h.uv, h.point);
+    ScatterResult res;
+    res.attenuation = v3(0, 0, 0);
+    res.scattered = Ray{v3(0, 0, 0), v3(0, 0, 0)};
+    bool ok = m.scatter(r, h, rng, res);
+    emit[3 * i] = e.x; emit[3 * i + 1] = e.y; emit[3 * i + 2] = e.z;
+    scattered[i] = ok ? 1 : 0;
+    if (!ok) { res.attenuation = v3(0, 0, 0); res.scattered = Ray{v3(0, 0, 0), v3(0, 0, 0)}; }
+    atten[3 * i] = res.attenuation.x; atten[3 * i + 1] = res.attenuation.y; atten[3 * i + 2] = res.attenuation.z;
+    out_o[3 * i] = res.scattered.origin.x; out_o[3 * i + 1] = res.scattered.origin.y; out_o[3 * i + 2] = res.scattered.origin.z;
+    out_d[3 * i] = res.scattered.dir.x; out_d[3 * i + 1] = res.scattered.dir.y; out_d[3 * i + 2] = res.scattered.dir.z;
+}
+// ... with EXPLICIT uniforms consumed in order (nu per item); consumed = uniforms used, -1 on overrun
 void orc_scatter_step(void* sp, uint32_t n, const int32_t* material, const float* ray_o, const float* ray_d,
                       const float* hit_t, const float* hit_point, const float* hit_normal, const float* hit_uv,
                       const float* uniforms, uint32_t nu, float* emit, int32_t* scattered, float* atten,
@@ -1568,26 +1596,23 @@ void orc_scatter_step(void* sp, uint32_t n, const int32_t* material, const float
         Rng rng;
         rng.arr = uniforms + (size_t)i * nu;
         rng.arr_n = (int)nu;
-        Ray r{v3(ray_o[3 * i], ray_o[3 * i + 1], ray_o[3 * i + 2]), v3(ray_d[3 * i], ray_d[3 * i + 1], ray_d[3 * i + 2])};
-        RaycastHit h;
-        h.t = hit_t[i];
-        h.point = v3(hit_point[3 * i], hit_point[3 * i + 1], hit_point[3 * i + 2]);
-        h.normal = v3(hit_normal[3 * i], hit_normal[3 * i + 1], hit_normal[3 * i + 2]);
-        h.uv = Vec2{hit_uv[2 * i], hit_uv[2 * i + 1]};
-        h.material = material[i];
-        const Material& m = *s->materials.at(material[i]);
-        Vec3 e = m.emit(h.uv, h.point);
-        ScatterResult res;
-        res.attenuation = v3(0, 0, 0);
-        res.scattered = Ray{v3(0, 0, 0), v3(0, 0, 0)};
-        bool ok = m.scatter(r, h, rng, res);
-        emit[3 * i] = e.x; emit[3 * i + 1] = e.y; emit[3 * i + 2] = e.z;
-        scattered[i] = ok ? 1 : 0;
-        if (!ok) { res.attenuation = v3(0, 0, 0); res.scattered = Ray{v3(0, 0, 0), v3(0, 0, 0)}; }
-        atten[3 * i] = res.attenuation.x; atten[3 * i + 1] = res.attenuation.y; atten[3 * i + 2] = res.attenuation.z;
-        out_o[3 * i] = res.scattered.origin.x; out_o[3 * i + 1] = res.scattered.origin.y; out_o[3 * i + 2] = res.scattered.origin.z;
-        out_d[3 * i] = res.scattered.dir.x; out_d[3 * i + 1] = res.scattered.dir.y; out_d[3 * i + 2] = res.scattered.dir.z;
+        scatter_one(s, i, material, ray_o, ray_d, hit_t, hit_point, hit_normal, hit_uv, rng, emit, scattered, atten, out_o, out_d);
         consumed[i] = rng.arr_overrun ? -1 : rng.arr_i;
+    }
+}
+// ... drawing from the keyed stream color() uses at bounce[i] of (pixel[i], sample[i]); consumed = uniforms drawn
+void orc_scatter_step_keyed(void* sp, uint64_t seed, uint32_t n, const int32_t* material, const float* ray_o,
+                            const float* ray_d, const float* hit_t, const float* hit_point, const float* hit_normal,
+                            const float* hit_uv, const uint32_t* pixel, const uint32_t* sample, const uint32_t* bounce,
+                            float* emit, int32_t* scattered, float* atten, float* out_o, float* out_d, int32_t* consumed) {
+    Scene* s = (Scene*)sp;
+    for (uint32_t i = 0; i < n; ++i) {
+        Rng rng;
+        rng.seed(seed);
+        rng.begin(pixel[i], sample[i]);
+        rng.set_stream(bounce[i], STREAM_SCATTER);
+        scatter_one(s, i, material, ray_o, ray_d, hit_t, hit_point, hit_normal, hit_uv, rng, emit, scattered, atten, out_o, out_d);
+        consumed[i] = (int32_t)rng.idx;
     }
 }
 

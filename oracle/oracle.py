@@ -295,6 +295,21 @@ class OracleScene:
                                   _fp(res["d"]), res["consumed"].ctypes.data_as(i32p))
         return res
 
+    def scatter_step_keyed(self, material, ray_o, ray_d, hit_t, hit_point, hit_normal, hit_uv, seed, pixel, sample, bounce):
+        n = len(material)
+        material = np.ascontiguousarray(material, np.int32)
+        arrs = [np.ascontiguousarray(a, np.float32) for a in (ray_o, ray_d, hit_t, hit_point, hit_normal, hit_uv)]
+        keys = [np.ascontiguousarray(np.broadcast_to(k, (n,)), np.uint32) for k in (pixel, sample, bounce)]
+        res = {"emit": np.zeros((n, 3), np.float32), "scattered": np.zeros(n, np.int32),
+               "atten": np.zeros((n, 3), np.float32), "o": np.zeros((n, 3), np.float32),
+               "d": np.zeros((n, 3), np.float32), "consumed": np.zeros(n, np.int32)}
+        i32p, u32p = C.POINTER(C.c_int32), C.POINTER(C.c_uint32)
+        self.lib.orc_scatter_step_keyed(self.h, C.c_uint64(seed), C.c_uint32(n), material.ctypes.data_as(i32p),
+                                        *[_fp(a) for a in arrs], *[k.ctypes.data_as(u32p) for k in keys],
+                                        _fp(res["emit"]), res["scattered"].ctypes.data_as(i32p), _fp(res["atten"]),
+                                        _fp(res["o"]), _fp(res["d"]), res["consumed"].ctypes.data_as(i32p))
+        return res
+
     def env_sample(self, dirs):
         d = np.ascontiguousarray(dirs, np.float32)
         out = np.zeros_like(d)
