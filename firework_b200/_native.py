@@ -62,7 +62,7 @@ EXPORTS = [
     "fw_device_count", "fw_measure_peaks", "fw_selftest_shared_division", "fw_obj_load", "fw_obj_num_models",
     "fw_obj_model_name", "fw_obj_model_sizes", "fw_obj_model_copy", "fw_obj_destroy", "fw_hdr_load", "fw_hdr_free", "fw_image_load", "fw_image_free", "fw_png_write", "fw_set_profiling", "fw_set_batch_paths", "fw_release_cached_memory", "fw_texture_store_stats",
     "fw_resolve_host", "fw_render_multi", "fw_scene_walk_info", "fw_first_hit_wavefront", "fw_render_adaptive",
-    "fw_render_aov", "fw_denoise_host", "fw_render_denoised", "fw_trace_rays", "fw_trace_rays_device",
+    "fw_render_aov", "fw_denoise_host", "fw_render_denoised", "fw_trace_rays", "fw_trace_rays_device", "fw_bvh_build",
 ]
 
 _lib = None
@@ -125,6 +125,7 @@ def lib():
         L.fw_scene_object_aabb.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         L.fw_scene_mesh_leaf_order.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int]
         L.fw_scene_bvh_nodes.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_int)]
+        L.fw_bvh_build.argtypes = [C.c_int, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         if hasattr(L, "fw_scene_linear_program"):   # absent only in older builds used for A/B timing
             L.fw_scene_linear_program.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
         L.fw_render.argtypes = [C.c_void_p, C.POINTER(FwParams), C.c_void_p, C.c_void_p, C.POINTER(FwStats)]

@@ -19,7 +19,7 @@ STATIC_LIB = os.path.join(HERE, "libfirework_b200.a")
 CLI = os.path.join(HERE, "bin", "firework")          # native driver (csrc/cli_main.cpp), links the static archive
 LINK_LIBS = ["-lcudart_static", "-lz", "-ldl", "-lpthread", "-lrt"]   # zlib: PNG inflate / deflate (images.cpp), .yml.gz (cli)
 SOURCES = ["api.cu", "multi_gpu.cu", "kernels_extend.cu", "kernels_walk.cu", "kernels_shade.cu", "kernels_probe.cu",
-           "kernels_adaptive.cu", "kernels_denoise.cu", "scene_host.cpp", "yaml_lite.cpp", "formats.cpp", "images.cpp"]
+           "kernels_adaptive.cu", "kernels_denoise.cu", "kernels_build.cu", "scene_host.cpp", "yaml_lite.cpp", "formats.cpp", "images.cpp"]
 HEADERS = ["fw_types.h", "scene_host.h", "yaml_lite.h", "device_math.cuh", "intersect.cuh", "shade.cuh", "wavefront.cuh",
            "wavefront_types.h", "launch.h", "api_internal.h", "walk.cuh", os.path.join("..", "..", "include", "firework_b200.h")]
 

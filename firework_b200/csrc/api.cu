@@ -647,8 +647,14 @@ int fw_scene_commit(fw_scene* sc, int device) {
         const fw_scene* src = sc->asset_src ? sc->asset_src : sc;
         for (const AssetDesc& a : src->desc.assets)
             if (!a.provided) return set_error(FW_ERR_ASSET, "asset `" + a.path + "` was not provided (fw_scene_set_image / fw_scene_set_hdr)");
-        int brc = fw_scene_build_host(sc);
-        if (brc != FW_OK) return brc;
+        if (!sc->built) {   // large trees are built on the device being committed to (kDeviceBvhMinItems)
+            int n = 0;
+            const bool dev_ok = cudaGetDeviceCount(&n) == cudaSuccess && device >= 0 && device < n;
+            std::string err;
+            BvhDeviceScope on(dev_ok ? device : -1);
+            if (!flatten_scene(sc->desc, sc->flat, err)) return set_error(on.code, err);
+            sc->built = true;
+        }
         int ndev = 0;
         FW_CUDA(cudaGetDeviceCount(&ndev));
         if (device < 0 || device >= ndev) return set_error(FW_ERR_CUDA, "no such CUDA device " + std::to_string(device));
@@ -814,6 +820,36 @@ int fw_scene_walk_info(const fw_scene* sc, int out[6]) {
     out[0] = F.walk_ok ? 1 : 0; out[1] = F.n_top_meshes; out[2] = F.top_wide_depth; out[3] = F.mesh_wide_depth;
     out[4] = F.walk_prim_bits; out[5] = (int)(F.tri_verts.size() / 3);
     return FW_OK;
+}
+int fw_bvh_build(int device, uint32_t n, const float* boxes, const uint8_t* unbounded, int32_t* items_out, float* nodes_out,
+                 int capacity_nodes, float root_box[6], int32_t info[4]) {
+    return guarded([&]() -> int {
+        if (n == 0) return set_error(FW_ERR_ARG, "n must be at least 1");
+        if (n > (uint32_t)INT32_MAX / 2) return set_error(FW_ERR_ARG, "n must be below 2^30");
+        if (!boxes || !items_out || !root_box || !info) return set_error(FW_ERR_ARG, "null argument");
+        if (capacity_nodes < 0) return set_error(FW_ERR_ARG, "capacity_nodes must not be negative");
+        if (device < -1) return set_error(FW_ERR_ARG, "device must be -1 (host) or a CUDA device");
+        std::vector<Box> b(n);
+        memcpy(b.data(), boxes, sizeof(Box) * (size_t)n);
+        std::vector<uint8_t> unb;
+        if (unbounded) unb.assign(unbounded, unbounded + n);
+        if (device >= 0) {
+            int ndev = 0;
+            FW_CUDA(cudaGetDeviceCount(&ndev));
+            if (device >= ndev) return set_error(FW_ERR_CUDA, "no such CUDA device " + std::to_string(device));
+        }
+        FlatBVH t;
+        std::string err;
+        const int rc = build_bvh_on(device, b, t, err, unbounded ? &unb : nullptr);
+        if (rc != FW_OK) return set_error(rc, err);
+        const int nodes = (int)(t.nodes.size() / 8);
+        memcpy(items_out, t.items.data(), sizeof(int) * (size_t)n);
+        if (nodes_out) memcpy(nodes_out, t.nodes.data(), sizeof(float4) * 8 * (size_t)std::min(nodes, capacity_nodes));
+        const Box& r = t.root_box;
+        root_box[0] = r.mn.x; root_box[1] = r.mn.y; root_box[2] = r.mn.z; root_box[3] = r.mx.x; root_box[4] = r.mx.y; root_box[5] = r.mx.z;
+        info[0] = nodes; info[1] = t.root_code; info[2] = t.wide_depth; info[3] = t.max_depth;
+        return FW_OK;
+    });
 }
 int fw_material_texture(const fw_scene* sc, int material) {
     if (!sc || material < 0 || material >= (int)sc->desc.mats.size()) return -1;

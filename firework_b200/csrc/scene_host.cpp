@@ -9,6 +9,7 @@
 #include <deque>
 #include <functional>
 
+#include "../../include/firework_b200.h"
 #include "yaml_lite.h"
 
 namespace fw {
@@ -401,7 +402,9 @@ static inline V3 box_center(const Box& b) {  // aabb.rs:59-61
 }
 
 // ------------------------------------------------------------------------------------------------------
-// BVH build: bvh.rs:21-71
+// BVH build: bvh.rs:21-71, in three stages: (a) the reference's median-split tree, which fixes the leaves;
+// (b) an SAH interior over those leaves; (c) the collapse into 4-wide nodes.  (a) and (b) run on the host or,
+// for large trees, on a CUDA device (kernels_build.cu); (c) is shared.
 // ------------------------------------------------------------------------------------------------------
 namespace {
 struct BuildNode {
@@ -411,25 +414,57 @@ struct BuildNode {
     int depth = 0;
     bool unbounded = false;     // some item below has a box that does not bound its geometry
 };
+// fminf / fmaxf as glibc computes them on x86-64 (minss / maxss plus its NaN path): a quiet NaN operand loses, two quiet
+// NaNs give the first, a signaling NaN gives a + b, and a tie (-0.0 against +0.0) gives the SECOND operand.  Spelled out
+// for the node boxes because a compiler may swap the operands of a call it knows to be commutative, and the signs of zero
+// in those boxes are part of the flattened tree.
+static inline bool is_snan(float x) {
+    uint32_t u;
+    memcpy(&u, &x, 4);
+    return (u & 0x7fc00000u) == 0x7f800000u && (u & 0x003fffffu) != 0;
+}
+static inline float lib_min(float a, float b) {
+    return a < b ? a : b < a ? b : (is_snan(a) || is_snan(b)) ? a + b : a != a ? (b != b ? a : b) : b != b ? a : b;
+}
+static inline float lib_max(float a, float b) {
+    return a > b ? a : b > a ? b : (is_snan(a) || is_snan(b)) ? a + b : a != a ? (b != b ? a : b) : b != b ? a : b;
+}
+// The median-split tree's boxes: box_expand(a, b).
+static inline Box node_union(const Box& a, const Box& b) {
+    return Box{V3{lib_min(a.mn.x, b.mn.x), lib_min(a.mn.y, b.mn.y), lib_min(a.mn.z, b.mn.z)},
+               V3{lib_max(a.mx.x, b.mx.x), lib_max(a.mx.y, b.mx.y), lib_max(a.mx.z, b.mx.z)}};
+}
+// An SAH interior node's box over children l and r, with the operand order its trees have always had.
+static inline Box sah_union(const Box& l, const Box& r) {
+    return Box{V3{lib_min(r.mn.x, l.mn.x), lib_min(r.mn.y, l.mn.y), lib_min(r.mn.z, l.mn.z)},
+               V3{lib_max(l.mx.x, r.mx.x), lib_max(r.mx.y, l.mx.y), lib_max(r.mx.z, l.mx.z)}};
+}
+// Stage (a).  With `sorted` the item order is already final (the device computed it) and only the shape and the boxes
+// are built here; the shape depends on n alone.
 struct Builder {
     const std::vector<Box>& boxes;
     std::vector<V3> centers;
     std::vector<int> order;
     std::vector<BuildNode> nodes;
     bool nan = false;
+    bool sorted = false;
     const std::vector<uint8_t>* unbounded = nullptr;
     explicit Builder(const std::vector<Box>& b) : boxes(b) {
-        centers.reserve(b.size());
-        for (const Box& x : b) centers.push_back(box_center(x));
         order.resize(b.size());
         for (size_t i = 0; i < b.size(); ++i) order[i] = (int)i;
     }
     int build(int lo, int n, int depth) {
-        int axis = depth % 3;
-        for (int i = lo; i < lo + n; ++i)
-            if (std::isnan(comp(centers[order[i]], axis))) nan = true;  // bvh.rs:34 would panic
-        std::stable_sort(order.begin() + lo, order.begin() + lo + n,
-                         [&](int a, int b) { return comp(centers[a], axis) < comp(centers[b], axis); });
+        if (!sorted) {
+            if (centers.empty()) {
+                centers.reserve(boxes.size());
+                for (const Box& x : boxes) centers.push_back(box_center(x));
+            }
+            int axis = depth % 3;
+            for (int i = lo; i < lo + n; ++i)
+                if (std::isnan(comp(centers[order[i]], axis))) nan = true;  // bvh.rs:34 would panic
+            std::stable_sort(order.begin() + lo, order.begin() + lo + n,
+                             [&](int a, int b) { return comp(centers[a], axis) < comp(centers[b], axis); });
+        }
         int id = (int)nodes.size();
         nodes.emplace_back();
         nodes[id].depth = depth;
@@ -439,7 +474,7 @@ struct Builder {
             nodes[id].count = 1;
             nodes[id].unbounded = unbounded && (*unbounded)[order[lo]];
         } else if (n == 2) {
-            nodes[id].box = box_expand(boxes[order[lo]], boxes[order[lo + 1]]);
+            nodes[id].box = node_union(boxes[order[lo]], boxes[order[lo + 1]]);
             nodes[id].first = lo;
             nodes[id].count = 2;
             nodes[id].unbounded = unbounded && ((*unbounded)[order[lo]] || (*unbounded)[order[lo + 1]]);
@@ -449,7 +484,7 @@ struct Builder {
             int r = build(lo + half, n - half, depth + 1);
             nodes[id].left = l;
             nodes[id].right = r;
-            nodes[id].box = box_expand(nodes[l].box, nodes[r].box);
+            nodes[id].box = node_union(nodes[l].box, nodes[r].box);
             nodes[id].unbounded = nodes[l].unbounded || nodes[r].unbounded;
         }
         return id;
@@ -460,158 +495,151 @@ static inline float as_float(int i) {
     memcpy(&f, &i, 4);
     return f;
 }
-}  // namespace
+constexpr int kSahMaxDepth = 22;   // binary levels below the root: keeps the traversal stack within FW_STACK
+static double half_area(const Box& x) {
+    double dx = (double)x.mx.x - x.mn.x, dy = (double)x.mx.y - x.mn.y, dz = (double)x.mx.z - x.mn.z;
+    dx = std::max(dx, 0.0); dy = std::max(dy, 0.0); dz = std::max(dz, 0.0);
+    return dx * dy + dy * dz + dz * dx;
+}
 
-bool build_bvh(const std::vector<Box>& item_boxes, FlatBVH& out, std::string& err,
-               const std::vector<uint8_t>* item_unbounded) {
-    out = FlatBVH();
-    if (item_boxes.empty()) {
-        err = "cannot build a BVH over zero items (the reference recurses forever: bvh.rs:59)";
-        return false;
+// Stage (b) over `leaves` (node ids in DFS order); appends the interior to `nodes`, returns the root.  With `recs`
+// (bvh_sah_device's records, `leaves` already in the device's final order) the splits are the device's and nothing is
+// sorted here; either way the nodes are made by the same code below, so their boxes are bit for bit the same.
+static int sah_tree(std::vector<BuildNode>& nodes, std::vector<int> leaves, const std::vector<SahRec>* recs) {
+    nodes.reserve(nodes.size() + leaves.size());
+    auto center = [&](int id, int a) {
+        const Box& x = nodes[id].box;
+        return a == 0 ? 0.5 * ((double)x.mn.x + x.mx.x) : a == 1 ? 0.5 * ((double)x.mn.y + x.mx.y) : 0.5 * ((double)x.mn.z + x.mx.z);
+    };
+    // Full-sweep SAH over the leaves, per node: order by centre along x, then (stably) y, then z; for every axis sweep
+    // the split position.  All per-node state lives in slices [lo, lo + n) of buffers sized once (a node is done with
+    // its slice before its children use theirs), and the leaf centres / areas are computed once: scene builds are on
+    // the end-to-end path of every render (SURVEY §8 f3), and the per-node vectors + std::stable_sort's temporary
+    // buffer were most of fw_scene_commit for a 500-object scene.
+    const int nl = (int)leaves.size();
+    const int n_bn = (int)nodes.size();
+    std::vector<double> ctr[3];
+    for (int a = 0; a < 3; ++a) {
+        ctr[a].resize(n_bn);
+        for (int id : leaves) {
+            double c = center(id, a);
+            ctr[a][id] = c == c ? c : INFINITY;   // NaN centre (unbounded box): any consistent place will do
+        }
     }
-    Builder b(item_boxes);
-    b.unbounded = item_unbounded;
-    b.nodes.reserve(item_boxes.size() * 2);
-    int root = b.build(0, (int)item_boxes.size(), 0);
-    if (b.nan) {
-        err = "Float comparison failed in BVH constructor (NaN centroid; bvh.rs:34)";
-        return false;
-    }
-    out.items = b.order;
-    for (const BuildNode& n : b.nodes) out.max_depth = std::max(out.max_depth, n.depth);
-    // Collapse the reference's binary tree two levels at a time into 4-wide nodes (breadth-first, so the top
-    // levels are contiguous).  A wide node holds the boxes of the binary node's grandchildren (or of a child that
-    // is itself a leaf).  Skipping the intermediate child's box test cannot change which leaves are reached: the
-    // child's box contains the grandchild's, and the slab arithmetic (aabb.rs:38-47) is monotonic in the box
-    // planes, so "grandchild box hit" implies "child box hit" bit for bit.
-    auto leaf_code = [](const BuildNode& n) { return ~(n.first * 2 + (n.count - 1)); };  // items [first, first+count)
-    out.root_box = b.nodes[root].box;
-    if (b.nodes[root].count > 0) {
-        out.root_code = leaf_code(b.nodes[root]);
-        return true;
-    }
-    // Interior re-clustering.  Which items a ray tests is decided by the LEAF boxes alone: a leaf (bvh.rs Leaf /
-    // DoubleLeaf, with the reference's box for it) is reached iff its own box test passes, because every ancestor's
-    // box contains it and the slab arithmetic is monotonic in the box planes.  Any hierarchy that conservatively
-    // bounds those leaves therefore yields the reference's candidate set, and the (t, DFS rank) merge rule does not
-    // depend on visiting order.  The reference's tree (median split on a cycling axis) supplies the leaves, their
-    // boxes and their DFS ranks; the interior nodes above them are rebuilt with a surface-area heuristic, which
-    // roughly halves the boxes a ray has to test (FW_BVH_SAH=0 keeps the reference's interior).
-    static const bool use_sah = [] { const char* e = getenv("FW_BVH_SAH"); return !e || atoi(e) != 0; }();
-    if (use_sah) {
-        std::vector<int> leaves;
-        for (int i = 0; i < (int)b.nodes.size(); ++i)
-            if (b.nodes[i].count > 0) leaves.push_back(i);   // creation order == DFS order
-        b.nodes.reserve(b.nodes.size() + leaves.size());
-        auto area = [](const Box& x) {
-            double dx = (double)x.mx.x - x.mn.x, dy = (double)x.mx.y - x.mn.y, dz = (double)x.mx.z - x.mn.z;
-            dx = std::max(dx, 0.0); dy = std::max(dy, 0.0); dz = std::max(dz, 0.0);
-            return dx * dy + dy * dz + dz * dx;
-        };
-        auto center = [&](int id, int a) {
-            const Box& x = b.nodes[id].box;
-            return a == 0 ? 0.5 * ((double)x.mn.x + x.mx.x) : a == 1 ? 0.5 * ((double)x.mn.y + x.mx.y) : 0.5 * ((double)x.mn.z + x.mx.z);
-        };
-        constexpr int kMaxDepth = 22;   // binary levels below the root: keeps the traversal stack within FW_STACK
-        // Full-sweep SAH over the leaves, per node: order by centre along x, then (stably) y, then z; for every axis sweep
-        // the split position.  All per-node state lives in slices [lo, lo + n) of buffers sized once (a node is done with
-        // its slice before its children use theirs), and the leaf centres / areas are computed once: scene builds are on
-        // the end-to-end path of every render (SURVEY §8 f3), and the per-node vectors + std::stable_sort's temporary
-        // buffer were most of fw_scene_commit for a 500-object scene.
-        const int nl = (int)leaves.size();
-        const int n_bn = (int)b.nodes.size();
-        std::vector<double> ctr[3];
-        for (int a = 0; a < 3; ++a) {
-            ctr[a].resize(n_bn);
-            for (int id : leaves) {
-                double c = center(id, a);
-                ctr[a][id] = c == c ? c : INFINITY;   // NaN centre (unbounded box): any consistent place will do
+    std::vector<int> ord[3];
+    for (int a = 0; a < 3; ++a) ord[a].resize(nl);
+    std::vector<double> right_area(nl);
+    std::vector<int> merge_tmp(nl);
+    auto sort_by = [&](int* v, int n, const std::vector<double>& key) {   // stable, ascending
+        if (n <= 32) {
+            for (int i = 1; i < n; ++i) {
+                int x = v[i];
+                double kx = key[x];
+                int j = i;
+                while (j > 0 && kx < key[v[j - 1]]) { v[j] = v[j - 1]; --j; }
+                v[j] = x;
+            }
+            return;
+        }
+        // bottom-up merge sort over runs of 16 sorted by insertion
+        for (int r = 0; r < n; r += 16) {
+            int e = std::min(n, r + 16);
+            for (int i = r + 1; i < e; ++i) {
+                int x = v[i];
+                double kx = key[x];
+                int j = i;
+                while (j > r && kx < key[v[j - 1]]) { v[j] = v[j - 1]; --j; }
+                v[j] = x;
             }
         }
-        std::vector<int> ord[3];
-        for (int a = 0; a < 3; ++a) ord[a].resize(nl);
-        std::vector<double> right_area(nl);
-        std::vector<int> merge_tmp(nl);
-        auto sort_by = [&](int* v, int n, const std::vector<double>& key) {   // stable, ascending
-            if (n <= 32) {
-                for (int i = 1; i < n; ++i) {
-                    int x = v[i];
-                    double kx = key[x];
-                    int j = i;
-                    while (j > 0 && kx < key[v[j - 1]]) { v[j] = v[j - 1]; --j; }
-                    v[j] = x;
-                }
-                return;
+        int* src = v;
+        int* dst = merge_tmp.data();
+        for (int w = 16; w < n; w *= 2) {
+            for (int r = 0; r < n; r += 2 * w) {
+                int m = std::min(n, r + w), e = std::min(n, r + 2 * w);
+                int i = r, j = m, o = r;
+                while (i < m && j < e) dst[o++] = key[src[j]] < key[src[i]] ? src[j++] : src[i++];
+                while (i < m) dst[o++] = src[i++];
+                while (j < e) dst[o++] = src[j++];
             }
-            // bottom-up merge sort over runs of 16 sorted by insertion
-            for (int r = 0; r < n; r += 16) {
-                int e = std::min(n, r + 16);
-                for (int i = r + 1; i < e; ++i) {
-                    int x = v[i];
-                    double kx = key[x];
-                    int j = i;
-                    while (j > r && kx < key[v[j - 1]]) { v[j] = v[j - 1]; --j; }
-                    v[j] = x;
-                }
+            std::swap(src, dst);
+        }
+        if (src != v) std::copy(src, src + n, v);
+    };
+    auto add_interior = [&](int l, int r, int depth) {
+        int id = (int)nodes.size();
+        nodes.emplace_back();
+        nodes[id].depth = depth;
+        nodes[id].left = l;
+        nodes[id].right = r;
+        nodes[id].box = sah_union(nodes[l].box, nodes[r].box);
+        nodes[id].unbounded = nodes[l].unbounded || nodes[r].unbounded;
+        return id;
+    };
+    std::function<int(int, int, int, int)> sah = [&](int lo, int n, int depth, int rec) -> int {
+        if (n == 1) return leaves[lo];
+        if (recs) {
+            const SahRec& q = (*recs)[rec];
+            int l = sah(lo, q.k, depth + 1, q.left);
+            int r = sah(lo + q.k, n - q.k, depth + 1, q.right);
+            return add_interior(l, r, depth);
+        }
+        int best_axis = -1, best_k = n / 2;
+        double best_cost = INFINITY;
+        int levels_needed = 0;
+        while ((1 << levels_needed) < n) ++levels_needed;
+        const bool balanced = depth + levels_needed >= kSahMaxDepth;
+        int items_total = 0;
+        for (int i = 0; i < n; ++i) items_total += nodes[leaves[lo + i]].count;
+        for (int a = 0; a < 3; ++a) {
+            int* tmp = ord[a].data() + lo;
+            const int* from = a == 0 ? leaves.data() + lo : ord[a - 1].data() + lo;
+            std::copy(from, from + n, tmp);
+            sort_by(tmp, n, ctr[a]);
+            Box acc = nodes[tmp[n - 1]].box;
+            for (int i = n - 1; i > 0; --i) {
+                acc = box_expand(acc, nodes[tmp[i]].box);
+                right_area[lo + i] = half_area(acc);
             }
-            int* src = v;
-            int* dst = merge_tmp.data();
-            for (int w = 16; w < n; w *= 2) {
-                for (int r = 0; r < n; r += 2 * w) {
-                    int m = std::min(n, r + w), e = std::min(n, r + 2 * w);
-                    int i = r, j = m, o = r;
-                    while (i < m && j < e) dst[o++] = key[src[j]] < key[src[i]] ? src[j++] : src[i++];
-                    while (i < m) dst[o++] = src[i++];
-                    while (j < e) dst[o++] = src[j++];
-                }
-                std::swap(src, dst);
+            acc = nodes[tmp[0]].box;
+            int items_left = 0;
+            for (int k = 1; k < n; ++k) {   // left = tmp[0..k), right = tmp[k..n)
+                acc = box_expand(acc, nodes[tmp[k - 1]].box);
+                items_left += nodes[tmp[k - 1]].count;
+                if (balanced && k != n / 2) continue;
+                double cost = half_area(acc) * items_left + right_area[lo + k] * (items_total - items_left);
+                if (cost < best_cost) { best_cost = cost; best_axis = a; best_k = k; }
             }
-            if (src != v) std::copy(src, src + n, v);
-        };
-        std::function<int(int, int, int)> sah = [&](int lo, int n, int depth) -> int {
-            if (n == 1) return leaves[lo];
-            int best_axis = -1, best_k = n / 2;
-            double best_cost = INFINITY;
-            int levels_needed = 0;
-            while ((1 << levels_needed) < n) ++levels_needed;
-            const bool balanced = depth + levels_needed >= kMaxDepth;
-            int items_total = 0;
-            for (int i = 0; i < n; ++i) items_total += b.nodes[leaves[lo + i]].count;
-            for (int a = 0; a < 3; ++a) {
-                int* tmp = ord[a].data() + lo;
-                const int* from = a == 0 ? leaves.data() + lo : ord[a - 1].data() + lo;
-                std::copy(from, from + n, tmp);
-                sort_by(tmp, n, ctr[a]);
-                Box acc = b.nodes[tmp[n - 1]].box;
-                for (int i = n - 1; i > 0; --i) {
-                    acc = box_expand(acc, b.nodes[tmp[i]].box);
-                    right_area[lo + i] = area(acc);
-                }
-                acc = b.nodes[tmp[0]].box;
-                int items_left = 0;
-                for (int k = 1; k < n; ++k) {   // left = tmp[0..k), right = tmp[k..n)
-                    acc = box_expand(acc, b.nodes[tmp[k - 1]].box);
-                    items_left += b.nodes[tmp[k - 1]].count;
-                    if (balanced && k != n / 2) continue;
-                    double cost = area(acc) * items_left + right_area[lo + k] * (items_total - items_left);
-                    if (cost < best_cost) { best_cost = cost; best_axis = a; best_k = k; }
-                }
-            }
-            if (best_axis < 0) { best_axis = 2; best_k = n / 2; }   // non-finite areas: any split is valid
-            std::copy(ord[best_axis].begin() + lo, ord[best_axis].begin() + lo + n, leaves.begin() + lo);
-            int l = sah(lo, best_k, depth + 1);
-            int r = sah(lo + best_k, n - best_k, depth + 1);
-            int id = (int)b.nodes.size();
-            b.nodes.emplace_back();
-            b.nodes[id].depth = depth;
-            b.nodes[id].left = l;
-            b.nodes[id].right = r;
-            b.nodes[id].box = box_expand(b.nodes[l].box, b.nodes[r].box);
-            b.nodes[id].unbounded = b.nodes[l].unbounded || b.nodes[r].unbounded;
-            return id;
-        };
-        root = sah(0, (int)leaves.size(), 0);
-    }
+        }
+        if (best_axis < 0) { best_axis = 2; best_k = n / 2; }   // non-finite areas: any split is valid
+        std::copy(ord[best_axis].begin() + lo, ord[best_axis].begin() + lo + n, leaves.begin() + lo);
+        int l = sah(lo, best_k, depth + 1, -1);
+        int r = sah(lo + best_k, n - best_k, depth + 1, -1);
+        return add_interior(l, r, depth);
+    };
+    return sah(0, nl, 0, 0);
+}
+
+// Stage (b) on a device: the splits and the final leaf order come from bvh_sah_device.
+static int sah_device(int device, std::vector<BuildNode>& nodes, const std::vector<int>& leaves, std::string& err) {
+    std::vector<Box> boxes(leaves.size());
+    std::vector<int> counts(leaves.size());
+    for (size_t i = 0; i < leaves.size(); ++i) { boxes[i] = nodes[leaves[i]].box; counts[i] = nodes[leaves[i]].count; }
+    std::vector<SahRec> recs;
+    std::vector<int> leaf_order;
+    if (!bvh_sah_device(device, boxes, counts, kSahMaxDepth, recs, leaf_order, err)) return -1;
+    std::vector<int> ordered(leaves.size());
+    for (size_t i = 0; i < leaves.size(); ++i) ordered[i] = leaves[leaf_order[i]];
+    return sah_tree(nodes, std::move(ordered), &recs);
+}
+
+// Stage (c): collapse the binary tree two levels at a time into 4-wide nodes (breadth-first, so the top levels are
+// contiguous).  A wide node holds the boxes of the binary node's grandchildren (or of a child that is itself a leaf).
+// Skipping the intermediate child's box test cannot change which leaves are reached: the child's box contains the
+// grandchild's, and the slab arithmetic (aabb.rs:38-47) is monotonic in the box planes, so "grandchild box hit" implies
+// "child box hit" bit for bit.  The greedy collapse of an SAH interior reads structure, boxes and leaf codes only.
+static void collapse(const std::vector<BuildNode>& nodes, int root, bool greedy, FlatBVH& out) {
+    auto leaf_code = [](const BuildNode& n) { return ~(n.first * 2 + (n.count - 1)); };  // items [first, first+count)
     out.root_code = 0;
     struct Pending { int bn; int wide; int depth; };
     std::deque<Pending> q;
@@ -622,31 +650,27 @@ bool build_bvh(const std::vector<Box>& item_boxes, FlatBVH& out, std::string& er
         Pending cur = q.front();
         q.pop_front();
         out.wide_depth = std::max(out.wide_depth, cur.depth);
-        const BuildNode& n = b.nodes[cur.bn];
+        const BuildNode& n = nodes[cur.bn];
         int kids[4], nk = 0;
-        if (use_sah) {
+        if (greedy) {
             // greedy collapse: open the interior child with the largest box until the four slots are used
-            auto half_area = [](const Box& x) {
-                double dx = std::max((double)x.mx.x - x.mn.x, 0.0), dy = std::max((double)x.mx.y - x.mn.y, 0.0), dz = std::max((double)x.mx.z - x.mn.z, 0.0);
-                return dx * dy + dy * dz + dz * dx;
-            };
             kids[nk++] = n.left; kids[nk++] = n.right;
             while (nk < 4) {
                 int pick = -1;
                 double best = -1.0;
                 for (int k = 0; k < nk; ++k)
-                    if (b.nodes[kids[k]].count == 0) {
-                        double a = half_area(b.nodes[kids[k]].box);
+                    if (nodes[kids[k]].count == 0) {
+                        double a = half_area(nodes[kids[k]].box);
                         if (!(a <= best)) { best = a; pick = k; }
                     }
                 if (pick < 0) break;
                 int open = kids[pick];
-                kids[pick] = b.nodes[open].left;
-                kids[nk++] = b.nodes[open].right;
+                kids[pick] = nodes[open].left;
+                kids[nk++] = nodes[open].right;
             }
         } else {
             for (int side : {n.left, n.right}) {
-                const BuildNode& c = b.nodes[side];
+                const BuildNode& c = nodes[side];
                 if (c.count > 0) kids[nk++] = side;
                 else { kids[nk++] = c.left; kids[nk++] = c.right; }
             }
@@ -655,7 +679,7 @@ bool build_bvh(const std::vector<Box>& item_boxes, FlatBVH& out, std::string& er
         int code[4], flag[4];
         for (int k = 0; k < 4; ++k) {
             if (k < nk) {
-                const BuildNode& c = b.nodes[kids[k]];
+                const BuildNode& c = nodes[kids[k]];
                 lo[0][k] = c.box.mn.x; lo[1][k] = c.box.mn.y; lo[2][k] = c.box.mn.z;
                 hi[0][k] = c.box.mx.x; hi[1][k] = c.box.mx.y; hi[2][k] = c.box.mx.z;
                 flag[k] = c.unbounded ? 1 : 0;
@@ -681,7 +705,69 @@ bool build_bvh(const std::vector<Box>& item_boxes, FlatBVH& out, std::string& er
         w[6] = float4{as_float(code[0]), as_float(code[1]), as_float(code[2]), as_float(code[3])};
         w[7] = float4{as_float(flag[0]), as_float(flag[1]), as_float(flag[2]), as_float(flag[3])};
     }
-    return true;
+}
+}  // namespace
+
+int build_bvh_on(int device, const std::vector<Box>& item_boxes, FlatBVH& out, std::string& err,
+                 const std::vector<uint8_t>* item_unbounded) {
+    out = FlatBVH();
+    if (item_boxes.empty()) {
+        err = "cannot build a BVH over zero items (the reference recurses forever: bvh.rs:59)";
+        return FW_ERR_SCENE;
+    }
+    Builder b(item_boxes);
+    b.unbounded = item_unbounded;
+    if (device >= 0) {
+        if (!bvh_leaf_order_device(device, item_boxes, b.order, b.nan, err)) return FW_ERR_CUDA;
+        b.sorted = true;
+    }
+    if (!b.nan) {
+        b.nodes.reserve(item_boxes.size() * 2);
+        b.build(0, (int)item_boxes.size(), 0);
+    }
+    if (b.nan) {
+        err = "Float comparison failed in BVH constructor (NaN centroid; bvh.rs:34)";
+        return FW_ERR_SCENE;
+    }
+    const int median_root = 0;   // creation order: the root comes first
+    out.items = b.order;
+    for (const BuildNode& n : b.nodes) out.max_depth = std::max(out.max_depth, n.depth);
+    out.root_box = b.nodes[median_root].box;
+    if (b.nodes[median_root].count > 0) {
+        out.root_code = ~(b.nodes[median_root].first * 2 + (b.nodes[median_root].count - 1));
+        return FW_OK;
+    }
+    // Interior re-clustering.  Which items a ray tests is decided by the LEAF boxes alone: a leaf (bvh.rs Leaf /
+    // DoubleLeaf, with the reference's box for it) is reached iff its own box test passes, because every ancestor's
+    // box contains it and the slab arithmetic is monotonic in the box planes.  Any hierarchy that conservatively
+    // bounds those leaves therefore yields the reference's candidate set, and the (t, DFS rank) merge rule does not
+    // depend on visiting order.  The reference's tree (median split on a cycling axis) supplies the leaves, their
+    // boxes and their DFS ranks; the interior nodes above them are rebuilt with a surface-area heuristic, which
+    // roughly halves the boxes a ray has to test (FW_BVH_SAH=0 keeps the reference's interior).
+    static const bool use_sah = [] { const char* e = getenv("FW_BVH_SAH"); return !e || atoi(e) != 0; }();
+    int root = median_root;
+    if (use_sah) {
+        std::vector<int> leaves;
+        for (int i = 0; i < (int)b.nodes.size(); ++i)
+            if (b.nodes[i].count > 0) leaves.push_back(i);   // creation order == DFS order
+        root = device >= 0 ? sah_device(device, b.nodes, leaves, err) : sah_tree(b.nodes, std::move(leaves), nullptr);
+        if (root < 0) return FW_ERR_CUDA;
+    }
+    collapse(b.nodes, root, use_sah, out);
+    return FW_OK;
+}
+
+static thread_local BvhDeviceScope* t_bvh_scope = nullptr;
+BvhDeviceScope::BvhDeviceScope(int d) : device(d), prev(t_bvh_scope) { t_bvh_scope = this; }
+BvhDeviceScope::~BvhDeviceScope() { t_bvh_scope = prev; }
+
+__attribute__((noinline)) bool build_bvh(const std::vector<Box>& item_boxes, FlatBVH& out, std::string& err,
+                                          const std::vector<uint8_t>* item_unbounded) {
+    BvhDeviceScope* sc = t_bvh_scope;
+    const int device = sc && sc->device >= 0 && item_boxes.size() >= kDeviceBvhMinItems ? sc->device : -1;
+    const int rc = build_bvh_on(device, item_boxes, out, err, item_unbounded);
+    if (rc != FW_OK && sc) sc->code = rc;
+    return rc == FW_OK;
 }
 
 // ------------------------------------------------------------------------------------------------------

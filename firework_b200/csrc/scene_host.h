@@ -68,8 +68,42 @@ struct FlatBVH {
 // The reference's median split (bvh.rs:21-71): stable sort on centroid[depth % 3], leaves of 1 or 2.
 // `item_unbounded` (optional, same length as item_boxes) marks items whose box does NOT bound their geometry
 // (Disk: disk.rs:85-90); every node above such an item is flagged so the traversal never distance-culls it.
+// device < 0 builds on the host; otherwise the sorts and the SAH splits run on that CUDA device (kernels_build.cu) and
+// the result is the host's, byte for byte.  Returns FW_OK or the FW_ERR_* code of `err`.
+int build_bvh_on(int device, const std::vector<Box>& item_boxes, FlatBVH& out, std::string& err,
+                 const std::vector<uint8_t>* item_unbounded = nullptr);
+// The tree flatten_scene builds: on the device of the calling thread's innermost BvhDeviceScope when it has at least
+// kDeviceBvhMinItems items, else on the host.
 bool build_bvh(const std::vector<Box>& item_boxes, FlatBVH& out, std::string& err,
                const std::vector<uint8_t>* item_unbounded = nullptr);
+// While alive, lets the calling thread's build_bvh calls build large trees on `device` (< 0: host), and records the
+// FW_ERR_* code of a failed build (FW_ERR_CUDA for a device failure) in `code`.  fw_scene_commit sets one around
+// flatten_scene, which therefore does not know where its trees are built.
+struct BvhDeviceScope {
+    explicit BvhDeviceScope(int device);
+    ~BvhDeviceScope();
+    BvhDeviceScope(const BvhDeviceScope&) = delete;
+    BvhDeviceScope& operator=(const BvhDeviceScope&) = delete;
+    int device;
+    int code = -2;   // FW_ERR_SCENE
+    BvhDeviceScope* prev;
+};
+
+// fw_scene_commit builds a tree of at least this many items on its device (DESIGN.md §8: measured crossover).
+constexpr size_t kDeviceBvhMinItems = 8192;
+
+// Device stages of build_bvh (kernels_build.cu).  bvh_leaf_order_device: the item order of the median-split tree, and
+// whether some node met a NaN centroid on its axis.  bvh_sah_device: the SAH interior over leaves with the given boxes
+// and item counts (DFS order); records in level order, parents before children, record 0 the root (no records when
+// there is one leaf); leaf_order is the final leaf permutation.
+struct SahRec {
+    int depth;
+    int left, right;   // record index (>= 0), or ~position of a single leaf in leaf_order
+    int k;             // leaves on the left
+};
+bool bvh_leaf_order_device(int device, const std::vector<Box>& boxes, std::vector<int>& order, bool& nan, std::string& err);
+bool bvh_sah_device(int device, const std::vector<Box>& leaf_boxes, const std::vector<int>& leaf_counts, int max_depth,
+                    std::vector<SahRec>& recs, std::vector<int>& leaf_order, std::string& err);
 
 struct HostFlat {
     std::vector<float4> nodes;

@@ -386,6 +386,24 @@ def selftest_shared_division(n_pairs: int, seed: int = 1, device: int = 0):
     return int(v[0]), int(v[1])
 
 
+def bvh_build(boxes, unbounded=None, device: int = 0) -> dict:
+    """fw_bvh_build: one BVH over boxes (n, 6) = (min xyz, max xyz), as a scene build makes each tree; on the host when
+    device = -1, else with the sorts and SAH splits on that CUDA device.  Returns items (leaf order), nodes (wide nodes,
+    (count, 32) float32), root_box and info {nodes, root_code, wide_depth, max_depth}."""
+    b = np.ascontiguousarray(boxes, np.float32).reshape(-1, 6)
+    n = b.shape[0]
+    u = None if unbounded is None else np.ascontiguousarray(unbounded, np.uint8).reshape(n)
+    items = np.empty(max(n, 1), np.int32)
+    root = np.empty(6, np.float32)
+    info = np.zeros(4, np.int32)
+    cap = 2 * n + 1   # the SAH tree has n_leaves - 1 <= n interior nodes; every wide node opens at least one of them
+    nodes = np.empty((cap, 32), np.float32)
+    N.check(N.lib().fw_bvh_build(int(device), n, N.ptr(b), None if u is None else N.ptr(u), N.ptr(items), N.ptr(nodes), cap,
+                                 N.ptr(root), N.ptr(info)))
+    return {"items": items[:n], "nodes": nodes[:info[0]].copy(), "root_box": root,
+            "info": {"nodes": int(info[0]), "root_code": int(info[1]), "wide_depth": int(info[2]), "max_depth": int(info[3])}}
+
+
 def texture_store_stats() -> dict:
     """fw_texture_store_stats: commits served from a resident array, uploads, arrays resident now and their bytes."""
     v = np.zeros(4, np.uint64)

@@ -79,7 +79,8 @@ int fw_scene_set_image(fw_scene* scene, int index, uint32_t width, uint32_t heig
 int fw_scene_set_hdr(fw_scene* scene, int index, uint32_t width, uint32_t height, const float* rgb32f);
 
 /* fw_scene_build_host: builds the BVHs with the reference's split rule (src/bvh.rs:21-71) and flattens the
- * scene into pointer-free arrays — host only, no CUDA.  fw_scene_commit: the same, then uploads to `device`. */
+ * scene into pointer-free arrays — host only, no CUDA.  fw_scene_commit: the same, then uploads to `device`; it builds
+ * the trees of at least 8192 items on `device` (fw_bvh_build), with the same result. */
 int fw_scene_build_host(fw_scene* scene);
 int fw_scene_commit(fw_scene* scene, int device);
 
@@ -273,6 +274,14 @@ int fw_scatter_step_keyed(fw_scene* scene, uint64_t seed, uint32_t n, const int3
 int fw_env_sample(fw_scene* scene, uint32_t n, const float* dirs, float* out);
 int fw_texture_sample(fw_scene* scene, int texture, uint32_t n, const float* uv, const float* point, float* out);
 int fw_material_texture(const fw_scene* scene, int material);  /* texture index of a material, or -1 */
+/* fw_bvh_build : one BVH over caller boxes (n x {min xyz, max xyz}; `unbounded` nullable, n bytes), as fw_scene_build_host
+ *                builds each tree (bvh.rs:21-71 leaves, SAH interior, 4-wide collapse): on the host when device = -1,
+ *                else with the sorts and splits on that CUDA device, byte for byte the host's result.  items_out (n) gets
+ *                the item ids in leaf order; nodes_out (nullable) up to capacity_nodes wide nodes (32 floats each,
+ *                fw_types.h); root_box the binary root's box; info = {wide nodes, root code, wide depth, binary depth}.
+ *                Argument errors (n = 0 included) come before any CUDA call; a NaN centroid gives FW_ERR_SCENE. */
+int fw_bvh_build(int device, uint32_t n, const float* boxes, const uint8_t* unbounded, int32_t* items_out, float* nodes_out,
+                 int capacity_nodes, float root_box[6], int32_t info[4]);
 int fw_camera(const fw_params* params, float out24[24]);        /* camera.rs:74-107 constants, host only */
 
 /* ---- misc ----------------------------------------------------------------------------------------------- */
